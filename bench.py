@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # our CUDA path
     python bench.py --impl reference [...]                         # the reference's CPU path
+    python bench.py --dump-outputs DIR [...]                       # also write the last timed step's outputs
 
 A step is one fwd+bwd of DenseCRFLoss over one batch of synthetic frames per GPU
 (configs[1] of BASELINE.json: 32 frames x 10 classes x 224x224, sigma_rgb=15, sigma_xy=100):
@@ -60,7 +61,14 @@ def parse_args():
                     help="skip the ResNet-50 train-step context run (other_inputs.train_step_resnet50)")
     ap.add_argument("--no-occupancy-sweep", dest="occupancy_sweep", action="store_false",
                     help="skip the 448x448 hash-load sweep (other_inputs.occupancy_sweep_448)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (rank 0: loss, segmentation gradient) as DIR/*.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 # ---------------------------------------------------------------------------
@@ -424,12 +432,16 @@ def run_ours(args, rank: int, local_rank: int, world: int):
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     ev0.record()
-    for i in range(args.steps):
+    for i in range(args.steps - 1):
         step(i)
+    loss_last = step(args.steps - 1).detach()   # the graph (it holds the step's buffers) is freed as after any step
     ev1.record()
     barrier()
     ms_total = ev0.elapsed_time(ev1)
     launches = lib.tcamcrf_launch_count() - launches0
+    # rank 0's outputs of the last timed step; every step returns fresh tensors, so these stay as that step left them
+    dumped = (loss_last, sets[(args.steps - 1) % len(sets)][3].grad) if args.dump_outputs and rank == 0 else None
+    del loss_last
 
     # per-stage times: the same steps again with CUDA events around every stage (tcamcrf_profile_*).  Kept out of
     # the timed region above because an event record between two kernels stops the next kernel's blocks from
@@ -657,6 +669,8 @@ def run_ours(args, rank: int, local_rank: int, world: int):
         "clocks": dict(sampler.summary(), window="warm-up + timed region + per-stage pass + e2e legs"),
         "other_inputs": extra,
     }
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, *dumped)
     emit(line)
     if parity is not None and not parity["ok"]:
         sys.stderr.write("bench.py: PARITY FAILED: %r\n" % (parity,))
@@ -925,6 +939,24 @@ def reference_cpu_crf(torch):
 
         _REF_CPU_CRF = Fn
     return _REF_CPU_CRF
+
+
+DUMP_MAX_VALUES = 1 << 23   # 32 MiB of float32
+
+
+def dump_outputs(out_dir: str, loss, grad) -> None:
+    """Writes the loss (loss.npy) and the gradient of the segmentations (segmentations_grad.npy) in float32.  A
+    gradient of more than DUMP_MAX_VALUES values is written as its values at a fixed set of flat positions
+    (numpy default_rng(0), ascending), the same for every build of the project, so that two builds can be compared
+    output for output."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), loss.detach().float().cpu().numpy())
+    grad = grad.detach()
+    if grad.numel() > DUMP_MAX_VALUES:
+        idx = np.sort(np.random.default_rng(0).choice(grad.numel(), DUMP_MAX_VALUES, replace=False))
+        grad = grad.reshape(-1)[torch.from_numpy(idx).to(grad.device)]
+    np.save(os.path.join(out_dir, "segmentations_grad.npy"), grad.float().cpu().numpy())
 
 
 _REAL_STDOUT = None

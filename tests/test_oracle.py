@@ -2,9 +2,11 @@
 
 * the C restatement (oracle/permuto_oracle.c) reproduces, bit for bit, every committed golden
   fixture -- those were produced by the reference's own C++ (tests/golden/make_golden.py);
-* where the reference build is present (oracle/_ref, i.e. in the build container) the two are
-  compared directly, including the lattice internals (offset_, barycentric_, neighbours, M).
+* for six more cases the filtered tensors and the lattice internals (offset_, barycentric_, neighbours, M)
+  match, bit for bit, digests stored from the reference build in tests/golden/lattice/, and the reference
+  build itself wherever it is present (oracle/_ref).
 """
+import hashlib
 import os
 
 import numpy as np
@@ -68,28 +70,51 @@ def test_port_lattice_size_matches_golden(oracle_mod, path):
     assert L.nbr.min() >= -1 and L.nbr.max() < L.m
 
 
-@pytest.mark.parametrize("kind", ["noise", "natural"])
-@pytest.mark.parametrize("shape", [(2, 2, 32, 40), (1, 3, 31, 37), (1, 1, 7, 5)])
-def test_port_vs_reference_build(oracle_mod, kind, shape):
-    if not oracle_mod.have_ref():
-        pytest.skip("oracle/_ref not built (no /root/reference on this box)")
+LATTICE_KINDS = ("noise", "natural")
+LATTICE_SHAPES = ((2, 2, 32, 40), (1, 3, 31, 37), (1, 1, 7, 5))
+
+
+def lattice_case_name(kind, shape):
+    return "%s_n%d_k%d_%dx%d" % ((kind,) + tuple(shape))
+
+
+def lattice_case_arrays(oracle_mod, kind, shape, ref):
+    """Filtered tensors of both wrappers and the first frame's two lattices (offset_, barycentric_, neighbour table,
+    M) for one case, from the reference build (ref=True) or the C restatement."""
     n, k, h, w = shape
     img = synth.make_images(n, h, w, kind, seed=7)
     seg = synth.make_segs(n, k, h, w, seed=7)
-    a = oracle_mod.port_bilateralfilter_batch(img, seg, n, k, h, w, 15.0, 100.0)
-    b = oracle_mod.ref_bilateralfilter_batch(img, seg, n, k, h, w, 15.0, 100.0)
-    assert np.array_equal(a, b)
-    a = oracle_mod.port_colorbilateralfilter_batch(img, seg, n, k, h, w, 15.0, 3)
-    b = oracle_mod.ref_colorbilateralfilter_batch(img, seg, n, k, h, w, 15.0, 3)
-    assert np.array_equal(a, b)
-    for Lp, Lr in ((oracle_mod.port_lattice_bilateral(img[0], h, w, 15.0, 100.0),
-                    oracle_mod.ref_lattice_bilateral(img[0], h, w, 15.0, 100.0)),
-                   (oracle_mod.port_lattice_color(img[0], h, w, 15.0, 3),
-                    oracle_mod.ref_lattice_color(img[0], h, w, 15.0, 3))):
-        assert Lp.m == Lr.m
-        assert np.array_equal(Lp.offset, Lr.offset)
-        assert np.array_equal(Lp.bary, Lr.bary)
-        assert np.array_equal(Lp.nbr, Lr.nbr)
+    o = oracle_mod
+    bf = o.ref_bilateralfilter_batch if ref else o.port_bilateralfilter_batch
+    cbf = o.ref_colorbilateralfilter_batch if ref else o.port_colorbilateralfilter_batch
+    out = {"bf_AS": bf(img, seg, n, k, h, w, 15.0, 100.0), "cbf_AS": cbf(img, seg, n, k, h, w, 15.0, 3)}
+    for tag, L in (("bf", (o.ref_lattice_bilateral if ref else o.port_lattice_bilateral)(img[0], h, w, 15.0, 100.0)),
+                   ("cbf", (o.ref_lattice_color if ref else o.port_lattice_color)(img[0], h, w, 15.0, 3))):
+        out[tag + "_M"] = np.int32(L.m)
+        out[tag + "_offset"] = np.ascontiguousarray(L.offset, dtype=np.int32)
+        out[tag + "_bary"] = np.ascontiguousarray(L.bary, dtype=np.float32)
+        out[tag + "_nbr"] = np.ascontiguousarray(L.nbr, dtype=np.int32)
+    return out
+
+
+def sha256_of(a):
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+@pytest.mark.parametrize("kind", LATTICE_KINDS)
+@pytest.mark.parametrize("shape", LATTICE_SHAPES)
+def test_port_vs_reference_build(oracle_mod, kind, shape):
+    """Bit for bit: against the digests stored in tests/golden/lattice/ (tests/golden/make_golden_lattice.py) and,
+    where oracle/_ref is built, against the live reference build too."""
+    port = lattice_case_arrays(oracle_mod, kind, shape, ref=False)
+    g = load_golden(os.path.join(GOLDEN, "lattice", lattice_case_name(kind, shape) + ".npz"))
+    for key, a in port.items():
+        assert a.dtype == np.dtype(str(g[key + "_dtype"])) and a.shape == tuple(g[key + "_shape"]), key
+        assert sha256_of(a) == str(g[key + "_sha256"]), (key, a.sum(dtype=np.float64), float(g[key + "_sum"]))
+    if oracle_mod.have_ref():
+        ref = lattice_case_arrays(oracle_mod, kind, shape, ref=True)
+        for key, a in port.items():
+            assert np.array_equal(a, ref[key]), key
 
 
 def test_filter_is_linear_and_symmetric_enough(oracle_mod):
