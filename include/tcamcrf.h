@@ -281,7 +281,8 @@ int tcam_seed_labels(const int *sel_dev, int kmax, int B, int H, int W, int ksz,
  *     the kernel by Philox4x32-10 keyed with the two words at rng_dev (fresh per call, e.g. from torch's generator);
  *   - labels_dev [B,H,W] int64 (or NULL): flat ksz x ksz dilation of the seeds, conflicts -> ignore (:239-254).
  * sel_dev [B,2,kmax] pixel indices (-1 = unused).  tcam_seed_fused_supported: the slice of a frame (H*W/8 pixels,
- * 8 bytes each) must fit the shared memory of an SM and kmax <= 32; otherwise use tcam_seed_select + tcam_seed_labels. */
+ * 8 bytes each) must fit the shared memory of an SM and kmax <= 32; otherwise use tcam_seed_select + tcam_seed_labels.
+ * It answers for the current device: ask with the device current that tcam_seed_fused will run on. */
 int tcam_seed_fused_supported(int HW, int kmax);
 int tcam_seed_fused(const float *cams_dev, int T, const int64_t *roi_dev, const float *q_dev, const int *q_offset_dev,
                     const int *n_cand_dev, const unsigned int *rng_dev, float max_p, int n_fg_fixed, int n_bg, int k_fg,

@@ -120,69 +120,6 @@ static Tuning &tuning()
 }
 
 // ---------------------------------------------------------------------------
-// optional per-stage timing (CUDA events on the caller's stream) + launch counter
-// ---------------------------------------------------------------------------
-enum Stage { kStBuild = 0, kStNeighbour, kStSplat, kStBlur, kStSlice, kStLoss, kStBackward, kStPrepare, kStSeed, kStCount };
-static_assert(kStCount == TCAMCRF_STAGES, "stage list and header disagree");
-
-struct Profiler {
-    std::mutex mu;
-    bool enabled = false;
-    struct Span {
-        int stage;
-        int launches;
-        cudaEvent_t a, b;
-    };
-    std::vector<Span> spans;
-    std::vector<cudaEvent_t> pool;
-    double ms[kStCount] = {0};
-    long long launches[kStCount] = {0};
-    long long total_launches = 0;
-
-    cudaEvent_t get()
-    {
-        if (!pool.empty()) {
-            cudaEvent_t e = pool.back();
-            pool.pop_back();
-            return e;
-        }
-        cudaEvent_t e = nullptr;
-        cudaEventCreate(&e);
-        return e;
-    }
-};
-static Profiler g_prof;
-
-// Brackets the launches of one stage.  When profiling is off it only counts launches.
-struct StageScope {
-    int stage, launches;
-    cudaStream_t st;
-    cudaEvent_t a = nullptr;
-    StageScope(int stage_, int launches_, cudaStream_t st_) : stage(stage_), launches(launches_), st(st_)
-    {
-        static const char *const names[kStCount] = {"tcamcrf:build", "tcamcrf:neighbour", "tcamcrf:splat", "tcamcrf:blur",
-                                                    "tcamcrf:slice", "tcamcrf:loss", "tcamcrf:backward",
-                                                    "tcamcrf:prepare", "tcamcrf:seed"};
-        nvtxRangePushA(names[stage]);   // host-side range around the launches of the stage (nsys / ncu --nvtx)
-        std::lock_guard<std::mutex> lock(g_prof.mu);
-        g_prof.total_launches += launches;
-        if (g_prof.enabled) {
-            a = g_prof.get();
-            cudaEventRecord(a, st);
-        }
-    }
-    ~StageScope()
-    {
-        nvtxRangePop();
-        if (!a) return;
-        std::lock_guard<std::mutex> lock(g_prof.mu);
-        cudaEvent_t b = g_prof.get();
-        cudaEventRecord(b, st);
-        g_prof.spans.push_back({stage, launches, a, b});
-    }
-};
-
-// ---------------------------------------------------------------------------
 // workspace layout
 // ---------------------------------------------------------------------------
 constexpr int kThreads = 256;
@@ -1626,40 +1563,227 @@ __global__ void __launch_bounds__(kThreads) temporal_max_kernel(const float *__r
 // ---------------------------------------------------------------------------
 // host-side drivers
 // ---------------------------------------------------------------------------
-static int g_sm_count = 0;
 
-static int sm_count()
-{
-    if (g_sm_count == 0) {
-        int dev = 0, sms = 0;
-        if (cudaGetDevice(&dev) == cudaSuccess &&
-            cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && sms > 0)
-            g_sm_count = sms;
-        else
-            g_sm_count = 148;
+// Vertex density of the recent calls, per workspace (density_hint below).
+#ifndef TCAMCRF_DENSITY_HINT
+#define TCAMCRF_DENSITY_HINT 1
+#endif
+struct DensityHints {
+    struct Slot {
+        void *ws;
+        int *word;            // pinned
+        unsigned int calls;   // calls seen on this workspace
+    };
+    std::mutex mu;
+    std::vector<Slot> slots;   // a handful of workspaces per process
+    cudaStream_t side = nullptr;                   // the copies run here, off the caller's stream
+    cudaEvent_t ev = nullptr;
+    // caller holds `mu`
+    Slot *find(void *ws, bool create)
+    {
+        for (auto &s : slots)
+            if (s.ws == ws) return &s;
+        if (!create) return nullptr;
+        int *p = nullptr;
+        if (cudaHostAlloc((void **)&p, sizeof(int), cudaHostAllocDefault) != cudaSuccess) {
+            cudaGetLastError();
+            return nullptr;
+        }
+        *p = 0;
+        slots.push_back({ws, p, 0u});
+        return &slots.back();
     }
-    return g_sm_count;
+};
+
+// The copy stream of the host-frames path (run_chunk_host_frames) and the events that fork and join it.
+struct CopyLane {
+    std::mutex mu;
+    cudaStream_t stream = nullptr;
+    std::vector<cudaEvent_t> events;
+    size_t next = 0;
+    int ready()   // this device's copy stream, created on first use
+    {
+        if (stream) return TCAMCRF_OK;
+        CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
+        return TCAMCRF_OK;
+    }
+    int event(cudaEvent_t *ev)
+    {
+        if (events.size() < 64) {
+            cudaEvent_t e = nullptr;
+            CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+            events.push_back(e);
+            *ev = e;
+            return TCAMCRF_OK;
+        }
+        *ev = events[next++ % events.size()];   // a waiter keeps the record it was given: re-recording is safe
+        return TCAMCRF_OK;
+    }
+};
+
+// Cached buffers, streams and events of the host-pointer path (host_run).
+struct HostCtx {
+    std::mutex mu;
+    void *buf = nullptr;
+    size_t cap = 0;
+    cudaStream_t stream = nullptr;   // compute
+    cudaStream_t s_in = nullptr;     // host -> device copies
+    cudaStream_t s_out = nullptr;    // device -> host copies
+    std::vector<cudaEvent_t> events;
+    void *pin = nullptr;             // pinned staging: grad_out in, per-group losses and status words out
+    size_t pin_cap = 0;
+};
+
+// Captured schedules of host_run, a handful per device (a trainer alternates between a few pinned buffers).
+struct HostGraphs {
+    struct Key {
+        tcamcrf_config cfg;
+        int N, K, H, W;
+        const void *images, *segs, *as_host, *grad_host, *buf, *pin;
+        int want_loss, dedup, dense, groups_knob, taper_knob, sec0_knob, grow_knob;
+        bool operator==(const Key &o) const { return memcmp(this, &o, sizeof(Key)) == 0; }
+    };
+    struct Item {
+        Key key;
+        cudaGraphExec_t exec;
+        int groups;
+        long long launches;      // kernels of one replay (for tcamcrf_launch_count)
+        unsigned long long used;
+    };
+    std::vector<Item> items;
+    unsigned long long tick = 0;
+    void clear()
+    {
+        for (auto &it : items) cudaGraphExecDestroy(it.exec);
+        items.clear();
+    }
+};
+
+// What the library keeps per CUDA device: a process may drive several (threads of DataParallel, or alternating
+// cuda:0 / cuda:1), and each gets its own limits, kernel attributes, streams, events and buffers.
+struct Device {
+    std::once_flag once;
+    int sms = 148;                           // multiprocessors
+    int select_smem = 0;                     // dynamic shared memory of seed_select_smem_kernel (0: opt-in refused)
+    int fused_smem = 0;                      // the same for seed_fused_kernel
+    DensityHints hints;
+    CopyLane lane;
+    HostCtx host;
+    HostGraphs graphs;                       // guarded by host.mu
+    std::vector<cudaEvent_t> timing_events;  // free events of the stage profiler, guarded by g_prof.mu
+
+    void init(int ordinal)   // runs once, with this device current
+    {
+        int v = 0, optin = 0;
+        if (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, ordinal) == cudaSuccess && v > 0) sms = v;
+        cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, ordinal);
+        cudaFuncAttributes fa;
+        int stat = 12 * 1024;
+        if (cudaFuncGetAttributes(&fa, seed_fused_kernel) == cudaSuccess) stat = (int)fa.sharedSizeBytes;
+        const int sel = optin - 2048, fused = optin - stat - 1024;   // 2 KB: seed_select_smem_kernel's static smem
+        const cudaFuncAttribute smem = cudaFuncAttributeMaxDynamicSharedMemorySize;
+        if (sel > 0 && cudaFuncSetAttribute(seed_select_smem_kernel, smem, sel) == cudaSuccess) select_smem = sel;
+        if (fused > 0 && cudaFuncSetAttribute(seed_fused_kernel, smem, fused) == cudaSuccess) fused_smem = fused;
+        cudaGetLastError();   // a refused opt-in leaves the kernel at the default limit: not an error of any call
+    }
+    cudaEvent_t timing_event()
+    {
+        cudaEvent_t e = nullptr;
+        if (timing_events.empty()) {
+            cudaEventCreate(&e);
+            return e;
+        }
+        e = timing_events.back();
+        timing_events.pop_back();
+        return e;
+    }
+};
+constexpr int kMaxDevices = 64;
+static Device g_devices[kMaxDevices];
+
+// The context of the current device, set up on its first use.
+static int this_device(Device **out)
+{
+    int ordinal = 0;
+    CUDA_TRY(cudaGetDevice(&ordinal));
+    if (ordinal < 0 || ordinal >= kMaxDevices)
+        return fail(TCAMCRF_ERR_INVALID, "device %d: the library serves devices 0..%d", ordinal, kMaxDevices - 1);
+    Device &dev = g_devices[ordinal];
+    std::call_once(dev.once, [&] { dev.init(ordinal); });
+    *out = &dev;
+    return TCAMCRF_OK;
 }
 
 // persistent kernels: one wave of resident CTAs (8 x 256 threads per SM)
-static int persistent_grid() { return sm_count() * 8; }
+static int persistent_grid(const Device &dev) { return dev.sms * 8; }
 
 // Exactly one resident wave of `kernel` (what its register use allows), so that the frame-ordered sweep of
 // the vertex kernels really has all blocks on the same frame at the same time.
 template <typename Kernel>
-static int resident_grid(Kernel kernel)
+static int resident_grid(const Device &dev, Kernel kernel)
 {
-    static int cached = 0;  // one instance per kernel type
-    if (cached == 0) {
-        int per_sm = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kThreads, 0) != cudaSuccess || per_sm < 1) {
+    static const int per_sm = [kernel] {   // one instance per kernel type; depends on the architecture only
+        int n = 0;
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kernel, kThreads, 0) != cudaSuccess || n < 1) {
             cudaGetLastError();
-            per_sm = 4;
+            n = 4;
         }
-        cached = per_sm * sm_count();
-    }
-    return cached;
+        return n;
+    }();
+    return per_sm * dev.sms;
 }
+
+// ---------------------------------------------------------------------------
+// optional per-stage timing (CUDA events on the caller's stream) + launch counter
+// ---------------------------------------------------------------------------
+enum Stage { kStBuild = 0, kStNeighbour, kStSplat, kStBlur, kStSlice, kStLoss, kStBackward, kStPrepare, kStSeed, kStCount };
+static_assert(kStCount == TCAMCRF_STAGES, "stage list and header disagree");
+
+struct Profiler {
+    std::mutex mu;
+    bool enabled = false;
+    struct Span {
+        int stage;
+        int launches;
+        Device *dev;   // whose pool the events go back to
+        cudaEvent_t a, b;
+    };
+    std::vector<Span> spans;
+    double ms[kStCount] = {0};
+    long long launches[kStCount] = {0};
+    long long total_launches = 0;
+};
+static Profiler g_prof;
+
+// Brackets the launches of one stage.  When profiling is off it only counts launches.
+struct StageScope {
+    int stage, launches;
+    cudaStream_t st;
+    Device *dev = nullptr;
+    cudaEvent_t a = nullptr;
+    StageScope(int stage_, int launches_, cudaStream_t st_) : stage(stage_), launches(launches_), st(st_)
+    {
+        static const char *const names[kStCount] = {"tcamcrf:build", "tcamcrf:neighbour", "tcamcrf:splat", "tcamcrf:blur",
+                                                    "tcamcrf:slice", "tcamcrf:loss", "tcamcrf:backward",
+                                                    "tcamcrf:prepare", "tcamcrf:seed"};
+        nvtxRangePushA(names[stage]);   // host-side range around the launches of the stage (nsys / ncu --nvtx)
+        std::lock_guard<std::mutex> lock(g_prof.mu);
+        g_prof.total_launches += launches;
+        if (g_prof.enabled && this_device(&dev) == TCAMCRF_OK) {
+            a = dev->timing_event();
+            cudaEventRecord(a, st);
+        }
+    }
+    ~StageScope()
+    {
+        nvtxRangePop();
+        if (!a) return;
+        std::lock_guard<std::mutex> lock(g_prof.mu);
+        cudaEvent_t b = dev->timing_event();
+        cudaEventRecord(b, st);
+        g_prof.spans.push_back({stage, launches, dev, a, b});
+    }
+};
 
 static void scale_factors(int d, EmbedConsts &ec)
 {
@@ -1748,29 +1872,29 @@ static void launch_pixel(bool splat, int V, const PixelParams &pp, dim3 grid, cu
 }
 
 template <int V, int KV>
-static void launch_blur_kv(const BlurParams &bp, int nc, cudaStream_t st)
+static void launch_blur_kv(const Device &dev, const BlurParams &bp, int nc, cudaStream_t st)
 {
-    launch_chained(blur_kernel<V, KV>, dim3(resident_grid(blur_kernel<V, KV>)), st, bp, nc);
+    launch_chained(blur_kernel<V, KV>, dim3(resident_grid(dev, blur_kernel<V, KV>)), st, bp, nc);
 }
 
-static void launch_blur(int V, const BlurParams &bp, int nc, cudaStream_t st)
+static void launch_blur(const Device &dev, int V, const BlurParams &bp, int nc, cudaStream_t st)
 {
     const int kv = bp.Kp / V;
     if (V == 4) {
         switch (kv) {
-        case 1: return launch_blur_kv<4, 1>(bp, nc, st);
-        case 2: return launch_blur_kv<4, 2>(bp, nc, st);
-        case 3: return launch_blur_kv<4, 3>(bp, nc, st);   // K = 9..12
-        case 4: return launch_blur_kv<4, 4>(bp, nc, st);
-        case 6: return launch_blur_kv<4, 6>(bp, nc, st);   // K = 21..24 (VOC's 21 classes)
-        default: return launch_blur_kv<4, 0>(bp, nc, st);
+        case 1: return launch_blur_kv<4, 1>(dev, bp, nc, st);
+        case 2: return launch_blur_kv<4, 2>(dev, bp, nc, st);
+        case 3: return launch_blur_kv<4, 3>(dev, bp, nc, st);   // K = 9..12
+        case 4: return launch_blur_kv<4, 4>(dev, bp, nc, st);
+        case 6: return launch_blur_kv<4, 6>(dev, bp, nc, st);   // K = 21..24 (VOC's 21 classes)
+        default: return launch_blur_kv<4, 0>(dev, bp, nc, st);
         }
     }
-    if (V == 2) return launch_blur_kv<2, 1>(bp, nc, st);   // Kp = 2 is the only even, non-multiple-of-4 row width
-    return launch_blur_kv<1, 1>(bp, nc, st);               // Kp = 1
+    if (V == 2) return launch_blur_kv<2, 1>(dev, bp, nc, st);   // Kp = 2 is the only even, non-multiple-of-4 row width
+    return launch_blur_kv<1, 1>(dev, bp, nc, st);               // Kp = 1
 }
 
-static int density_hint(void *ws);   // largest per-frame vertex count seen lately on a workspace (0: unknown); below
+static int density_hint(Device &dev, void *ws);   // largest per-frame vertex count lately on ws (0: unknown); below
 
 // "Dense" lattice: more than one vertex per four pixels in the fullest frame lately (iid-noise frames have ~1.1 per
 // pixel, real frames ~0.06).  Selects kernel variants that are both correct for every input.
@@ -1780,14 +1904,14 @@ static bool lattice_is_dense(int hint, int P) { return (long long)hint * 4 > (lo
 // only the images.  `zero_values`: also clear the value rows in the same launch (the device path does; the
 // host path clears them group by group in value_stages).
 template <int D>
-static int lattice_stages(const tcamcrf_config *cfg, const Plan &pl, bool u8, const void *images, int frame0, int nc,
-                          char *ws, bool zero_values, cudaStream_t st)
+static int lattice_stages(Device &dev, const tcamcrf_config *cfg, const Plan &pl, bool u8, const void *images,
+                          int frame0, int nc, char *ws, bool zero_values, cudaStream_t st)
 {
     int *ctrl = (int *)(ws + pl.off_ctrl);
     Entry *table = (Entry *)(ws + pl.off_table);
     {
         StageScope scope(kStPrepare, 1, st);
-        prepare_kernel<<<persistent_grid(), kThreads, 0, st>>>(table, ctrl, frame0, nc, pl.chunk, pl.geom, pl.sig);
+        prepare_kernel<<<persistent_grid(dev), kThreads, 0, st>>>(table, ctrl, frame0, nc, pl.chunk, pl.geom, pl.sig);
     }
     {
         StageScope scope(kStBuild, 1, st);
@@ -1818,7 +1942,7 @@ static int lattice_stages(const tcamcrf_config *cfg, const Plan &pl, bool u8, co
         dim3 bgrid(pl.blocks_per_frame, nc);
 #endif
         // sparse lattice lately (or nothing known yet): deduplicate the block's keys in shared memory first
-        bool dedup = !lattice_is_dense(density_hint(ws), pl.P);
+        bool dedup = !lattice_is_dense(density_hint(dev, ws), pl.P);
         if (tuning().build_dedup >= 0) dedup = tuning().build_dedup != 0;   // tests and sweeps: force either way
         if (dedup)   // one block per 32 x 8 tile; one more row of blocks for the ghost pixel's block
             bgrid = dim3(nc, (pl.H + kTileH - 1) / kTileH + ((pl.P & 3) != 0 ? 1 : 0), (pl.W + kTileW - 1) / kTileW);
@@ -1843,7 +1967,7 @@ static int lattice_stages(const tcamcrf_config *cfg, const Plan &pl, bool u8, co
     vp.zero_values = zero_values ? 1 : 0;
     {
         StageScope scope(kStNeighbour, 1, st);
-        launch_chained(neighbour_kernel<D>, dim3(resident_grid(neighbour_kernel<D>)), st, vp, nc);
+        launch_chained(neighbour_kernel<D>, dim3(resident_grid(dev, neighbour_kernel<D>)), st, vp, nc);
     }
     CUDA_TRY(cudaGetLastError());
     return TCAMCRF_OK;
@@ -1856,50 +1980,6 @@ static int lattice_stages(const tcamcrf_config *cfg, const Plan &pl, bool u8, co
 // vertex count (kCtrlPrevMax) is copied into a pinned word with an asynchronous device-to-host copy on the caller's
 // stream -- no synchronisation; the next calls read whatever has arrived (one or two calls old).  It only selects
 // between kernels that are both correct for every input.
-#ifndef TCAMCRF_DENSITY_HINT
-#define TCAMCRF_DENSITY_HINT 1
-#endif
-struct DensityHints {
-    struct Slot {
-        void *ws;
-        int *word;            // pinned
-        unsigned int calls;   // calls seen on this workspace
-    };
-    std::mutex mu;
-    std::vector<Slot> slots;   // a handful of workspaces per process
-    cudaStream_t side = nullptr;                   // the copies run here, off the caller's stream
-    cudaEvent_t ev = nullptr;
-    // caller holds `mu`
-    Slot *find(void *ws, bool create)
-    {
-        for (auto &s : slots)
-            if (s.ws == ws) return &s;
-        if (!create) return nullptr;
-        int *p = nullptr;
-        if (cudaHostAlloc((void **)&p, sizeof(int), cudaHostAllocDefault) != cudaSuccess) {
-            cudaGetLastError();
-            return nullptr;
-        }
-        *p = 0;
-        slots.push_back({ws, p, 0u});
-        return &slots.back();
-    }
-};
-// Process-level helpers (density hints, the copy lane of the host-frames path, the host-pointer context) exist once
-// PER DEVICE: a process that drives several GPUs (threads of DataParallel, or alternating cuda:0 / cuda:1) gets
-// separate streams, events and buffers for each, and nothing is re-created or leaked on a device switch.
-constexpr int kMaxDevices = 64;
-static int current_device_slot()
-{
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) {
-        cudaGetLastError();
-        dev = 0;
-    }
-    return (dev >= 0 && dev < kMaxDevices) ? dev : 0;
-}
-static DensityHints g_hints_dev[kMaxDevices];
-
 static bool stream_is_capturing(cudaStream_t st)
 {
     cudaStreamCaptureStatus status = cudaStreamCaptureStatusNone;
@@ -1911,48 +1991,46 @@ static bool stream_is_capturing(cudaStream_t st)
 }
 
 // largest per-frame vertex count seen lately on this workspace (0: unknown)
-static int density_hint(void *ws)
+static int density_hint(Device &dev, void *ws)
 {
     if (!TCAMCRF_DENSITY_HINT) return 0;
-    DensityHints &g_hints = g_hints_dev[current_device_slot()];
-    std::lock_guard<std::mutex> lock(g_hints.mu);
-    DensityHints::Slot *slot = g_hints.find(ws, false);
+    std::lock_guard<std::mutex> lock(dev.hints.mu);
+    DensityHints::Slot *slot = dev.hints.find(ws, false);
     return slot ? *(volatile int *)slot->word : 0;
 }
 
 // Queue the refresh of the hint behind the work already on `st`, on a side stream: the caller's stream never waits
 // for the copy (in-stream it costs ~5 us per call, more than the hint is worth on short steps).  Nothing is done
 // while a graph is being captured (an unjoined fork is not capturable; the hint then keeps its last value).
-static void density_hint_refresh(const Plan &pl, char *ws, cudaStream_t st)
+static void density_hint_refresh(Device &dev, const Plan &pl, char *ws, cudaStream_t st)
 {
     if (!TCAMCRF_DENSITY_HINT) return;
     if (stream_is_capturing(st)) return;   // (also: no pinned allocation while a capture is open)
-    DensityHints &g_hints = g_hints_dev[current_device_slot()];
-    std::lock_guard<std::mutex> lock(g_hints.mu);
-    DensityHints::Slot *slot = g_hints.find(ws, true);
+    std::lock_guard<std::mutex> lock(dev.hints.mu);
+    DensityHints::Slot *slot = dev.hints.find(ws, true);
     if (!slot) return;
     // every 8th call is plenty for a hint (the three driver calls below cost ~10 us of host time, which shows on
     // 0.25 ms steps); the first two calls on a workspace always refresh
     const unsigned int c = slot->calls++;
     if (c >= 2 && (c & 7u) != 0) return;
-    if (!g_hints.side) {   // this device's side stream, created on first use
-        if (cudaStreamCreateWithFlags(&g_hints.side, cudaStreamNonBlocking) != cudaSuccess ||
-            cudaEventCreateWithFlags(&g_hints.ev, cudaEventDisableTiming) != cudaSuccess) {
+    if (!dev.hints.side) {   // this device's side stream, created on first use
+        if (cudaStreamCreateWithFlags(&dev.hints.side, cudaStreamNonBlocking) != cudaSuccess ||
+            cudaEventCreateWithFlags(&dev.hints.ev, cudaEventDisableTiming) != cudaSuccess) {
             cudaGetLastError();
-            g_hints.side = nullptr;
+            dev.hints.side = nullptr;
             return;
         }
     }
-    cudaEventRecord(g_hints.ev, st);
-    cudaStreamWaitEvent(g_hints.side, g_hints.ev, 0);
+    cudaEventRecord(dev.hints.ev, st);
+    cudaStreamWaitEvent(dev.hints.side, dev.hints.ev, 0);
     cudaMemcpyAsync(slot->word, ws + pl.off_ctrl + kCtrlPrevMax * sizeof(int), sizeof(int), cudaMemcpyDeviceToHost,
-                    g_hints.side);
+                    dev.hints.side);
 }
 
 // Stage 2: splat -> blur x(d+1) -> slice (+ loss) for the frames [frame0, frame0 + nc) of a chunk whose lattice
 // is built.  segs / as_out point at frame0.  `zero_values`: the value rows were not cleared by lattice_stages.
 template <int D>
-static int value_stages(const Plan &pl, const float *segs, float *as_out, int frame0, int nc, char *ws,
+static int value_stages(Device &dev, const Plan &pl, const float *segs, float *as_out, int frame0, int nc, char *ws,
                         bool zero_values, bool want_loss, float *loss_final, float n_norm, int flags, cudaStream_t st)
 {
     int *ctrl = (int *)(ws + pl.off_ctrl);
@@ -1971,7 +2049,7 @@ static int value_stages(const Plan &pl, const float *segs, float *as_out, int fr
         vp.frame0 = frame0;
         vp.zero_values = 1;
         StageScope scope(kStSplat, 1, st);
-        vertex_init_kernel<<<resident_grid(vertex_init_kernel), kThreads, 0, st>>>(vp, nc);
+        vertex_init_kernel<<<resident_grid(dev, vertex_init_kernel), kThreads, 0, st>>>(vp, nc);
     }
     const dim3 pgrid(pl.blocks_per_frame, nc);
     const int V = (pl.Kp % 4 == 0) ? 4 : (pl.Kp % 2 == 0) ? 2 : 1;
@@ -1994,7 +2072,7 @@ static int value_stages(const Plan &pl, const float *segs, float *as_out, int fr
     pp.Kp = pl.Kp;
     pp.frame0 = frame0;
     // dense lattice lately (more than one vertex per four pixels in the fullest frame): row-cooperative splat
-    pp.dense = lattice_is_dense(density_hint(ws), pl.P) ? 1 : 0;
+    pp.dense = lattice_is_dense(density_hint(dev, ws), pl.P) ? 1 : 0;
     if (tuning().dense >= 0) pp.dense = tuning().dense != 0;   // tests and sweeps: force either way
     pp.pool = pl.pool;
     pp.alpha = 1.0f / (1 + powf(2, -D));
@@ -2017,7 +2095,7 @@ static int value_stages(const Plan &pl, const float *segs, float *as_out, int fr
             bl.Kp = pl.Kp;
             bl.stride = pl.stride;
             bl.frame0 = frame0;
-            launch_blur(V, bl, nc, st);
+            launch_blur(dev, V, bl, nc, st);
             float *t = src;
             src = dst;
             dst = t;
@@ -2045,27 +2123,27 @@ static int value_stages(const Plan &pl, const float *segs, float *as_out, int fr
     return fail(TCAMCRF_ERR_INVALID, "unsupported lattice dimension %d", dim)
 
 // `images` points at frame 0 of the chunk; the lattice of frames [frame0, frame0 + nc) is built.
-static int run_lattice(const tcamcrf_config *cfg, const Plan &pl, bool u8, const void *images, int frame0, int nc,
-                       char *ws, bool zero_values, cudaStream_t st)
+static int run_lattice(Device &dev, const tcamcrf_config *cfg, const Plan &pl, bool u8, const void *images, int frame0,
+                       int nc, char *ws, bool zero_values, cudaStream_t st)
 {
-    TCAMCRF_DISPATCH_D(pl.D, lattice_stages<D>(cfg, pl, u8, images, frame0, nc, ws, zero_values, st));
+    TCAMCRF_DISPATCH_D(pl.D, lattice_stages<D>(dev, cfg, pl, u8, images, frame0, nc, ws, zero_values, st));
 }
 
-static int run_values(const Plan &pl, const float *segs, float *as_out, int frame0, int nc, char *ws,
+static int run_values(Device &dev, const Plan &pl, const float *segs, float *as_out, int frame0, int nc, char *ws,
                       bool zero_values, bool want_loss, float *loss_final, float n_norm, int flags, cudaStream_t st)
 {
-    TCAMCRF_DISPATCH_D(pl.D, value_stages<D>(pl, segs, as_out, frame0, nc, ws, zero_values, want_loss, loss_final,
+    TCAMCRF_DISPATCH_D(pl.D, value_stages<D>(dev, pl, segs, as_out, frame0, nc, ws, zero_values, want_loss, loss_final,
                                              n_norm, flags, st));
 }
 
-static int run_chunk(const tcamcrf_config *cfg, const Plan &pl, bool u8, const void *images, const float *segs,
-                     float *as_out, int nc, char *ws, bool want_loss, float *loss_final, float n_norm,
-                     int flags, cudaStream_t st)
+static int run_chunk(Device &dev, const tcamcrf_config *cfg, const Plan &pl, bool u8, const void *images,
+                     const float *segs, float *as_out, int nc, char *ws, bool want_loss, float *loss_final,
+                     float n_norm, int flags, cudaStream_t st)
 {
-    int rc = run_lattice(cfg, pl, u8, images, 0, nc, ws, true, st);
+    int rc = run_lattice(dev, cfg, pl, u8, images, 0, nc, ws, true, st);
     if (rc) return rc;
-    rc = run_values(pl, segs, as_out, 0, nc, ws, false, want_loss, loss_final, n_norm, flags, st);
-    density_hint_refresh(pl, ws, st);
+    rc = run_values(dev, pl, segs, as_out, 0, nc, ws, false, want_loss, loss_final, n_norm, flags, st);
+    density_hint_refresh(dev, pl, ws, st);
     return rc;
 }
 
@@ -2074,34 +2152,9 @@ static int run_chunk(const tcamcrf_config *cfg, const Plan &pl, bool u8, const v
 // library while the lattice of the sections that have arrived is being built on the caller's stream, instead of
 // one copy followed by one build.  Fork/join with events only: nothing synchronises, and the pattern can be
 // captured in a CUDA graph (pinned source).
-struct CopyLane {
-    std::mutex mu;
-    cudaStream_t stream = nullptr;
-    std::vector<cudaEvent_t> events;
-    size_t next = 0;
-    int ready()   // this device's copy stream, created on first use
-    {
-        if (stream) return TCAMCRF_OK;
-        CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
-        return TCAMCRF_OK;
-    }
-    int event(cudaEvent_t *ev)
-    {
-        if (events.size() < 64) {
-            cudaEvent_t e = nullptr;
-            CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-            events.push_back(e);
-            *ev = e;
-            return TCAMCRF_OK;
-        }
-        *ev = events[next++ % events.size()];   // a waiter keeps the record it was given: re-recording is safe
-        return TCAMCRF_OK;
-    }
-};
-static CopyLane g_lane_dev[kMaxDevices];
-
+//
 // One chunk whose frames come from the host: `img_host` / `img_dev` point at frame 0 of the chunk.
-static int run_chunk_host_frames(const tcamcrf_config *cfg, const Plan &pl, bool u8, const char *img_host,
+static int run_chunk_host_frames(Device &dev, const tcamcrf_config *cfg, const Plan &pl, bool u8, const char *img_host,
                                  char *img_dev, const float *segs, float *as_out, int nc, bool first_chunk,
                                  bool last_chunk, char *ws, bool want_loss, float *loss_final, float n_norm, int flags,
                                  cudaStream_t st)
@@ -2113,18 +2166,17 @@ static int run_chunk_host_frames(const tcamcrf_config *cfg, const Plan &pl, bool
     if (per < 4) per = nc < 4 ? nc : 4;
     const size_t elem = u8 ? 1 : sizeof(float);
     const size_t frame = (size_t)cfg->image_stride_planes * pl.P;   // elements per image
-    CopyLane &g_lane = g_lane_dev[current_device_slot()];
-    std::lock_guard<std::mutex> lock(g_lane.mu);
-    int rc = g_lane.ready();
+    std::lock_guard<std::mutex> lock(dev.lane.mu);
+    int rc = dev.lane.ready();
     if (rc) return rc;
     cudaEvent_t ev;
     if (first_chunk) {
         // the staging buffer may still be read by work queued earlier on the caller's stream; later chunks of the
         // call use other parts of it, and their copies simply queue behind the first chunk's on the copy stream
-        rc = g_lane.event(&ev);
+        rc = dev.lane.event(&ev);
         if (rc) return rc;
         CUDA_TRY(cudaEventRecord(ev, st));
-        CUDA_TRY(cudaStreamWaitEvent(g_lane.stream, ev, 0));
+        CUDA_TRY(cudaStreamWaitEvent(dev.lane.stream, ev, 0));
     }
     for (int f0 = 0; f0 < nc; f0 += per) {
         const int fn = nc - f0 < per ? nc - f0 : per;
@@ -2132,16 +2184,16 @@ static int run_chunk_host_frames(const tcamcrf_config *cfg, const Plan &pl, bool
         // the very last image of the batch may be shorter than the stride (see host_run)
         if (last_chunk && f0 + fn == nc) elems = ((size_t)(fn - 1) * cfg->image_stride_planes + cfg->channels) * pl.P;
         CUDA_TRY(cudaMemcpyAsync(img_dev + (size_t)f0 * frame * elem, img_host + (size_t)f0 * frame * elem, elems * elem,
-                                 cudaMemcpyHostToDevice, g_lane.stream));
-        rc = g_lane.event(&ev);
+                                 cudaMemcpyHostToDevice, dev.lane.stream));
+        rc = dev.lane.event(&ev);
         if (rc) return rc;
-        CUDA_TRY(cudaEventRecord(ev, g_lane.stream));
+        CUDA_TRY(cudaEventRecord(ev, dev.lane.stream));
         CUDA_TRY(cudaStreamWaitEvent(st, ev, 0));
-        rc = run_lattice(cfg, pl, u8, img_dev, f0, fn, ws, true, st);
+        rc = run_lattice(dev, cfg, pl, u8, img_dev, f0, fn, ws, true, st);
         if (rc) return rc;
     }
-    rc = run_values(pl, segs, as_out, 0, nc, ws, false, want_loss, loss_final, n_norm, flags, st);
-    density_hint_refresh(pl, ws, st);
+    rc = run_values(dev, pl, segs, as_out, 0, nc, ws, false, want_loss, loss_final, n_norm, flags, st);
+    density_hint_refresh(dev, pl, ws, st);
     return rc;
 }
 
@@ -2160,6 +2212,9 @@ static int run_filter(const tcamcrf_config *cfg, bool u8, const void *images, co
     if (((uintptr_t)workspace & 255) != 0) return fail(TCAMCRF_ERR_WORKSPACE, "workspace must be 256-byte aligned");
     if (((uintptr_t)segs & 3) || ((uintptr_t)as_out & 3) || (!u8 && ((uintptr_t)images & 3)))
         return fail(TCAMCRF_ERR_INVALID, "float buffers must be 4-byte aligned");
+    Device *dev = nullptr;
+    rc = this_device(&dev);
+    if (rc) return rc;
     char *ws = (char *)workspace;
     // status word + loss accumulator start clean for this call (MAGIC / DIRTY persist with the workspace)
     CUDA_TRY(cudaMemsetAsync(ws + pl.off_ctrl, 0, kCtrlResetInts * sizeof(int), st));
@@ -2169,13 +2224,13 @@ static int run_filter(const tcamcrf_config *cfg, bool u8, const void *images, co
         const char *img = (const char *)images + (size_t)n0 * cfg->image_stride_planes * pl.P * img_elem;
         const bool last = n0 + nc >= N;
         if (images_host)
-            rc = run_chunk_host_frames(cfg, pl, u8,
+            rc = run_chunk_host_frames(*dev, cfg, pl, u8,
                                        (const char *)images_host + (size_t)n0 * cfg->image_stride_planes * pl.P * img_elem,
                                        const_cast<char *>(img), segs + (size_t)n0 * K * pl.P,
                                        as_out + (size_t)n0 * K * pl.P, nc, n0 == 0, last, ws, loss != nullptr,
                                        last ? loss : nullptr, n_norm, flags, st);
         else
-            rc = run_chunk(cfg, pl, u8, img, segs + (size_t)n0 * K * pl.P, as_out + (size_t)n0 * K * pl.P, nc, ws,
+            rc = run_chunk(*dev, cfg, pl, u8, img, segs + (size_t)n0 * K * pl.P, as_out + (size_t)n0 * K * pl.P, nc, ws,
                            loss != nullptr, last ? loss : nullptr, n_norm, flags, st);
         if (rc) return rc;
     }
@@ -2185,19 +2240,6 @@ static int run_filter(const tcamcrf_config *cfg, bool u8, const void *images, co
 // ---------------------------------------------------------------------------
 // host-pointer (drop-in) path: cached device buffers, chunk-pipelined copies
 // ---------------------------------------------------------------------------
-struct HostCtx {
-    std::mutex mu;
-    void *buf = nullptr;
-    size_t cap = 0;
-    cudaStream_t stream = nullptr;   // compute
-    cudaStream_t s_in = nullptr;     // host -> device copies
-    cudaStream_t s_out = nullptr;    // device -> host copies
-    std::vector<cudaEvent_t> events;
-    void *pin = nullptr;             // pinned staging: grad_out in, per-group losses and status words out
-    size_t pin_cap = 0;
-};
-static HostCtx g_host_dev[kMaxDevices];
-
 static int host_pin_reserve(HostCtx &g_host, size_t bytes)
 {
     if (g_host.pin_cap >= bytes) return TCAMCRF_OK;
@@ -2300,7 +2342,7 @@ static int check_device()
 //
 // One call is ~200 driver calls (copies, events, ~130 launches): about as long on the CPU as the link needs for the
 // bytes.  With pinned buffers the whole schedule is therefore captured ONCE into a CUDA graph, keyed by the problem
-// and the buffer addresses, and a call is one graph launch (HostGraphs below).
+// and the buffer addresses, and a call is one graph launch (HostGraphs).
 struct HostJob {
     tcamcrf_config cfg;
     Plan pl;
@@ -2336,8 +2378,9 @@ static void host_groups(int frames, int equal_size, int taper, std::vector<int> 
 
 // Queues the whole call on the three streams.  `st` is the origin: s_in / s_out fork from it and join it again, so
 // the same code runs eagerly or under stream capture.  `groups_out`: number of groups (entries of h_loss / h_status).
-static int host_enqueue(HostCtx &g_host, const HostJob &j, HostTrace &trace, int *groups_out)
+static int host_enqueue(Device &dev, const HostJob &j, HostTrace &trace, int *groups_out)
 {
+    HostCtx &g_host = dev.host;
     const Plan &pl = j.pl;
     const int N = j.N, K = j.K;
     cudaStream_t st = g_host.stream, s_in = g_host.s_in, s_out = g_host.s_out;
@@ -2396,7 +2439,7 @@ static int host_enqueue(HostCtx &g_host, const HostJob &j, HostTrace &trace, int
             CUDA_TRY(cudaEventRecord(ev_img, s_in));
             trace.mark("images in", c0 + f0, s_in);
             CUDA_TRY(cudaStreamWaitEvent(st, ev_img, 0));
-            rc = run_lattice(&j.cfg, pl, false, j.d_img + (size_t)c0 * img_frame, f0, fn, j.d_ws, false, st);
+            rc = run_lattice(dev, &j.cfg, pl, false, j.d_img + (size_t)c0 * img_frame, f0, fn, j.d_ws, false, st);
             if (rc) return rc;
             trace.mark("lattice", c0 + f0, st);
             host_groups(fn, group, taper, sizes);
@@ -2418,15 +2461,15 @@ static int host_enqueue(HostCtx &g_host, const HostJob &j, HostTrace &trace, int
                 CUDA_TRY(cudaStreamWaitEvent(st, ev_in, 0));
                 // every group reports its own share of the loss (already divided by the full batch size N)
                 CUDA_TRY(cudaMemsetAsync(j.d_ws + pl.off_acc, 0, sizeof(double), st));
-                rc = run_values(pl, j.d_seg + n0 * seg_frame, j.d_as + n0 * seg_frame, g0, nc, j.d_ws, true, j.want_loss,
-                                j.want_loss ? j.d_loss + gi : nullptr, (float)N, 0, st);
+                rc = run_values(dev, pl, j.d_seg + n0 * seg_frame, j.d_as + n0 * seg_frame, g0, nc, j.d_ws, true,
+                                j.want_loss, j.want_loss ? j.d_loss + gi : nullptr, (float)N, 0, st);
                 if (rc) return rc;
                 CUDA_TRY(cudaMemcpyAsync(j.d_status + gi, j.d_ws + pl.off_ctrl, sizeof(int), cudaMemcpyDeviceToDevice, st));
                 if (j.grad_host) {
                     StageScope scope(kStBackward, 1, st);
                     const size_t count = (size_t)nc * seg_frame;
                     size_t blocks = (count / 4 + kThreads - 1) / kThreads;
-                    if (blocks > (size_t)sm_count() * 8) blocks = (size_t)sm_count() * 8;
+                    if (blocks > (size_t)persistent_grid(dev)) blocks = (size_t)persistent_grid(dev);
                     if (blocks < 1) blocks = 1;
                     loss_backward_kernel<<<(unsigned)blocks, kThreads, 0, st>>>(j.d_as + n0 * seg_frame, j.d_scal,
                                                                                 j.d_grad + n0 * seg_frame, count, (float)N,
@@ -2463,32 +2506,6 @@ static int host_enqueue(HostCtx &g_host, const HostJob &j, HostTrace &trace, int
     return TCAMCRF_OK;
 }
 
-// Captured schedules of host_run, a handful per device (a trainer alternates between a few pinned buffers).
-struct HostGraphs {
-    struct Key {
-        tcamcrf_config cfg;
-        int N, K, H, W;
-        const void *images, *segs, *as_host, *grad_host, *buf, *pin;
-        int want_loss, dedup, dense, groups_knob, taper_knob, sec0_knob, grow_knob;
-        bool operator==(const Key &o) const { return memcmp(this, &o, sizeof(Key)) == 0; }
-    };
-    struct Item {
-        Key key;
-        cudaGraphExec_t exec;
-        int groups;
-        long long launches;      // kernels of one replay (for tcamcrf_launch_count)
-        unsigned long long used;
-    };
-    std::vector<Item> items;
-    unsigned long long tick = 0;
-    void clear()
-    {
-        for (auto &it : items) cudaGraphExecDestroy(it.exec);
-        items.clear();
-    }
-};
-static HostGraphs g_host_graphs[kMaxDevices];
-
 static bool host_pinned(const void *p)
 {
     if (!p) return true;
@@ -2512,9 +2529,11 @@ static int host_run(const tcamcrf_config *cfg_in, const float *images, const flo
     rc = make_plan(&j.cfg, N, K, H, W, j.pl);
     if (rc) return rc;
     const Plan &pl = j.pl;
-    const int dev = current_device_slot();
-    HostCtx &g_host = g_host_dev[dev];
-    HostGraphs &graphs = g_host_graphs[dev];
+    Device *dev = nullptr;
+    rc = this_device(&dev);
+    if (rc) return rc;
+    HostCtx &g_host = dev->host;
+    HostGraphs &graphs = dev->graphs;
     std::lock_guard<std::mutex> lock(g_host.mu);
     const int ngroups = N + 8;   // upper bound: a group holds at least one frame
     const size_t P = (size_t)H * W;
@@ -2553,7 +2572,7 @@ static int host_run(const tcamcrf_config *cfg_in, const float *images, const flo
     j.h_loss = j.h_gout + 1;
     j.h_status = (int *)(j.h_loss + ngroups);
     j.max_groups = ngroups;
-    const int hint = density_hint(j.d_ws);
+    const int hint = density_hint(*dev, j.d_ws);
     j.dedup_hint = !lattice_is_dense(hint, pl.P);
     j.dense_hint = lattice_is_dense(hint, pl.P);
     *j.h_gout = grad_out;
@@ -2586,11 +2605,11 @@ static int host_run(const tcamcrf_config *cfg_in, const float *images, const flo
         g_prof.total_launches += hit->launches;
     } else {
         trace.begin(g_host.s_in);
-        rc = host_enqueue(g_host, j, trace, &gi);
+        rc = host_enqueue(*dev, j, trace, &gi);
         if (rc) return rc;
         trace.host_mark("enqueued");
     }
-    density_hint_refresh(pl, j.d_ws, st);
+    density_hint_refresh(*dev, pl, j.d_ws, st);
     CUDA_TRY(cudaStreamSynchronize(st));
     trace.host_mark("synced");
     trace.end();
@@ -2620,7 +2639,7 @@ static int host_run(const tcamcrf_config *cfg_in, const float *images, const flo
         int groups = 0;
         if (cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal) == cudaSuccess) {
             HostTrace off;
-            const int crc = host_enqueue(g_host, j, off, &groups);
+            const int crc = host_enqueue(*dev, j, off, &groups);
             const cudaError_t ce = cudaStreamEndCapture(st, &graph);
             cudaGraphExec_t exec = nullptr;
             if (!crc && ce == cudaSuccess && graph && cudaGraphInstantiate(&exec, graph, 0) == cudaSuccess) {
@@ -2722,9 +2741,10 @@ int tcamcrf_filter_transposed(const tcamcrf_config *cfg, const void *images_dev,
                       workspace_bytes, (cudaStream_t)cuda_stream, kFlagReverseBlur);
 }
 
-// Checks shared by the two lattice entry points; the plan must describe ONE chunk holding all N frames.
+// Checks shared by the two lattice entry points (the plan must describe ONE chunk holding all N frames), and the
+// current device's context.
 static int lattice_plan(const tcamcrf_config *cfg, int N, int K, int H, int W, void *workspace, size_t ws_bytes,
-                        Plan &pl)
+                        Plan &pl, Device **dev)
 {
     if (!cfg || !workspace) return fail(TCAMCRF_ERR_INVALID, "null pointer argument");
     int rc = make_plan(cfg, N, K, H, W, pl);
@@ -2734,7 +2754,7 @@ static int lattice_plan(const tcamcrf_config *cfg, int N, int K, int H, int W, v
     if (ws_bytes < pl.total)
         return fail(TCAMCRF_ERR_WORKSPACE, "workspace too small: %zu < %zu bytes", ws_bytes, pl.total);
     if (((uintptr_t)workspace & 255) != 0) return fail(TCAMCRF_ERR_WORKSPACE, "workspace must be 256-byte aligned");
-    return TCAMCRF_OK;
+    return this_device(dev);
 }
 
 int tcamcrf_key_range_ok(const tcamcrf_config *cfg, int H, int W, float max_value)
@@ -2774,11 +2794,12 @@ int tcamcrf_lattice_build(const tcamcrf_config *cfg, const void *images_dev, int
 {
     if (!images_dev) return fail(TCAMCRF_ERR_INVALID, "null pointer argument");
     Plan pl;
-    int rc = lattice_plan(cfg, N, K, H, W, workspace, workspace_bytes, pl);
+    Device *dev = nullptr;
+    int rc = lattice_plan(cfg, N, K, H, W, workspace, workspace_bytes, pl, &dev);
     if (rc) return rc;
     cudaStream_t st = (cudaStream_t)cuda_stream;
     CUDA_TRY(cudaMemsetAsync((char *)workspace + pl.off_ctrl, 0, kCtrlResetInts * sizeof(int), st));
-    return run_lattice(cfg, pl, images_u8 != 0, images_dev, 0, N, (char *)workspace, false, st);
+    return run_lattice(*dev, cfg, pl, images_u8 != 0, images_dev, 0, N, (char *)workspace, false, st);
 }
 
 int tcamcrf_lattice_apply(const tcamcrf_config *cfg, const float *segs_dev, float *out_dev, float *loss_dev, int N,
@@ -2787,14 +2808,15 @@ int tcamcrf_lattice_apply(const tcamcrf_config *cfg, const float *segs_dev, floa
 {
     if (!segs_dev || !out_dev) return fail(TCAMCRF_ERR_INVALID, "null pointer argument");
     Plan pl;
-    int rc = lattice_plan(cfg, N, K, H, W, workspace, workspace_bytes, pl);
+    Device *dev = nullptr;
+    int rc = lattice_plan(cfg, N, K, H, W, workspace, workspace_bytes, pl, &dev);
     if (rc) return rc;
     if (((uintptr_t)segs_dev & 3) || ((uintptr_t)out_dev & 3))
         return fail(TCAMCRF_ERR_INVALID, "float buffers must be 4-byte aligned");
     cudaStream_t st = (cudaStream_t)cuda_stream;
     // the loss accumulator starts at zero; the status word of the build is kept (a poisoned lattice stays poisoned)
     if (loss_dev) CUDA_TRY(cudaMemsetAsync((char *)workspace + pl.off_acc, 0, sizeof(double), st));
-    return run_values(pl, segs_dev, out_dev, 0, N, (char *)workspace, true, loss_dev != nullptr, loss_dev, n_norm,
+    return run_values(*dev, pl, segs_dev, out_dev, 0, N, (char *)workspace, true, loss_dev != nullptr, loss_dev, n_norm,
                       transposed ? kFlagReverseBlur : 0, st);
 }
 
@@ -2862,10 +2884,11 @@ int tcamcrf_loss_backward_logits_weighted(const float *as_dev, const float *logi
     if (!as_dev || !logits_dev || !grad_out_dev || !grad_logits_dev)
         return fail(TCAMCRF_ERR_INVALID, "null pointer argument");
     if (N < 1 || K < 2 || H < 1 || W < 1) return fail(TCAMCRF_ERR_INVALID, "N,H,W must be positive and K >= 2");
+    Device *dev = nullptr;
+    if (const int rc = this_device(&dev)) return rc;
     const long long pixels = (long long)N * H * W;
     long long blocks = (pixels + kThreads - 1) / kThreads;
-    const long long cap = (long long)sm_count() * 8;
-    if (blocks > cap) blocks = cap;
+    if (blocks > persistent_grid(*dev)) blocks = persistent_grid(*dev);
     StageScope scope(kStBackward, 1, (cudaStream_t)cuda_stream);
     loss_backward_logits_kernel<<<(unsigned)blocks, kThreads, 0, (cudaStream_t)cuda_stream>>>(
         as_dev, logits_dev, grad_out_dev, grad_logits_dev, K, H * W, pixels, n_norm, weight);
@@ -2886,9 +2909,10 @@ int tcamcrf_loss_backward_weighted(const float *as_dev, const float *grad_out_de
     if (count == 0) return TCAMCRF_OK;
     if (((uintptr_t)as_dev & 3) || ((uintptr_t)grad_seg_dev & 3))
         return fail(TCAMCRF_ERR_INVALID, "buffers must be 4-byte aligned");
+    Device *dev = nullptr;
+    if (const int rc = this_device(&dev)) return rc;
     size_t blocks = (count / 4 + kThreads - 1) / kThreads;
-    const size_t cap = (size_t)sm_count() * 8;
-    if (blocks > cap) blocks = cap;
+    if (blocks > (size_t)persistent_grid(*dev)) blocks = persistent_grid(*dev);
     if (blocks < 1) blocks = 1;
     StageScope scope(kStBackward, 1, (cudaStream_t)cuda_stream);
     loss_backward_kernel<<<(unsigned)blocks, kThreads, 0, (cudaStream_t)cuda_stream>>>(as_dev, grad_out_dev,
@@ -2923,7 +2947,10 @@ int tcamcrf_debug_lattice(const tcamcrf_config *cfg, const float *image_host, in
     if (rc) return rc;
     const size_t P = (size_t)H * W;
     const int dp1 = pl.D + 1;
-    HostCtx &g_host = g_host_dev[current_device_slot()];
+    Device *dev = nullptr;
+    rc = this_device(&dev);
+    if (rc) return rc;
+    HostCtx &g_host = dev->host;
     std::lock_guard<std::mutex> lock(g_host.mu);
     const size_t img_bytes = align_up((size_t)c.channels * P * sizeof(float), 256);
     const size_t seg_bytes = align_up(P * sizeof(float), 256);
@@ -3061,8 +3088,8 @@ int tcamcrf_profile_read(double *ms, long long *launches, int reset)
             g_prof.ms[sp.stage] += t;
             g_prof.launches[sp.stage] += sp.launches;
         }
-        g_prof.pool.push_back(sp.a);
-        g_prof.pool.push_back(sp.b);
+        sp.dev->timing_events.push_back(sp.a);
+        sp.dev->timing_events.push_back(sp.b);
     }
     g_prof.spans.clear();
     for (int i = 0; i < kStCount; i++) {
@@ -3090,6 +3117,8 @@ int tcam_seed_select(const float *cams_dev, int T, const int64_t *roi_dev, const
         return fail(TCAMCRF_ERR_INVALID, "null pointer argument");
     if (B < 1 || T < 1 || HW < 1 || kmax < 1 || k_fg < 0 || k_bg < 0)
         return fail(TCAMCRF_ERR_INVALID, "B,T,HW,kmax must be positive and k_fg,k_bg non-negative");
+    Device *dev = nullptr;
+    if (const int rc = this_device(&dev)) return rc;
     SeedParams sp;
     sp.cams = cams_dev;
     sp.roi = reinterpret_cast<const long long *>(roi_dev);
@@ -3109,21 +3138,7 @@ int tcam_seed_select(const float *cams_dev, int T, const int64_t *roi_dev, const
         StageScope scope(kStSeed, 1, (cudaStream_t)cuda_stream);
         // keys of a sample in shared memory when the frame fits (4 bytes per pixel of the 227 KB an SM has)
         const size_t smem = (size_t)HW * sizeof(unsigned int);
-        static int smem_limit = -1;   // 0: the opt-in was refused
-        if (smem_limit < 0) {
-            int dev = 0, optin = 0;
-            cudaGetDevice(&dev);
-            cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-            optin -= 2048;   // the kernel's static shared memory
-            if (optin > 0 && cudaFuncSetAttribute(seed_select_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                  optin) == cudaSuccess)
-                smem_limit = optin;
-            else {
-                cudaGetLastError();
-                smem_limit = 0;
-            }
-        }
-        if (TCAMCRF_SEED_SMEM && smem <= (size_t)smem_limit)
+        if (TCAMCRF_SEED_SMEM && smem <= (size_t)dev->select_smem)
             seed_select_smem_kernel<<<dim3(2, B), kSeedThreads, smem, (cudaStream_t)cuda_stream>>>(sp);
         else
             seed_select_kernel<<<dim3(2, B), kSeedThreads, 0, (cudaStream_t)cuda_stream>>>(sp);
@@ -3132,35 +3147,14 @@ int tcam_seed_select(const float *cams_dev, int T, const int64_t *roi_dev, const
     return TCAMCRF_OK;
 }
 
-// Largest dynamic shared memory seed_fused_kernel may use on this device (0: the opt-in was refused).
-static int seed_fused_smem_limit()
-{
-    static int limit = -1;
-    if (limit < 0) {
-        int dev = 0, optin = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-        cudaFuncAttributes fa;
-        int stat = 12 * 1024;
-        if (cudaFuncGetAttributes(&fa, seed_fused_kernel) == cudaSuccess) stat = (int)fa.sharedSizeBytes;
-        optin -= stat + 1024;
-        if (optin > 0 && cudaFuncSetAttribute(seed_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, optin) ==
-                             cudaSuccess)
-            limit = optin;
-        else {
-            cudaGetLastError();
-            limit = 0;
-        }
-    }
-    return limit;
-}
-
 static int seed_fused_slice(int HW) { return ((HW + kSeedCluster - 1) / kSeedCluster + 3) / 4 * 4; }
 
 int tcam_seed_fused_supported(int HW, int kmax)
 {
     if (HW < 1 || kmax < 1 || kmax > kSeedFusedMaxK) return 0;
-    return (size_t)seed_fused_slice(HW) * 2 * sizeof(unsigned int) <= (size_t)seed_fused_smem_limit() ? 1 : 0;
+    Device *dev = nullptr;
+    if (this_device(&dev)) return 0;
+    return (size_t)seed_fused_slice(HW) * 2 * sizeof(unsigned int) <= (size_t)dev->fused_smem ? 1 : 0;
 }
 
 int tcam_seed_fused(const float *cams_dev, int T, const int64_t *roi_dev, const float *q_dev, const int *q_offset_dev,
@@ -3271,10 +3265,11 @@ int tcam_seed_labels(const int *sel_dev, int kmax, int B, int H, int W, int ksz,
 {
     if (!sel_dev || !out_dev) return fail(TCAMCRF_ERR_INVALID, "null pointer argument");
     if (B < 1 || H < 1 || W < 1 || kmax < 1 || ksz < 1) return fail(TCAMCRF_ERR_INVALID, "B,H,W,kmax,ksz must be positive");
+    Device *dev = nullptr;
+    if (const int rc = this_device(&dev)) return rc;
     const long long total = (long long)B * H * W;
     long long blocks = (total + 255) / 256;
-    const long long cap = (long long)sm_count() * 8;
-    if (blocks > cap) blocks = cap;
+    if (blocks > persistent_grid(*dev)) blocks = persistent_grid(*dev);
     {
         StageScope scope(kStSeed, 1, (cudaStream_t)cuda_stream);
         seed_labels_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)cuda_stream>>>(
@@ -3301,10 +3296,11 @@ int tcam_temporal_max(const float *cams_dev, float *out_dev, int B, int T, int H
 {
     if (!cams_dev || !out_dev) return fail(TCAMCRF_ERR_INVALID, "null pointer argument");
     if (B < 1 || T < 1 || HW < 1) return fail(TCAMCRF_ERR_INVALID, "B,T,HW must be positive");
+    Device *dev = nullptr;
+    if (const int rc = this_device(&dev)) return rc;
     const long long total = (long long)B * HW;
     long long blocks = (total + kThreads - 1) / kThreads;
-    const long long cap = (long long)sm_count() * 8;
-    if (blocks > cap) blocks = cap;
+    if (blocks > persistent_grid(*dev)) blocks = persistent_grid(*dev);
     StageScope scope(kStSeed, 1, (cudaStream_t)cuda_stream);
     temporal_max_kernel<<<(unsigned)blocks, kThreads, 0, (cudaStream_t)cuda_stream>>>(cams_dev, out_dev, T, HW, total);
     CUDA_TRY(cudaGetLastError());
@@ -3356,10 +3352,11 @@ int tcam_prepare_std_cams(const float *cams_dev, float *out_dev, int B, int h, i
 {
     if (!cams_dev || !out_dev) return fail(TCAMCRF_ERR_INVALID, "null pointer argument");
     if (B < 1 || h < 1 || w < 1 || H < 1 || W < 1) return fail(TCAMCRF_ERR_INVALID, "sizes must be positive");
+    Device *dev = nullptr;
+    if (const int rc = this_device(&dev)) return rc;
     const long long total = (long long)B * H * W;
     long long blocks = (total + 255) / 256;
-    const long long cap = (long long)sm_count() * 8;
-    if (blocks > cap) blocks = cap;
+    if (blocks > persistent_grid(*dev)) blocks = persistent_grid(*dev);
     StageScope scope(kStSeed, 1, (cudaStream_t)cuda_stream);
     // ATen: scale = (float)input_size / output_size when no scale factor is given (upsample with size=)
     prepare_std_cams_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)cuda_stream>>>(

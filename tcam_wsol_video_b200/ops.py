@@ -39,7 +39,9 @@ def _workspace(device: torch.device, nbytes: int) -> torch.Tensor:
 
 
 def release_workspaces() -> None:
+    """Drops the cached per-(device, stream) buffers: the CRF workspaces and the seed cross-entropy scratch."""
     _workspaces.clear()
+    _seed_ce_scratch.clear()
 
 
 def _prep_images(images: torch.Tensor, device: torch.device) -> Tuple[torch.Tensor, bool]:

@@ -217,28 +217,28 @@ class TCAMSeeder(nn.Module):
         b, t, h, w = cams.shape
         device = cams.device
         kmax = max(self.max_, self.min_, 1)
-        fused = bool(lib.tcam_seed_fused_supported(h * w, kmax))
-        n_fg_fixed = int(self.max_p * (h * w)) if self.max_ > 0 else 0       # tcam_seeding.py:515,519
-        n_bg = int(self.min_p * h * w) if self.min_ > 0 else 0                # tcam_seeding.py:567
-        rng = q = q_off = n_cand = None
-        if counts is None and fused:
-            # two words from torch's CUDA generator key the in-kernel Philox stream of this call
-            rng = torch.randint(0, 2 ** 31 - 1, (2,), dtype=torch.int32, device=device)
-        else:
-            if counts is None:
-                counts_t = self._candidate_counts_device(cams.amax(dim=1, keepdim=True) if t > 1 else cams, roi)
-                q = torch.empty(b * 2 * h * w, dtype=torch.float32, device=device).exponential_(1)
-                q_off = torch.arange(2 * b, dtype=torch.int32, device=device) * (h * w)
-                n_cand = counts_t.reshape(-1)
-            else:
-                q, offsets = self._draws(counts, device)
-                meta = torch.from_numpy(np.concatenate([offsets.reshape(-1), counts.reshape(-1)]).astype(np.int32)).to(device)
-                q_off, n_cand = meta[: 2 * b], meta[2 * b:]
-        cam_max = torch.empty((b, h, w), dtype=torch.float32, device=device)
-        sel = torch.empty((b, 2, kmax), dtype=torch.int32, device=device)
-        out = None if sparse else torch.empty((b, h, w), dtype=torch.long, device=device)
-        stream = torch.cuda.current_stream(device).cuda_stream
         with torch.cuda.device(device):
+            fused = bool(lib.tcam_seed_fused_supported(h * w, kmax))   # answers for the current device
+            n_fg_fixed = int(self.max_p * (h * w)) if self.max_ > 0 else 0       # tcam_seeding.py:515,519
+            n_bg = int(self.min_p * h * w) if self.min_ > 0 else 0                # tcam_seeding.py:567
+            rng = q = q_off = n_cand = None
+            if counts is None and fused:
+                # two words from torch's CUDA generator key the in-kernel Philox stream of this call
+                rng = torch.randint(0, 2 ** 31 - 1, (2,), dtype=torch.int32, device=device)
+            else:
+                if counts is None:
+                    counts_t = self._candidate_counts_device(cams.amax(dim=1, keepdim=True) if t > 1 else cams, roi)
+                    q = torch.empty(b * 2 * h * w, dtype=torch.float32, device=device).exponential_(1)
+                    q_off = torch.arange(2 * b, dtype=torch.int32, device=device) * (h * w)
+                    n_cand = counts_t.reshape(-1)
+                else:
+                    q, offsets = self._draws(counts, device)
+                    meta = torch.from_numpy(np.concatenate([offsets.reshape(-1), counts.reshape(-1)]).astype(np.int32)).to(device)
+                    q_off, n_cand = meta[: 2 * b], meta[2 * b:]
+            cam_max = torch.empty((b, h, w), dtype=torch.float32, device=device)
+            sel = torch.empty((b, 2, kmax), dtype=torch.int32, device=device)
+            out = None if sparse else torch.empty((b, h, w), dtype=torch.long, device=device)
+            stream = torch.cuda.current_stream(device).cuda_stream
             if fused:
                 _lib.check(lib.tcam_seed_fused(
                     cams.data_ptr(), t, roi.data_ptr() if roi is not None else None,

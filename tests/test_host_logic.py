@@ -272,6 +272,16 @@ def test_tuning_knobs_are_set_at_run_time():
         _lib.set_tuning("NO_SUCH_KNOB", 1)
 
 
+def test_release_workspaces_clears_every_cached_buffer():
+    """Both caches keyed by (device, stream, ...) are dropped: a trainer that changes streams or batch sizes can
+    release what it no longer uses."""
+    from tcam_wsol_video_b200 import ops
+    ops._workspaces[(0, 1)] = object()
+    ops._seed_ce_scratch[(0, 1, 4)] = object()
+    ops.release_workspaces()
+    assert not ops._workspaces and not ops._seed_ce_scratch
+
+
 def test_weight_is_folded_only_when_it_is_a_plain_number():
     import torch
     from tcam_wsol_video_b200.dense_crf_loss import _folded_weight
