@@ -193,6 +193,14 @@ int tcamcrf_workspace_status(void *workspace, void *cuda_stream, int *dev_status
 int tcamcrf_debug_lattice(const tcamcrf_config *cfg, const float *image_host, int H, int W, int32_t *offset_host,
                           float *bary_host, int *vertices, int32_t *nbr_host, size_t nbr_cap);
 
+/* Seeding introspection for tests: the random words and Exp(1) draws tcam_seed_fused makes without q_dev, through
+ * the same device functions.  tcam_debug_seed_draws: for every (b < B, side < 2, pixel < HW), the Philox4x32-10 word
+ * of counter (pixel, 2b + side, 0x5eed, 0) keyed by the two words at rng_dev, and its draw; words_dev / draws_dev
+ * [B,2,HW].  tcam_debug_exp_draws: the draw of each of the n words at words_dev. */
+int tcam_debug_seed_draws(const unsigned int *rng_dev, int B, int HW, unsigned int *words_dev, float *draws_dev,
+                          void *cuda_stream);
+int tcam_debug_exp_draws(const unsigned int *words_dev, int n, float *draws_dev, void *cuda_stream);
+
 /* ---- drop-in host API (reference names and argument lists) ---- */
 int bilateralfilter(float *image, int len_image, float *in, int len_in, float *out, int len_out, int H, int W,
                     float sigmargb, float sigmaxy);
@@ -278,7 +286,9 @@ int tcam_seed_labels(const int *sel_dev, int kmax, int B, int H, int W, int ksz,
  *     pixel index (stable sort); selected = top-k of p / q, p = value (weighted_fg) or 1;
  *   - q: the caller's Exp(1) draws in row-major candidate order (q_dev + q_offset_dev [B,2]: bit-identical to
  *     tcam_seed_select, i.e. to the reference's multinomial given the same stream), or, with q_dev == NULL, drawn in
- *     the kernel by Philox4x32-10 keyed with the two words at rng_dev (fresh per call, e.g. from torch's generator);
+ *     the kernel by Philox4x32-10 keyed with the two words at rng_dev (fresh per call, e.g. from torch's generator):
+ *     draw = -logf((2m + 1) * 2^-24), m = the top 23 bits of the word of (sample, side, pixel), so every draw is
+ *     finite and > 0 (tcam_debug_seed_draws returns them);
  *   - labels_dev [B,H,W] int64 (or NULL): flat ksz x ksz dilation of the seeds, conflicts -> ignore (:239-254).
  * sel_dev [B,2,kmax] pixel indices (-1 = unused).  tcam_seed_fused_supported: the slice of a frame (H*W/8 pixels,
  * 8 bytes each) must fit the shared memory of an SM and kmax <= 32; otherwise use tcam_seed_select + tcam_seed_labels.

@@ -65,7 +65,10 @@ def prepare_std_cams_disq(std_cams: torch.Tensor, image_size) -> torch.Tensor:
     return cams
 
 
-def sample_fg(cam, roi, fg, max_p, max_, seed_tech):
+def fg_candidates(cam, roi, max_p):
+    """The first half of _SFG.forward (tcam_seeding.py:498-530): (n, _cam, tmp) with n the number of candidates, _cam
+    the scores (cam*roi + 1e-8 or cam + 1e-8) and tmp [h,w] 1 at the n largest scores (stable sort: ties to the
+    lower pixel index), 0 elsewhere."""
     h, w = cam.shape
     if roi is not None:
         n = roi.sum()
@@ -77,10 +80,27 @@ def sample_fg(cam, roi, fg, max_p, max_, seed_tech):
     n = int(max_p * n)
     _cam_flatten = _cam.view(h * w)
     val, idx_ = torch.sort(_cam_flatten, dim=0, descending=True, stable=True)
+    tmp = _cam_flatten * 0.
+    tmp[idx_[:n]] = 1
+    return n, _cam, tmp.view(h, w)
+
+
+def bg_candidates(cam, min_p):
+    """The first half of _SBG.forward (tcam_seeding.py:555-580): (n, tmp) with tmp [h,w] 1 at the n smallest
+    cam + 1e-8 (stable sort), 0 elsewhere."""
+    h, w = cam.shape
+    n = int(min_p * h * w)
+    _cam = cam + 1e-8
+    _cam_flatten = _cam.view(h * w)
+    val, idx_ = torch.sort(_cam_flatten, dim=0, descending=False, stable=True)
+    tmp = _cam_flatten * 0.
+    tmp[idx_[:n]] = 1
+    return n, tmp.view(h, w)
+
+
+def sample_fg(cam, roi, fg, max_p, max_, seed_tech):
+    n, _cam, tmp = fg_candidates(cam, roi, max_p)
     if (n > 0) and (max_ > 0):
-        tmp = _cam_flatten * 0.
-        tmp[idx_[:n]] = 1
-        tmp = tmp.view(h, w)
         _idx = torch.nonzero(tmp, as_tuple=True)
         if seed_tech == SEED_UNIFORM:
             probs = torch.ones(n, dtype=torch.float, device=cam.device)
@@ -95,15 +115,8 @@ def sample_fg(cam, roi, fg, max_p, max_, seed_tech):
 
 
 def sample_bg(cam, bg, min_p, min_):
-    h, w = cam.shape
-    n = int(min_p * h * w)
-    _cam = cam + 1e-8
-    _cam_flatten = _cam.view(h * w)
-    val, idx_ = torch.sort(_cam_flatten, dim=0, descending=False, stable=True)
+    n, tmp = bg_candidates(cam, min_p)
     if (n > 0) and (min_ > 0):
-        tmp = _cam_flatten * 0.
-        tmp[idx_[:n]] = 1
-        tmp = tmp.view(h, w)
         _idx = torch.nonzero(tmp, as_tuple=True)
         probs = torch.ones(n, dtype=torch.float, device=cam.device)   # _SBG is always built with SEED_UNIFORM
         selected = probs.multinomial(num_samples=min(min_, n), replacement=False)

@@ -111,6 +111,8 @@ SIGNATURES = {
     "tcamcrf_loss_backward_logits_weighted": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_float, c_float, c_void_p]),
     "tcamcrf_workspace_status": (c_int, [c_void_p, c_void_p, POINTER(c_int), POINTER(c_int)]),
     "tcamcrf_debug_lattice": (c_int, [_cfgp, c_void_p, c_int, c_int, c_void_p, c_void_p, POINTER(c_int), c_void_p, c_size_t]),
+    "tcam_debug_seed_draws": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p]),
+    "tcam_debug_exp_draws": (c_int, [c_void_p, c_int, c_void_p, c_void_p]),
     "bilateralfilter": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_float, c_float]),
     "bilateralfilter_batch": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_float, c_float]),
     "colorbilateralfilter": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_float, c_int]),

@@ -477,12 +477,41 @@ __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k)
     return c;
 }
 
-// Exp(1) draw of (sample, side, pixel): -log(u), u uniform in (0, 1)
-__device__ __forceinline__ float seed_exp_draw(uint2 key, int b, int side, int pixel)
+// random word of (sample, side, pixel): first output word of Philox4x32-10 at counter (pixel, 2b + side, 0x5eed, 0)
+__device__ __forceinline__ unsigned int seed_philox_word(uint2 key, int b, int side, int pixel)
 {
-    const uint4 r = philox4x32_10(make_uint4((unsigned int)pixel, (unsigned int)(b * 2 + side), 0x5eedu, 0u), key);
-    const float u = ((float)(r.x >> 8) + 0.5f) * (1.0f / 16777216.0f);
-    return -__logf(u);
+    return philox4x32_10(make_uint4((unsigned int)pixel, (unsigned int)(b * 2 + side), 0x5eedu, 0u), key).x;
+}
+
+// Exp(1) draw from a 32-bit word: -log(u), u = (2m + 1) * 2^-24 with m = word >> 9.  2m + 1 < 2^24, so u is exact in
+// float32 and lies in [2^-24, 1 - 2^-24]: the draw is finite and > 0 (5.96e-8 .. 16.6), and u never rounds to 1 (a
+// zero draw would score -inf, the score of a non-candidate).  The smallest draws decide the picks and come from u near
+// 1, where __logf's absolute error bound is a few percent of the result; logf is within 1 ulp there.
+__device__ __forceinline__ float exp1_from_word(unsigned int word)
+{
+    const float u = (float)((word >> 9) * 2u + 1u) * (1.0f / 16777216.0f);
+    return -logf(u);
+}
+
+// test hooks (tcam_debug_seed_draws / tcam_debug_exp_draws): the words and draws seed_fused_kernel makes.
+// words / draws [B][2][HW]
+__global__ void __launch_bounds__(256) seed_debug_draws_kernel(const unsigned int *__restrict__ rng, int B, int HW,
+                                                               unsigned int *__restrict__ words, float *__restrict__ draws)
+{
+    const uint2 key = make_uint2(__ldg(rng), __ldg(rng + 1));
+    const long long total = (long long)B * 2 * HW;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+        const int bs = (int)(i / HW), pixel = (int)(i - (long long)bs * HW);
+        const unsigned int w = seed_philox_word(key, bs >> 1, bs & 1, pixel);
+        words[i] = w;
+        draws[i] = exp1_from_word(w);
+    }
+}
+
+__global__ void __launch_bounds__(256) seed_debug_exp_kernel(const unsigned int *__restrict__ words, int n,
+                                                             float *__restrict__ draws)
+{
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) draws[i] = exp1_from_word(words[i]);
 }
 
 __device__ __forceinline__ float nanmax(float m, float v)   // torch.maximum: NaN if either is NaN
@@ -782,7 +811,7 @@ __global__ void __launch_bounds__(kSeedFusedThreads) seed_fused_kernel(const See
                 float sc = -INFINITY;
                 if (is_cand) {
                     const float val = float_from_order_key(side ? key : ~key);
-                    const float draw = q ? __ldg(q + cr++) : seed_exp_draw(rkey, b, side, lo + i);
+                    const float draw = q ? __ldg(q + cr++) : exp1_from_word(seed_philox_word(rkey, b, side, lo + i));
                     sc = __fdiv_rn(weighted ? val : 1.0f, draw);
                 }
                 keys[i] = __float_as_uint(sc);

@@ -2995,6 +2995,33 @@ int tcamcrf_debug_lattice(const tcamcrf_config *cfg, const float *image_host, in
     return TCAMCRF_OK;
 }
 
+int tcam_debug_seed_draws(const unsigned int *rng_dev, int B, int HW, unsigned int *words_dev, float *draws_dev,
+                          void *cuda_stream)
+{
+    if (!rng_dev || !words_dev || !draws_dev) return fail(TCAMCRF_ERR_INVALID, "null pointer argument");
+    if (B < 1 || HW < 1) return fail(TCAMCRF_ERR_INVALID, "B,HW must be positive");
+    Device *dev = nullptr;
+    if (const int rc = this_device(&dev)) return rc;
+    long long blocks = ((long long)B * 2 * HW + 255) / 256;
+    if (blocks > persistent_grid(*dev)) blocks = persistent_grid(*dev);
+    seed_debug_draws_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)cuda_stream>>>(rng_dev, B, HW, words_dev, draws_dev);
+    CUDA_TRY(cudaGetLastError());
+    return TCAMCRF_OK;
+}
+
+int tcam_debug_exp_draws(const unsigned int *words_dev, int n, float *draws_dev, void *cuda_stream)
+{
+    if (!words_dev || !draws_dev) return fail(TCAMCRF_ERR_INVALID, "null pointer argument");
+    if (n < 1) return fail(TCAMCRF_ERR_INVALID, "n must be positive");
+    Device *dev = nullptr;
+    if (const int rc = this_device(&dev)) return rc;
+    long long blocks = ((long long)n + 255) / 256;
+    if (blocks > persistent_grid(*dev)) blocks = persistent_grid(*dev);
+    seed_debug_exp_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)cuda_stream>>>(words_dev, n, draws_dev);
+    CUDA_TRY(cudaGetLastError());
+    return TCAMCRF_OK;
+}
+
 // ---- drop-in host API ------------------------------------------------------
 
 int bilateralfilter(float *image, int len_image, float *in, int len_in, float *out, int len_out, int H, int W,
