@@ -217,9 +217,15 @@ int tcamcrf_loss_fwd_bwd_host(const tcamcrf_config *cfg, const float *images_hos
                               float *loss_host, float *grad_host, int N, int K, int H, int W, float grad_out);
 
 /* Tuning knobs (sweeps and tests; never needed for correctness).  The library reads TCAMCRF_<NAME> from the
- * environment once, at first use; this sets a knob at run time instead.  name: "CHUNK", "DENSE", "HIMG_SECTIONS",
- * "HOST_GROUPS", "HOST_SECTION0", "HOST_TRACE" (with or without the TCAMCRF_ prefix); value < 0 (or 0 where 0 is
- * not meaningful) restores the default. */
+ * environment once, at first use; this sets a knob at run time instead.  name, with or without the TCAMCRF_ prefix:
+ *   "DENSE"          1 / 0: the row-cooperative splat on / off, whatever the density hint says
+ *   "BUILD_DEDUP"    1 / 0: the shared-memory dedup lattice build on / off, whatever the density hint says
+ *   "HIMG_SECTIONS"  sections (1..64) of a chunk on the host-frames path (tcamcrf_loss_forward_host_frames)
+ *   "HOST_GROUPS"    value-stage groups (1..64) per chunk on the host-pointer path (tcamcrf_loss_fwd_bwd_host)
+ *   "HOST_SECTION0"  frames of the first lattice section on the host-pointer path
+ *   "HOST_GROW"      factor by which each later section on the host-pointer path grows over the one before
+ *   "HOST_TRACE"     1: print the timeline of every host-pointer call to stderr (runs the schedule eagerly)
+ * value < 0 (or 0 where 0 is not meaningful) restores the default.  Any other name is refused. */
 int tcamcrf_set_tuning(const char *name, int value);
 
 /* ---- measurement hooks (bench.py) ----

@@ -69,11 +69,10 @@ def needs_build() -> bool:
 
 
 def build(force: bool = False, verbose: bool = False) -> str:
-    """Compile csrc/*.cu into csrc/libtcamcrf.so for sm_100a (cross-compiles without a GPU)."""
+    """Compile csrc/tcamcrf.cu into csrc/libtcamcrf.so with NVCC_FLAGS only (sm_100a; cross-compiles without a GPU)."""
     if not force and not needs_build():
         return LIB_PATH
-    extra = os.environ.get("TCAMCRF_NVCC_EXTRA", "").split()   # e.g. -DTCAMCRF_NBR_U=4 for tuning sweeps
-    cmd = [_nvcc()] + NVCC_FLAGS + extra + ["-o", LIB_PATH] + SOURCES
+    cmd = [_nvcc()] + NVCC_FLAGS + ["-o", LIB_PATH] + SOURCES
     res = subprocess.run(cmd, capture_output=True, text=True)
     if verbose or res.returncode != 0:
         print(" ".join(cmd))

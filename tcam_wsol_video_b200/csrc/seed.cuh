@@ -438,10 +438,7 @@ __global__ void __launch_bounds__(kSeedThreads) seed_select_smem_kernel(const Se
 namespace cg = cooperative_groups;
 
 constexpr int kSeedCluster = 8;          // portable cluster size
-#ifndef TCAMCRF_SEED_THREADS
-#define TCAMCRF_SEED_THREADS 512
-#endif
-constexpr int kSeedFusedThreads = TCAMCRF_SEED_THREADS;   // 512 or 1024
+constexpr int kSeedFusedThreads = 512;
 static_assert(kSeedFusedThreads >= 512 && kSeedFusedThreads <= 1024 && kSeedFusedThreads % 32 == 0, "one thread per (side, bin)");
 constexpr int kSeedFusedMaxK = 32;       // seeds per side this kernel handles (larger k: the two-kernel path)
 

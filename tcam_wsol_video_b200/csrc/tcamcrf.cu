@@ -51,10 +51,6 @@
 #include "lattice.cuh"
 #include "seed.cuh"
 
-#ifndef TCAMCRF_SEED_SMEM
-#define TCAMCRF_SEED_SMEM 1
-#endif
-
 namespace tcamcrf {
 
 // ---------------------------------------------------------------------------
@@ -84,15 +80,12 @@ static int fail(int code, const char *fmt, ...)
 // tcamcrf_set_tuning() -- no getenv on the call path.  0 / -1 = library default.
 // ---------------------------------------------------------------------------
 struct Tuning {
-    int chunk = 0;            // TCAMCRF_CHUNK: frames per pass (sweeps)
     int dense = -1;           // TCAMCRF_DENSE: force the row-cooperative splat on (1) / off (0); -1 = density hint
     int build_dedup = -1;     // TCAMCRF_BUILD_DEDUP: force the shared-memory dedup build on (1) / off (0); -1 = density hint
     int himg_sections = 0;    // TCAMCRF_HIMG_SECTIONS: sections of a chunk on the host-frames path
     int host_groups = 0;      // TCAMCRF_HOST_GROUPS: value-stage groups per chunk on the host-pointer path
     int host_section0 = 0;    // TCAMCRF_HOST_SECTION0: frames of the first section on the host-pointer path
     int host_trace = 0;       // TCAMCRF_HOST_TRACE: print the timeline of host_run
-    int host_taper = -1;      // TCAMCRF_HOST_TAPER: group = 1/taper of the frames left (0: equal groups; -1: default)
-    int host_graph = 1;       // TCAMCRF_HOST_GRAPH: replay the host-pointer schedule as a CUDA graph (pinned buffers)
     int host_grow = 0;        // TCAMCRF_HOST_GROW: each section of the host-pointer path is this many times the one before
 };
 static int env_int(const char *name, int dflt)
@@ -104,15 +97,12 @@ static Tuning &tuning()
 {
     static Tuning t = [] {
         Tuning x;
-        x.chunk = env_int("TCAMCRF_CHUNK", 0);
         x.dense = env_int("TCAMCRF_DENSE", -1);
         x.build_dedup = env_int("TCAMCRF_BUILD_DEDUP", -1);
         x.himg_sections = env_int("TCAMCRF_HIMG_SECTIONS", 0);
         x.host_groups = env_int("TCAMCRF_HOST_GROUPS", 0);
         x.host_section0 = env_int("TCAMCRF_HOST_SECTION0", 0);
         x.host_trace = getenv("TCAMCRF_HOST_TRACE") != nullptr;
-        x.host_taper = env_int("TCAMCRF_HOST_TAPER", -1);
-        x.host_graph = env_int("TCAMCRF_HOST_GRAPH", 1);
         x.host_grow = env_int("TCAMCRF_HOST_GROW", 0);
         return x;
     }();
@@ -195,7 +185,6 @@ static int make_plan(const tcamcrf_config *cfg, int N, int K, int H, int W, Plan
     pl.W = W;
     pl.P = H * W;
     int chunk = cfg->chunk_frames > 0 ? cfg->chunk_frames : 64;
-    if (tuning().chunk > 0) chunk = tuning().chunk;   // tuning sweeps only (tools/sweep.sh)
     if (chunk > 256) chunk = 256;  // kMaxChunk: the vertex kernels keep a per-frame prefix sum in shared memory
     pl.chunk = chunk < N ? chunk : N;
     // every pixel (+ the ghost pixel) contributes at most d+1 distinct vertices
@@ -226,7 +215,7 @@ static int make_plan(const tcamcrf_config *cfg, int N, int K, int H, int W, Plan
         if (most < 1) return fail(TCAMCRF_ERR_INVALID, "image too large");
         if (pl.chunk > most) pl.chunk = (int)most;
     }
-    if (cfg->chunk_frames <= 0 && tuning().chunk <= 0) {
+    if (cfg->chunk_frames <= 0) {
         // default chunk: keep the workspace of large frames within ~16 GiB (64 frames of 1024x1024 would take 47)
         const double per_frame = (double)pl.slots * sizeof(Entry) + 2.0 * (D + 1) * pl.P * 4.0 +
                                  (double)pl.stride * (8.0 + (D + 1) * 8.0 + 2.0 * pl.Kp * 4.0);
@@ -273,20 +262,13 @@ static int make_plan(const tcamcrf_config *cfg, int N, int K, int H, int W, Plan
 // pdl_launch_dependents() only AFTER its own pdl_wait(): when kernel X+1 starts, all blocks of X are past their
 // wait, hence X-1 and everything before it is complete.  So, ahead of its wait, a kernel may READ what kernels
 // up to X-2 (and the caller) produced, and must not write anything.
-#ifndef TCAMCRF_PDL
-#define TCAMCRF_PDL 1
-#endif
 __device__ __forceinline__ void pdl_wait()
 {
-#if TCAMCRF_PDL
     asm volatile("griddepcontrol.wait;" ::: "memory");
-#endif
 }
 __device__ __forceinline__ void pdl_launch_dependents()
 {
-#if TCAMCRF_PDL
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
 }
 
 struct BuildParams {
@@ -320,15 +302,10 @@ __device__ __forceinline__ float load_pixel<uint8_t>(const void *base, size_t id
     return (float)__ldg((const uint8_t *)base + idx);
 }
 
-#ifndef TCAMCRF_ADAPTIVE_TABLE
-#define TCAMCRF_ADAPTIVE_TABLE 1
-#endif
 // primary-tier slots per vertex of the previous call (rounded up to a power of two).  Measured, noise K=10, 32 frames:
 // 4 -> build 0.206 / neighbour 0.130 / clear 0.028 ms; 2 (tables of all frames fit the L2) -> 0.211 / 0.159 / 0.016;
 // 1 -> 0.343 / 0.481 / 0.036: the probe count matters, not where the table lives.
-#ifndef TCAMCRF_TABLE_HEADROOM
-#define TCAMCRF_TABLE_HEADROOM 4
-#endif
+constexpr unsigned int kTableHeadroom = 4;
 // Clears the tables of `nc` frames: always the primary tier, the overflow tier only when the workspace is
 // new (magic mismatch) or the previous use spilled into it.  Also zeroes the per-frame vertex counters.
 __global__ void __launch_bounds__(kThreads) prepare_kernel(Entry *table, int *ctrl, int frame0, int nc, int chunk,
@@ -340,17 +317,15 @@ __global__ void __launch_bounds__(kThreads) prepare_kernel(Entry *table, int *ct
     const bool full = frame0 == 0 && ((ctrl[kCtrlMagic] != sig) || (ctrl[kCtrlDirty] != 0));
     // primary-tier size for this call (see effective_geom); later sections of a chunk take the first one's
     unsigned int eff = geom.slots1;
-#if TCAMCRF_ADAPTIVE_TABLE
     if (frame0 > 0) {
         eff = (unsigned int)ctrl[kCtrlEffSlots];
     } else if (!full) {
-        const unsigned int want = (unsigned int)TCAMCRF_TABLE_HEADROOM * (unsigned int)ctrl[kCtrlPrevMax];
+        const unsigned int want = kTableHeadroom * (unsigned int)ctrl[kCtrlPrevMax];
         unsigned int e = geom.slots1 >> 4;   // floor: bounds what a bad guess costs (window-long probe chains)
         if (e < 4096u) e = 4096u;
         while (e < want && e < geom.slots1) e <<= 1;
         eff = e < geom.slots1 ? e : geom.slots1;
     }
-#endif
     const unsigned int slots = geom.base2 + geom.slots2;
     geom.slots1 = eff;
     const long long n_primary = (long long)nc * geom.slots1;
@@ -383,15 +358,7 @@ __global__ void __launch_bounds__(kThreads) prepare_kernel(Entry *table, int *ct
 // Occupancy target of the build kernel: 5 blocks of 256 threads per SM caps it at 48 registers (a few
 // spills).  Measured on B200 (K=2, noise / natural frames, ms per 32-frame batch): 3 blocks 0.250 / 0.143,
 // 4 blocks 0.221 / 0.119, 5 blocks 0.214 / 0.109, 6 blocks 0.218 / 0.107, 8 blocks 0.235 / 0.107.
-#ifndef TCAMCRF_BUILD_INTERLEAVE
-#define TCAMCRF_BUILD_INTERLEAVE 1
-#endif
-#ifndef TCAMCRF_BUILD_MINBLOCKS
-#define TCAMCRF_BUILD_MINBLOCKS 5
-#endif
-#ifndef TCAMCRF_BUILD_CAS_BATCH
-#define TCAMCRF_BUILD_CAS_BATCH 1
-#endif
+constexpr int kBuildMinBlocks = 5;
 // Front end shared by the two build kernels: the pixel's features (initializePermutohedral, bilateralfilter.cpp:4-19 /
 // colorbilateralfilter.cpp:4-15), its embedding, the d+1 packed keys of its simplex, and the barycentric weights,
 // which leave the registers right here.  Reads the caller's images only, so it runs ahead of griddepcontrol.wait (the
@@ -438,15 +405,10 @@ __device__ __forceinline__ bool build_front(const BuildParams &p, int n, int pix
 }
 
 template <int D, typename ImgT>
-__global__ void __launch_bounds__(kThreads, TCAMCRF_BUILD_MINBLOCKS) build_kernel(const BuildParams p)
+__global__ void __launch_bounds__(kThreads, kBuildMinBlocks) build_kernel(const BuildParams p)
 {
-#if TCAMCRF_BUILD_INTERLEAVE
     const int n = p.frame0 + blockIdx.x;
     const int pix = blockIdx.y * kThreads + threadIdx.x;
-#else
-    const int n = p.frame0 + blockIdx.y;
-    const int pix = blockIdx.x * kThreads + threadIdx.x;
-#endif
     const bool valid = pix < p.P;
     // The reference embeds pixels four at a time and also inserts the zero-feature padding pixels of the
     // last partial block (permutohedral.cpp:173,238-251).  Those vertices are never splatted to, but they
@@ -513,7 +475,6 @@ __global__ void __launch_bounds__(kThreads, TCAMCRF_BUILD_MINBLOCKS) build_kerne
     constexpr int kLockstepRounds = 6;
     int rounds = 0;
     for (; rounds < kLockstepRounds && pend; rounds++) {
-#if TCAMCRF_BUILD_CAS_BATCH
         // every claim of the round is issued before any result is looked at: with the compare-and-swap and the test of
         // its result in one branch per key, a warp went through up to d+1 atomic round trips one after the other
         unsigned int tried = 0;
@@ -540,25 +501,6 @@ __global__ void __launch_bounds__(kThreads, TCAMCRF_BUILD_MINBLOCKS) build_kerne
             else
                 slot[r] = (int)(((unsigned int)slot[r] + 1u) & mask1);
         }
-#else
-#pragma unroll
-        for (int r = 0; r <= D; r++) {
-            if (!(pend & (1u << r))) continue;
-            unsigned long long c = cur[r];
-            if (c == kEmptyKey) {
-                c = atomicCAS(&tab[slot[r]].key, kEmptyKey, key[r]);
-                vid[r] = -1;   // ours to allocate below, or created this instant by another thread
-                if (c == kEmptyKey) {
-                    wonmask |= 1u << r;
-                    c = key[r];
-                }
-            }
-            if (c == key[r])
-                pend &= ~(1u << r);
-            else
-                slot[r] = (int)(((unsigned int)slot[r] + 1u) & mask1);
-        }
-#endif
 #pragma unroll
         for (int r = 0; r <= D; r++)
             if (pend & (1u << r)) load_entry_cg(tab + slot[r], cur[r], vid[r]);
@@ -634,13 +576,7 @@ __global__ void __launch_bounds__(kThreads, TCAMCRF_BUILD_MINBLOCKS) build_kerne
 // pick their result up from shared memory.  All of the shared-memory phase runs ahead of griddepcontrol.wait, i.e.
 // while prepare_kernel is still clearing the tables.  Same table protocol and the same results as build_kernel (ids
 // are a relabelling); the host picks per call from the density hint, like the splat variant.
-#ifndef TCAMCRF_TILE_W
-#define TCAMCRF_TILE_W 32
-#endif
-#ifndef TCAMCRF_TILE_H
-#define TCAMCRF_TILE_H 8
-#endif
-constexpr int kTileW = TCAMCRF_TILE_W, kTileH = TCAMCRF_TILE_H;   // pixel tile of a build_dedup_kernel block
+constexpr int kTileW = 32, kTileH = 8;   // pixel tile of a build_dedup_kernel block
 constexpr int kTileThreads = kTileW * kTileH;
 static_assert(kTileW == 8 || kTileW == 16 || kTileW == 32, "a warp covers whole row segments of the tile");
 static_assert(kTileThreads % 32 == 0 && kTileThreads <= 256, "tile = one thread block");
@@ -655,11 +591,9 @@ struct DedupTable {
     static constexpr unsigned int kShift = 32 - kBits;
 };
 
-#ifndef TCAMCRF_DEDUP_MINBLOCKS
-#define TCAMCRF_DEDUP_MINBLOCKS 8
-#endif
+constexpr int kDedupMinBlocks = 8;
 template <int D, typename ImgT>
-__global__ void __launch_bounds__(kTileThreads, TCAMCRF_DEDUP_MINBLOCKS) build_dedup_kernel(const BuildParams p)
+__global__ void __launch_bounds__(kTileThreads, kDedupMinBlocks) build_dedup_kernel(const BuildParams p)
 {
     constexpr int kSlots = DedupTable<D>::kSlots;
     __shared__ __align__(16) unsigned long long s_key[kSlots];
@@ -1565,9 +1499,6 @@ __global__ void __launch_bounds__(kThreads) temporal_max_kernel(const float *__r
 // ---------------------------------------------------------------------------
 
 // Vertex density of the recent calls, per workspace (density_hint below).
-#ifndef TCAMCRF_DENSITY_HINT
-#define TCAMCRF_DENSITY_HINT 1
-#endif
 struct DensityHints {
     struct Slot {
         void *ws;
@@ -1640,7 +1571,7 @@ struct HostGraphs {
         tcamcrf_config cfg;
         int N, K, H, W;
         const void *images, *segs, *as_host, *grad_host, *buf, *pin;
-        int want_loss, dedup, dense, groups_knob, taper_knob, sec0_knob, grow_knob;
+        int want_loss, dedup, dense, groups_knob, sec0_knob, grow_knob;
         bool operator==(const Key &o) const { return memcmp(this, &o, sizeof(Key)) == 0; }
     };
     struct Item {
@@ -1806,7 +1737,7 @@ static void launch_chained_block(void (*kernel)(KArgs...), dim3 grid, int thread
     lc.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = TCAMCRF_PDL;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
     lc.attrs = attr;
     lc.numAttrs = 1;
     cudaLaunchKernelEx(&lc, kernel, std::forward<Args>(args)...);
@@ -1936,11 +1867,7 @@ static int lattice_stages(Device &dev, const tcamcrf_config *cfg, const Plan &pl
         bp.sigma_xy = cfg->sigma_xy;
         bp.frame0 = frame0;
         scale_factors(D, bp.ec);
-#if TCAMCRF_BUILD_INTERLEAVE
         dim3 bgrid(nc, pl.blocks_per_frame);
-#else
-        dim3 bgrid(pl.blocks_per_frame, nc);
-#endif
         // sparse lattice lately (or nothing known yet): deduplicate the block's keys in shared memory first
         bool dedup = !lattice_is_dense(density_hint(dev, ws), pl.P);
         if (tuning().build_dedup >= 0) dedup = tuning().build_dedup != 0;   // tests and sweeps: force either way
@@ -1993,7 +1920,6 @@ static bool stream_is_capturing(cudaStream_t st)
 // largest per-frame vertex count seen lately on this workspace (0: unknown)
 static int density_hint(Device &dev, void *ws)
 {
-    if (!TCAMCRF_DENSITY_HINT) return 0;
     std::lock_guard<std::mutex> lock(dev.hints.mu);
     DensityHints::Slot *slot = dev.hints.find(ws, false);
     return slot ? *(volatile int *)slot->word : 0;
@@ -2004,7 +1930,6 @@ static int density_hint(Device &dev, void *ws)
 // while a graph is being captured (an unjoined fork is not capturable; the hint then keeps its last value).
 static void density_hint_refresh(Device &dev, const Plan &pl, char *ws, cudaStream_t st)
 {
-    if (!TCAMCRF_DENSITY_HINT) return;
     if (stream_is_capturing(st)) return;   // (also: no pinned allocation while a capture is open)
     std::lock_guard<std::mutex> lock(dev.hints.mu);
     DensityHints::Slot *slot = dev.hints.find(ws, true);
@@ -2361,19 +2286,11 @@ struct HostJob {
     bool dedup_hint, dense_hint;   // part of the graph key: the kernel variants are chosen at enqueue time
 };
 
-// group sizes of the value stages for `frames` frames: equal groups (`taper` <= 0) or each group a 1/taper share of
-// what is left (at least one frame), so the last groups -- whose compute and copy back nothing overlaps -- are small
-static void host_groups(int frames, int equal_size, int taper, std::vector<int> &out)
+// group sizes of the value stages for `frames` frames: groups of `size` frames, the last one shorter
+static void host_groups(int frames, int size, std::vector<int> &out)
 {
     out.clear();
-    int left = frames;
-    while (left > 0) {
-        int g = taper > 0 ? (left + taper - 1) / taper : equal_size;
-        if (g < 1) g = 1;
-        if (g > left) g = left;
-        out.push_back(g);
-        left -= g;
-    }
+    for (int left = frames; left > 0; left -= size) out.push_back(size < left ? size : left);
 }
 
 // Queues the whole call on the three streams.  `st` is the origin: s_in / s_out fork from it and join it again, so
@@ -2399,12 +2316,11 @@ static int host_enqueue(Device &dev, const HostJob &j, HostTrace &trace, int *gr
     // Value-stage groups (measured on B200, tools/r2_host_sweep.sh, 32 frames): wide batches (K >= 6: the
     // segmentations are most of the bytes) in groups of 2 frames, so that results flow back almost as soon as their
     // inputs are in (K=10: 2.18 -> 2.06 ms per call); narrow ones in groups of a quarter chunk.  TCAMCRF_HOST_GROUPS
-    // = groups per chunk; TCAMCRF_HOST_TAPER > 0 = each group 1/taper of what is left.
+    // = groups per chunk.
     int group = K >= 6 ? 2 : (pl.chunk + 3) / 4;
     if (tuning().host_groups >= 1 && tuning().host_groups <= 64)
         group = (pl.chunk + tuning().host_groups - 1) / tuning().host_groups;
     if (group < 1) group = 1;
-    const int taper = tuning().host_taper >= 0 ? tuning().host_taper : 0;
     std::vector<int> sizes;
     int gi = 0;   // running group index
     for (int c0 = 0; c0 < N; c0 += pl.chunk) {
@@ -2442,7 +2358,7 @@ static int host_enqueue(Device &dev, const HostJob &j, HostTrace &trace, int *gr
             rc = run_lattice(dev, &j.cfg, pl, false, j.d_img + (size_t)c0 * img_frame, f0, fn, j.d_ws, false, st);
             if (rc) return rc;
             trace.mark("lattice", c0 + f0, st);
-            host_groups(fn, group, taper, sizes);
+            host_groups(fn, group, sizes);
             if (f0 == 0 && fn < cn && fn <= group) sizes.assign(1, fn);   // a small first section stays whole
             int g0 = f0;
             for (size_t si = 0; si < sizes.size(); si++, gi++) {
@@ -2582,7 +2498,7 @@ static int host_run(const tcamcrf_config *cfg_in, const float *images, const flo
     int gi = 0;
     // the captured schedule needs pinned buffers (a copy from pageable memory cannot be captured), and neither the
     // per-stage profiler nor the trace (both record timing events between the kernels)
-    const bool graph_ok = tuning().host_graph != 0 && !g_prof.enabled && tuning().host_trace == 0 &&
+    const bool graph_ok = !g_prof.enabled && tuning().host_trace == 0 &&
                           host_pinned(images) && host_pinned(segs) && host_pinned(as_host) && host_pinned(grad_host);
     HostGraphs::Key key;
     memset(&key, 0, sizeof(key));
@@ -2593,7 +2509,7 @@ static int host_run(const tcamcrf_config *cfg_in, const float *images, const flo
         key.images = images; key.segs = segs; key.as_host = as_host; key.grad_host = grad_host;
         key.buf = g_host.buf; key.pin = g_host.pin;
         key.want_loss = j.want_loss; key.dedup = j.dedup_hint; key.dense = j.dense_hint;
-        key.groups_knob = tuning().host_groups; key.taper_knob = tuning().host_taper; key.sec0_knob = tuning().host_section0; key.grow_knob = tuning().host_grow;
+        key.groups_knob = tuning().host_groups; key.sec0_knob = tuning().host_section0; key.grow_knob = tuning().host_grow;
         for (auto &it : graphs.items)
             if (it.key == key) hit = &it;
     }
@@ -3086,15 +3002,12 @@ int tcamcrf_set_tuning(const char *name, int value)
     if (!name) return fail(TCAMCRF_ERR_INVALID, "null knob name");
     if (strncmp(name, "TCAMCRF_", 8) == 0) name += 8;
     Tuning &t = tuning();
-    if (!strcmp(name, "CHUNK")) t.chunk = value > 0 ? value : 0;
-    else if (!strcmp(name, "DENSE")) t.dense = value < 0 ? -1 : (value != 0);
+    if (!strcmp(name, "DENSE")) t.dense = value < 0 ? -1 : (value != 0);
     else if (!strcmp(name, "BUILD_DEDUP")) t.build_dedup = value < 0 ? -1 : (value != 0);
     else if (!strcmp(name, "HIMG_SECTIONS")) t.himg_sections = value > 0 ? value : 0;
     else if (!strcmp(name, "HOST_GROUPS")) t.host_groups = value > 0 ? value : 0;
     else if (!strcmp(name, "HOST_SECTION0")) t.host_section0 = value > 0 ? value : 0;
     else if (!strcmp(name, "HOST_TRACE")) t.host_trace = value > 0;
-    else if (!strcmp(name, "HOST_TAPER")) t.host_taper = value;
-    else if (!strcmp(name, "HOST_GRAPH")) t.host_graph = value < 0 ? 1 : (value != 0);
     else if (!strcmp(name, "HOST_GROW")) t.host_grow = value > 0 ? value : 0;
     else return fail(TCAMCRF_ERR_INVALID, "unknown tuning knob '%s'", name);
     return TCAMCRF_OK;
@@ -3165,7 +3078,7 @@ int tcam_seed_select(const float *cams_dev, int T, const int64_t *roi_dev, const
         StageScope scope(kStSeed, 1, (cudaStream_t)cuda_stream);
         // keys of a sample in shared memory when the frame fits (4 bytes per pixel of the 227 KB an SM has)
         const size_t smem = (size_t)HW * sizeof(unsigned int);
-        if (TCAMCRF_SEED_SMEM && smem <= (size_t)dev->select_smem)
+        if (smem <= (size_t)dev->select_smem)
             seed_select_smem_kernel<<<dim3(2, B), kSeedThreads, smem, (cudaStream_t)cuda_stream>>>(sp);
         else
             seed_select_kernel<<<dim3(2, B), kSeedThreads, 0, (cudaStream_t)cuda_stream>>>(sp);

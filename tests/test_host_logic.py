@@ -263,13 +263,16 @@ def test_key_range_is_refused_on_the_host():
 
 
 def test_tuning_knobs_are_set_at_run_time():
-    """The TCAMCRF_* environment variables are read once; tests and sweeps change knobs through the C ABI."""
-    _lib.set_tuning("DENSE", 1)
-    _lib.set_tuning("TCAMCRF_HOST_GROUPS", 3)
-    _lib.set_tuning("DENSE", -1)
-    _lib.set_tuning("HOST_GROUPS", -1)
-    with pytest.raises(_lib.TcamCrfError, match="unknown tuning knob"):
-        _lib.set_tuning("NO_SUCH_KNOB", 1)
+    """The TCAMCRF_* environment variables are read once; tests and sweeps change knobs through the C ABI.  Knobs
+    whose experiments are decided (CHUNK, HOST_TAPER, HOST_GRAPH) are gone and are refused like any unknown name."""
+    for name in ("DENSE", "BUILD_DEDUP", "HIMG_SECTIONS", "HOST_GROUPS", "HOST_SECTION0", "HOST_GROW", "HOST_TRACE"):
+        _lib.set_tuning(name, 1)
+        _lib.set_tuning(name, -1)
+        _lib.set_tuning("TCAMCRF_" + name, 1)
+        _lib.set_tuning("TCAMCRF_" + name, -1)
+    for name in ("NO_SUCH_KNOB", "CHUNK", "HOST_TAPER", "HOST_GRAPH"):
+        with pytest.raises(_lib.TcamCrfError, match="unknown tuning knob"):
+            _lib.set_tuning(name, 1)
 
 
 def test_release_workspaces_clears_every_cached_buffer():

@@ -21,16 +21,16 @@ while time.time() - t0 < budget:
     colour = rng.random() < 0.3
     srgb = float(rng.choice([3.0, 8.0, 15.0, 40.0, 120.0])); sxy = float(rng.choice([5.0, 30.0, 100.0, 400.0]))
     u8 = rng.random() < 0.4
-    for name, val in (("BUILD_DEDUP", int(rng.integers(-1, 2))), ("DENSE", int(rng.integers(-1, 2))),
-                      ("CHUNK", int(rng.choice([0, 0, 1, 2, 3])))):
-        _lib.set_tuning(name, val)
+    for name in ("BUILD_DEDUP", "DENSE"):
+        _lib.set_tuning(name, int(rng.integers(-1, 2)))
+    chunk = int(rng.choice([0, 0, 1, 2, 3]))   # frames per pass (0: the library's default)
     seg = synth.make_segs(n, k, h, w, seed=int(rng.integers(1 << 30)))
     if colour:
         dim = int(rng.integers(1, 7))
         planes = rng.integers(0, 256, size=(1, dim, h, w)).astype(np.float32)      # one frame: the batch loop strides by 3
         n = 1; seg = seg[:1]
         want = oracle.port_colorbilateralfilter_batch(planes, seg, 1, k, h, w, srgb, dim).reshape(seg.shape)
-        cfg = _lib.make_config(_lib.FEAT_COLOR, dim, srgb)
+        cfg = _lib.make_config(_lib.FEAT_COLOR, dim, srgb, chunk_frames=chunk)
         img = planes
         tag = f"colour{dim}"
     else:
@@ -38,7 +38,7 @@ while time.time() - t0 < budget:
         img = synth.make_images(n, h, w, kind, seed=int(rng.integers(1 << 30)), channels=ch)
         want = np.stack([oracle.port_filter_features(oracle.xy_features(h, w, sxy, img[i], srgb), seg[i])
                          for i in range(n)]).reshape(seg.shape)
-        cfg = _lib.make_config(_lib.FEAT_XY_RGB, ch, srgb, sxy)
+        cfg = _lib.make_config(_lib.FEAT_XY_RGB, ch, srgb, sxy, chunk_frames=chunk)
         tag = f"xy+{ch}"
     if not _lib.load().tcamcrf_key_range_ok(cfg, h, w, 255.0):
         continue
@@ -53,7 +53,7 @@ while time.time() - t0 < budget:
     if not (err < 1e-4) or not np.isfinite(loss.item()):
         fails += 1
         print("FAIL", dict(n=n, k=k, h=h, w=w, kind=kind, tag=tag, srgb=srgb, sxy=sxy, u8=u8, err=err), flush=True)
-for name in ("BUILD_DEDUP", "DENSE", "CHUNK"):
-    _lib.set_tuning(name, -1 if name != "CHUNK" else 0)
+for name in ("BUILD_DEDUP", "DENSE"):
+    _lib.set_tuning(name, -1)
 print(f"fuzz: {cases} cases in {time.time() - t0:.0f} s, {fails} failures, worst normwise rel err {worst:.2e}; lattices {kinds}")
 sys.exit(1 if fails else 0)

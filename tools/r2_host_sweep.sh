@@ -13,7 +13,6 @@ for s0 in 2 4; do for grow in 1 2 3; do for groups in 8 16; do
 done; done; done
 run "TCAMCRF_HOST_SECTION0=8 TCAMCRF_HOST_GROW=1 TCAMCRF_HOST_GROUPS=8"
 run "TCAMCRF_HOST_SECTION0=8 TCAMCRF_HOST_GROW=1 TCAMCRF_HOST_GROUPS=16"
-run "TCAMCRF_HOST_SECTION0=4 TCAMCRF_HOST_GROW=2 TCAMCRF_HOST_TAPER=4"
 run "TCAMCRF_HOST_SECTION0=1 TCAMCRF_HOST_GROW=2 TCAMCRF_HOST_GROUPS=16"
 KS="2"
 for s0 in 4 8 16; do for grow in 1 2; do for groups in 2 4 8; do
