@@ -152,6 +152,15 @@ def port_lattice_color(image, H, W, sigma_rgb, DIM) -> Lattice:
     return _port_lattice_from_handle(lib, h, DIM, H * W)
 
 
+def port_lattice_features(features) -> Lattice:
+    """The lattice of explicit per-pixel features [n, d] (already divided by their sigmas): Permutohedral::init
+    (permutohedral.cpp:115-297), for layouts the two wrappers do not build (x, y + 1, 2 or 4 planes)."""
+    lib = load_port()
+    features = _f32(features)
+    n, d = features.shape
+    return _port_lattice_from_handle(lib, lib.po_build(_ptr(features.ravel()), d, n), d, n)
+
+
 def port_filter_features(features, planes) -> np.ndarray:
     """Filters `planes` [K, n] through the lattice of explicit per-pixel features [n, d] (already divided by
     their sigmas): Permutohedral::init + one compute per plane (permutohedral.cpp:115-297, 507-572).
