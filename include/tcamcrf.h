@@ -41,7 +41,7 @@
 extern "C" {
 #endif
 
-#define TCAMCRF_VERSION 103
+#define TCAMCRF_VERSION 104
 
 /* host-side status codes */
 #define TCAMCRF_OK 0
@@ -249,10 +249,11 @@ int tcam_temporal_max(const float *cams_dev, float *out_dev, int B, int T, int H
  * cams_dev [B,H*W]; thresh_dev [B] on the 0..255 scale (tcam_otsu_roi's thresholds, or thresh*255);
  * roi_dev [B,H*W] int64 0/1: the selected 4-connected component of cam*255 >= thresh; bbox_dev [B,4] int32
  * x0,y0,x1,y1 (cv2.boundingRect convention of dlib/utils/wsol.py:133-137); bbox_mask_dev [B,H*W] float 0/1.
- * p_min_area: a densest component smaller than p_min_area*H*W gives way to the largest one. */
+ * p_min_area: a densest component smaller than p_min_area*H*W gives way to the largest one; a double, so that the
+ * product is the reference's float64 (h*w)*p_min_area_roi and a component of exactly that area is kept. */
 size_t tcam_roi_components_scratch_bytes(int B, int H, int W);
 int tcam_roi_components(const float *cams_dev, const float *thresh_dev, long long *roi_dev, float *bbox_mask_dev,
-                        int *bbox_dev, int B, int H, int W, int largest_only, float p_min_area, void *scratch_dev,
+                        int *bbox_dev, int B, int H, int W, int largest_only, double p_min_area, void *scratch_dev,
                         size_t scratch_bytes, void *cuda_stream);
 
 /* The same with the loader's per-frame re-normalisation first (re_normalize_cam, dlib/datasets/wsol_loader.py:

@@ -13,6 +13,8 @@ stream.  It runs on whatever device its inputs are on and uses the very same tor
                           /root/reference; requirements.txt:36): out = max over the ksz x ksz window whose
                           origin is (ksz//2, ksz//2), positions outside the image ignored (geodesic border)
   tcam_seeder_forward  <- TCAMSeeder.forward  tcam_seeding.py:178-256
+  paint_seed_labels    <- its painting tail, tcam_seeding.py:239-254 (seed_labels_from_sel: the same from a
+                          [B,2,kmax] selection, what SparseSeeds holds)
 
 Parity of flat_dilation and of torch 2.11's multinomial/sort against the versions the reference pins
 (torch 1.11, kornia 0.6.4) is UNPINNED: no reference test fixes them and those packages are not installed
@@ -145,24 +147,44 @@ def flat_dilation(x: torch.Tensor, ksz: int) -> torch.Tensor:
     return F.max_pool2d(padded, kernel_size=ksz, stride=1).to(x.dtype)
 
 
-def tcam_seeder_forward(x, roi=None, *, seed_tech, min_, max_, min_p, max_p, ksz, ignore_idx, use_roi):
-    b, d, h, w = x.shape
-    assert d == 1
-    out = torch.zeros((b, h, w), dtype=torch.long, device=x.device) + ignore_idx
-    all_fg = torch.zeros((b, h, w), dtype=torch.long, device=x.device)
-    all_bg = torch.zeros((b, h, w), dtype=torch.long, device=x.device)
-    for i in range(b):
-        _roi = roi[i].squeeze() if roi is not None else None
-        all_fg[i], all_bg[i] = one_sample(x[i].squeeze(), _roi, min_p=min_p, max_p=max_p, min_=min_, max_=max_,
-                                          seed_tech=seed_tech, use_roi=use_roi)
-    all_fg = flat_dilation(all_fg.unsqueeze(1), ksz).squeeze(1)
-    all_bg = flat_dilation(all_bg.unsqueeze(1), ksz).squeeze(1)
+def paint_seed_labels(fg, bg, ksz, ignore_idx):
+    """The painting tail of TCAMSeeder.forward (tcam_seeding.py:239-254): fg, bg [B,H,W] long 0/1 seed maps -> the
+    [B,H,W] long label map.  Both sides are dilated; a pixel claimed by both is ignored."""
+    b, h, w = fg.shape
+    out = torch.zeros((b, h, w), dtype=torch.long, device=fg.device) + ignore_idx
+    all_fg = flat_dilation(fg.unsqueeze(1), ksz).squeeze(1).clone()
+    all_bg = flat_dilation(bg.unsqueeze(1), ksz).squeeze(1).clone()
     outer = all_fg + all_bg
     all_fg[outer == 2] = 0
     all_bg[outer == 2] = 0
     out[all_fg == 1] = 1
     out[all_bg == 1] = 0
     return out.detach()
+
+
+def seed_labels_from_sel(sel, ksz, h, w, ignore_idx):
+    """The label map of selected seed pixels: sel [B,2,kmax] (side 0 foreground, 1 background; flat pixel indices,
+    -1 = unused slot) -> one-hot fg / bg maps -> paint_seed_labels."""
+    sel = torch.as_tensor(sel).long().cpu()
+    b = sel.shape[0]
+    maps = torch.zeros((2, b, h * w), dtype=torch.long)
+    for i in range(b):
+        for side in range(2):
+            idx = sel[i, side]
+            maps[side, i, idx[idx >= 0]] = 1
+    return paint_seed_labels(maps[0].view(b, h, w), maps[1].view(b, h, w), ksz, ignore_idx)
+
+
+def tcam_seeder_forward(x, roi=None, *, seed_tech, min_, max_, min_p, max_p, ksz, ignore_idx, use_roi):
+    b, d, h, w = x.shape
+    assert d == 1
+    all_fg = torch.zeros((b, h, w), dtype=torch.long, device=x.device)
+    all_bg = torch.zeros((b, h, w), dtype=torch.long, device=x.device)
+    for i in range(b):
+        _roi = roi[i].squeeze() if roi is not None else None
+        all_fg[i], all_bg[i] = one_sample(x[i].squeeze(), _roi, min_p=min_p, max_p=max_p, min_=min_, max_=max_,
+                                          seed_tech=seed_tech, use_roi=use_roi)
+    return paint_seed_labels(all_fg, all_bg, ksz, ignore_idx)
 
 
 # --------------------------------------------------------------------------------------------------

@@ -10,7 +10,7 @@ import ctypes
 import os
 import shutil
 import subprocess
-from ctypes import POINTER, Structure, c_char_p, c_float, c_int, c_size_t, c_void_p
+from ctypes import POINTER, Structure, c_char_p, c_double, c_float, c_int, c_size_t, c_void_p
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
@@ -123,7 +123,7 @@ SIGNATURES = {
     "tcamcrf_launch_count": (ctypes.c_longlong, []),
     "tcam_temporal_max": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "tcam_roi_components_scratch_bytes": (c_size_t, [c_int, c_int, c_int]),
-    "tcam_roi_components": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_float, c_void_p, c_size_t, c_void_p]),
+    "tcam_roi_components": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_double, c_void_p, c_size_t, c_void_p]),
     "tcam_temporal_max_renorm": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_float, c_void_p]),
     "tcam_prepare_std_cams": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "tcam_seed_select": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,

@@ -1015,7 +1015,9 @@ __global__ void __launch_bounds__(256) seed_ce_forward_kernel(const SeedCeParams
         for (int k = 0; k < p.K; k++) zmax = fmaxf(zmax, __ldg(z + (size_t)k * HW + pix));
         float sum = 0.f;
         for (int k = 0; k < p.K; k++) sum += expf(__ldg(z + (size_t)k * HW + pix) - zmax);
-        lsum += (logf(sum) + zmax) - __ldg(z + (size_t)label * HW + pix);   // -log_softmax(z)[label]
+        // -log_softmax(z)[label], rounded like torch's (z - max) - log(sum): forming log(sum) + zmax first would
+        // round a confident pixel's loss (~e^-margin) at the magnitude of zmax
+        lsum += (zmax - __ldg(z + (size_t)label * HW + pix)) + logf(sum);
         cnt++;
     }
 #pragma unroll

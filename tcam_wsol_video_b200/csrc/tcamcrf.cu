@@ -3254,7 +3254,7 @@ size_t tcam_roi_components_scratch_bytes(int B, int H, int W)
 }
 
 int tcam_roi_components(const float *cams_dev, const float *thresh_dev, long long *roi_dev, float *bbox_mask_dev,
-                        int *bbox_dev, int B, int H, int W, int largest_only, float p_min_area, void *scratch_dev,
+                        int *bbox_dev, int B, int H, int W, int largest_only, double p_min_area, void *scratch_dev,
                         size_t scratch_bytes, void *cuda_stream)
 {
     if (!cams_dev || !thresh_dev || !roi_dev || !bbox_mask_dev || !bbox_dev || !scratch_dev)
@@ -3272,7 +3272,7 @@ int tcam_roi_components(const float *cams_dev, const float *thresh_dev, long lon
     // min_area = (h * w) * p_min_area_roi in float64 (tcam_seeding.py:364)
     roi_components_kernel<<<B, kSeedThreads, 0, (cudaStream_t)cuda_stream>>>(
         cams_dev, thresh_dev, roi_dev, bbox_mask_dev, bbox_dev, labels, area, sum, H, W, largest_only ? 1 : 0,
-        (double)((long long)H * W) * (double)p_min_area);
+        (double)((long long)H * W) * p_min_area);
     CUDA_TRY(cudaGetLastError());
     return TCAMCRF_OK;
 }

@@ -48,7 +48,7 @@ ROI_SELECT = [ROI_ALL, ROI_H_DENSITY, ROI_LARGEST]
 class SparseSeeds(object):
     """The seeder's output before it is painted into a label map: the selected pixel indices ``sel`` [B,2,kmax] int32
     (side 0 = foreground, 1 = background, -1 = unused) with the dilation size and the ignore index that turn them into
-    labels.  ``SelfLearningTcams`` / ``FusedTcamLosses`` take it as ``seeds`` and compute the cross-entropy from the
+    labels.  Unused slots are trailing: ``dense()`` (``seed_labels_kernel``) stops reading a side at its first -1.  ``SelfLearningTcams`` / ``FusedTcamLosses`` take it as ``seeds`` and compute the cross-entropy from the
     2*kmax*ksz^2 labelled pixels per sample directly (the map is 99.96 % ignore with the README recipe); ``dense()``
     paints the reference's [B,H,W] long map when something else needs it."""
 

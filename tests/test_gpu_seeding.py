@@ -128,14 +128,22 @@ def test_seeder_api_surface(torch_cuda):
     assert ((seeds == 1) <= (eroded == 1)).all()
 
 
-@pytest.mark.parametrize("kind", ["bilinear", "uniform", "quantised", "flat"])
-def test_otsu_roi_matches_numpy_restatement(torch_cuda, kind):
+OTSU_CASES = [pytest.param(kind, (224, 224), id=kind) for kind in ("bilinear", "uniform", "quantised", "flat")]
+OTSU_CASES += [pytest.param(kind, shape, id=f"{kind}-{shape[0]}x{shape[1]}")
+               for shape in ((1, 1), (1, 2), (2, 1), (1, 300)) for kind in ("bilinear", "uniform", "two_valued")]
+OTSU_CASES += [pytest.param(kind, shape, id=f"{kind}-{shape[0]}x{shape[1]}")
+               for shape in ((224, 224), (1, 300)) for kind in ("two_valued", "outlier", "unnormalised")]
+
+
+@pytest.mark.parametrize("kind,shape", OTSU_CASES)
+def test_otsu_roi_matches_numpy_restatement(torch_cuda, kind, shape):
     """tcam_otsu_roi vs the reference's CPU recipe (np.histogram + scikit-image's Otsu restated): same
-    threshold bit for bit and the same mask, on CAM-like, uniform, heavily tied and flat inputs."""
+    threshold bit for bit and the same mask, on CAM-like, uniform, heavily tied and flat inputs, two-valued maps, a
+    flat map with one outlier and an unnormalised map in [-3, 40], at 224x224 and on 1x1, 1x2, 2x1 and 1x300 frames."""
     torch = torch_cuda
     from oracle import seeding as ref
     from tcam_wsol_video_b200 import ops
-    b, h, w = 6, 224, 224
+    b, (h, w) = 6, shape
     g = torch.Generator().manual_seed(17)
     if kind == "bilinear":
         cam = torch.nn.functional.interpolate(torch.rand((b, 1, 28, 28), generator=g), size=(h, w), mode="bilinear",
@@ -144,6 +152,13 @@ def test_otsu_roi_matches_numpy_restatement(torch_cuda, kind):
         cam = torch.rand((b, 1, h, w), generator=g)
     elif kind == "quantised":
         cam = torch.randint(0, 7, (b, 1, h, w), generator=g).float() / 9 + 0.01
+    elif kind == "two_valued":
+        cam = torch.where(torch.rand((b, 1, h, w), generator=g) < 0.3, 0.8, 0.15)
+    elif kind == "outlier":
+        cam = torch.full((b, 1, h, w), 0.4)
+        cam.view(b, -1)[torch.arange(b), torch.randint(0, h * w, (b,), generator=g)] = 0.9
+    elif kind == "unnormalised":
+        cam = torch.rand((b, 1, h, w), generator=g) * 43 - 3
     else:
         cam = torch.full((b, 1, h, w), 0.3)
         cam[1] = torch.rand((1, h, w), generator=g) * 0.5       # one non-flat sample among flat ones
@@ -394,3 +409,93 @@ def test_roi_components_match_the_reference_class_run_with_opencv(torch_cuda):
         assert np.array_equal(roi.cpu().numpy(), g[f"c{ci}_roi"]), ci
         assert np.array_equal(bbox.cpu().numpy(), g[f"c{ci}_bbox"]), ci
         assert np.array_equal(mask.cpu().numpy(), g[f"c{ci}_mask"]), ci
+
+
+def _dyadic_cam(mask, seed):
+    """mask [h,w] bool -> cam: foreground pixels take dyadic values in [0.5, 1) (exact float32 and float64 sums in
+    any order), background 0."""
+    rng = np.random.default_rng(seed)
+    return np.where(mask, 0.5 + rng.integers(0, 32, mask.shape) / 64.0, 0.0).astype(np.float32)
+
+
+def _roi_shapes():
+    """(name, cam [h,w] float32, p_min_area) drawn to stress the union-find, the tie-breaking and the selection."""
+    shapes = []
+
+    def serpentine(h, w):
+        y, x = np.mgrid[0:h, 0:w]
+        return (y % 2 == 0) | ((y % 4 == 1) & (x == w - 1)) | ((y % 4 == 3) & (x == 0))
+
+    for h, w in ((640, 640), (37, 61)):
+        shapes.append((f"serpentine{h}x{w}", _dyadic_cam(serpentine(h, w), h), 0.05))
+    h, w = 96, 96
+    y, x = np.mgrid[0:h, 0:w] - (h - 1) / 2.0
+    phase = np.mod(np.hypot(y, x) - 12.0 * np.arctan2(y, x) / (2 * np.pi), 12.0)
+    shapes.append(("spirals", np.where(phase < 4, 0.75, np.where((phase >= 6) & (phase < 10), 0.625, 0.0))
+                   .astype(np.float32), 0.05))
+    comb = np.zeros((50, 40), bool)
+    comb[:, ::2] = True
+    comb[-1] = True                                              # the teeth join only in the last row
+    shapes.append(("comb", _dyadic_cam(comb, 3), 0.05))
+    stairs = np.zeros((40, 50), bool)
+    for i in range(0, 38, 2):
+        stairs[i:i + 2, i:i + 2] = True                          # 2x2 blocks touching only at corners
+    for i in range(40):
+        stairs[i, min(49, 45 - i)] = True                        # an anti-diagonal line: single pixels
+    shapes.append(("diagonal", _dyadic_cam(stairs, 4), 0.05))
+    y, x = np.mgrid[0:37, 0:53]
+    shapes.append(("checkerboard", np.where((x + y) % 2 == 0, 0.75, 0.0).astype(np.float32), 0.0005))
+    ties = np.zeros((40, 50), np.float32)
+    block = np.array([[0.5, 0.75, 0.875], [0.625, 0.9375, 0.5], [0.75, 0.5, 0.5625]], np.float32)
+    for k, (y0, x0) in enumerate([(30, 5), (3, 40), (3, 10), (20, 25)]):
+        ties[y0:y0 + 3, x0:x0 + 3] = np.rot90(block, k)          # same values, another order: same sum exactly
+    shapes.append(("equal_density", ties, 0.004))   # min area 8: the densest is kept
+    # the p_min_area boundary: the densest component's area is exactly H*W*p (kept) or one less (the largest wins)
+    for (h, w, p, dense_hw, big_hw) in ((40, 50, 0.05, (10, 10), (15, 20)), (100, 100, 0.05, (20, 25), (30, 30)),
+                                        (10, 10, 0.6, (6, 10), (3, 10))):
+        for drop in (0, 1):
+            cam = np.zeros((h, w), np.float32)
+            cam[:dense_hw[0], :dense_hw[1]] = 0.9375
+            if drop:
+                cam[0, 0] = 0.0
+            cam[h - big_hw[0]:, w - big_hw[1]:] = 0.5
+            assert (cam == 0.9375).sum() == h * w * p - drop
+            shapes.append((f"min_area{h}x{w}_p{p}_minus{drop}", cam, p))
+    border = np.zeros((30, 45), bool)
+    border[10:20, 40:] = True                                    # touches the right border
+    border[25:, 5:15] = True                                     # touches the bottom border
+    border[26:, 30:] = True                                      # the bottom-right corner
+    shapes.append(("borders", _dyadic_cam(border, 5), 0.05))
+    rng = np.random.default_rng(6)
+    for h, w in ((1, 64), (64, 1), (1, 1)):
+        shapes.append((f"line{h}x{w}", _dyadic_cam(rng.random((h, w)) < 0.5, h + w), 0.05))
+        shapes.append((f"full{h}x{w}", _dyadic_cam(np.ones((h, w), bool), 7), 0.05))
+    shapes.append(("full", _dyadic_cam(np.ones((33, 47), bool), 8), 0.05))
+    shapes.append(("empty", np.zeros((33, 47), np.float32), 0.05))
+    return shapes
+
+
+@pytest.mark.parametrize("method", ["roi_high_density", "largest"])
+@pytest.mark.parametrize("thresh", [0.5, None], ids=["fixed", "otsu"])
+def test_roi_components_on_drawn_shapes(torch_cuda, method, thresh):
+    """roi_components_kernel on masks drawn to break it: a serpentine and two interleaved spirals (long union chains),
+    a comb joined in its last row, corner-touching blocks (4-connectivity), a checkerboard and equal-density
+    components (exact ties: the first component in raster order wins), the p_min_area boundary (area exactly H*W*p
+    is kept), border-touching components, 1xW / Hx1 / 1x1 frames, full and empty frames.  Every shape runs alone and
+    batched with the other shapes of its frame size; roi, bbox and bbox mask must equal the restatement's exactly."""
+    torch = torch_cuda
+    from oracle import seeding as oseed
+    from tcam_wsol_video_b200 import ops
+    groups = {}
+    for name, cam, p in _roi_shapes():
+        groups.setdefault((cam.shape, p), []).append((name, cam))
+    for (_, p), items in groups.items():
+        batch = torch.from_numpy(np.stack([cam for _, cam in items])).cuda()
+        batched = ops.roi_components(batch, method == "largest", p, thresh)
+        for i, (name, cam) in enumerate(items):
+            want = oseed.roi_components_single_cam(cam, method, p, thresh=thresh)
+            alone = ops.roi_components(batch[i:i + 1], method == "largest", p, thresh)
+            for got in ((batched[0][i], batched[1][i], batched[2][i]), (alone[0][0], alone[1][0], alone[2][0])):
+                assert np.array_equal(got[0].cpu().numpy(), want[0]), name
+                assert np.array_equal(got[2].cpu().numpy().reshape(1, 4), want[2]), name
+                assert np.array_equal(got[1].cpu().numpy(), want[1]), name

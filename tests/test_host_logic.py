@@ -100,7 +100,7 @@ def test_library_exports_every_declared_symbol():
     assert declared == set(_lib.SIGNATURES), declared ^ set(_lib.SIGNATURES)
     for name in declared:
         assert hasattr(lib, name), f"{name} declared in include/tcamcrf.h but not exported"
-    assert lib.tcamcrf_version() == 103
+    assert lib.tcamcrf_version() == 104
 
 
 def test_workspace_sizing_and_argument_validation():

@@ -289,3 +289,36 @@ def test_flat_dilation_agrees_with_opencv():
         for b in range(2):
             want = cv2.dilate(x[b, 0], np.ones((k, k), np.uint8))
             assert np.array_equal(got[b, 0], want), k
+
+
+@pytest.mark.parametrize("ksz", [1, 2, 3, 4, 5])
+def test_seed_labels_from_sel_repaints_the_seeder(ksz):
+    """seed_labels_from_sel (the label map of a [B,2,kmax] selection, which the sparse cross-entropy tests compare the
+    kernels with) must repaint tcam_seeder_forward's map from the seeds the restated seeder picked: odd and even
+    windows, windows that overlap on one side, fg/bg conflicts, a sample without seeds."""
+    import torch
+    from oracle import seeding as oseed
+    b, h, w, k = 4, 13, 17, 12
+    cam = torch.rand((b, 1, h, w), generator=torch.Generator().manual_seed(ksz))
+    cam[2] = 0.5                                                 # flat: no seeds
+    kw = dict(seed_tech="seed_uniform", min_=k, max_=k, min_p=0.5, max_p=0.5, use_roi=False)
+    torch.manual_seed(11)
+    want = oseed.tcam_seeder_forward(cam, None, ksz=ksz, ignore_idx=-255, **kw)
+    torch.manual_seed(11)                                        # the same draws, sample by sample
+    sel = torch.full((b, 2, k), -1, dtype=torch.int32)
+    fg, bg = torch.zeros((b, h, w), dtype=torch.long), torch.zeros((b, h, w), dtype=torch.long)
+    for i in range(b):
+        fg[i], bg[i] = oseed.one_sample(cam[i, 0], None, **{n: kw[n] for n in ("min_p", "max_p", "min_", "max_",
+                                                                              "seed_tech", "use_roi")})
+        for side, m in enumerate((fg[i], bg[i])):
+            idx = torch.nonzero(m.reshape(-1)).flatten()
+            sel[i, side, :idx.numel()] = idx.int()
+    got = oseed.seed_labels_from_sel(sel, ksz, h, w, -255)
+    assert torch.equal(got, want)
+    assert (sel[2] == -1).all() and (got[2] == -255).all()
+    if ksz > 1:
+        dil_fg = oseed.flat_dilation(fg.unsqueeze(1), ksz).squeeze(1)
+        dil_bg = oseed.flat_dilation(bg.unsqueeze(1), ksz).squeeze(1)
+        assert ((dil_fg == 1) & (dil_bg == 1)).any()             # conflicts: ignored
+        win = torch.nn.functional.conv2d(fg.unsqueeze(1).float(), torch.ones(1, 1, ksz, ksz), padding=ksz - 1)
+        assert (win > 1).any()                                   # windows overlapping on one side
