@@ -56,6 +56,11 @@ extern "C" {
 #define TCAMCRF_DEV_POOL_FULL 2   /* vertex pool overflowed */
 #define TCAMCRF_DEV_KEY_RANGE 4   /* lattice coordinate outside the packed-key range */
 
+/* element types of logits (the *_typed entry points) */
+#define TCAMCRF_DTYPE_F32 0  /* float32 */
+#define TCAMCRF_DTYPE_F16 1  /* IEEE half */
+#define TCAMCRF_DTYPE_BF16 2 /* bfloat16 */
+
 /* feature kinds */
 #define TCAMCRF_FEAT_XY_RGB 0 /* (x/sxy, y/sxy, c0/srgb, ..): d = 2 + channels; reference bilateralfilter: channels = 3 */
 #define TCAMCRF_FEAT_COLOR 1  /* (c0/srgb, ..): d = channels; reference colorbilateralfilter */
@@ -181,6 +186,27 @@ int tcamcrf_loss_backward_logits(const float *as_dev, const float *logits_dev, c
 int tcamcrf_loss_backward_logits_weighted(const float *as_dev, const float *logits_dev, const float *grad_out_dev,
                                           float *grad_logits_dev, int N, int K, int H, int W, float n_norm,
                                           float weight, void *cuda_stream);
+
+/* The logits entry points for logits of any TCAMCRF_DTYPE_* element type: what a model run under autocast hands
+ * the loss (fp16 or bf16), read as they are, with no float32 copy.  Logits are widened on load (exact) and
+ * everything after is the float32 computation: AS, the loss and the workspace stay float32, and the gradient is
+ * written in the logits' type, rounded once from the float32 value.  Given the same AS, the gradient has the bits of
+ * the float32 entry point on the widened logits followed by a cast to the logits' type.  Logits must be aligned to
+ * their element size.  The float32 entry points above are these with TCAMCRF_DTYPE_F32.  An unknown dtype code
+ * returns TCAMCRF_ERR_INVALID. */
+int tcamcrf_loss_forward_logits_typed(const tcamcrf_config *cfg, const void *images_dev, int images_u8,
+                                      const void *logits_dev, int logits_dtype, float *as_dev, float *loss_dev, int N,
+                                      int K, int H, int W, float n_norm, void *workspace, size_t workspace_bytes,
+                                      void *cuda_stream);
+/* tcamcrf_loss_forward_host_frames with logits != 0, for logits of any TCAMCRF_DTYPE_* type. */
+int tcamcrf_loss_forward_host_frames_typed(const tcamcrf_config *cfg, const void *images_host, void *images_stage_dev,
+                                           int images_u8, const void *logits_dev, int logits_dtype, float *as_dev,
+                                           float *loss_dev, int N, int K, int H, int W, float n_norm, void *workspace,
+                                           size_t workspace_bytes, void *cuda_stream);
+/* grad_logits_dev has the logits' element type. */
+int tcamcrf_loss_backward_logits_typed(const float *as_dev, const void *logits_dev, int logits_dtype,
+                                       const float *grad_out_dev, void *grad_logits_dev, int N, int K, int H, int W,
+                                       float n_norm, float weight, void *cuda_stream);
 
 /* Reads the device status word of a workspace (synchronises the stream).  Returns 0 or TCAMCRF_DEV_* bits
  * in *dev_status; also writes the number of lattice vertices of the last chunk to *vertices (may be NULL). */
@@ -321,6 +347,27 @@ int tcam_seed_ce_forward(const float *logits_dev, const int *sel_dev, int kmax, 
 int tcam_seed_ce_backward(const float *logits_dev, const int *sel_dev, int kmax, int B, int K, int H, int W, int ksz,
                           const float *count_dev, const float *grad_out_dev, float scale, float *grad_logits_dev,
                           void *cuda_stream);
+
+/* The same for logits of any TCAMCRF_DTYPE_* element type (see tcamcrf_loss_forward_logits_typed); the loss, count
+ * and total stay float32.  The backward's grad_logits_dev has the logits' type: each labelled element becomes
+ * round(widen(old) + (grad_out * scale) * d loss / d logits), one rounding. */
+int tcam_seed_ce_forward_typed(const void *logits_dev, int logits_dtype, const int *sel_dev, int kmax, int B, int K,
+                               int H, int W, int ksz, float *scratch_dev, float *loss_dev, float *count_dev,
+                               const float *add_dev, float weight, float *total_dev, void *cuda_stream);
+int tcam_seed_ce_backward_typed(const void *logits_dev, int logits_dtype, const int *sel_dev, int kmax, int B, int K,
+                                int H, int W, int ksz, const float *count_dev, const float *grad_out_dev, float scale,
+                                void *grad_logits_dev, void *cuda_stream);
+
+/* Backward of crf_weight * CRF(softmax(logits)) + ce_weight * CE(logits, seeds) (the forward being
+ * tcamcrf_loss_forward_logits_typed with loss_weight = crf_weight and tcam_seed_ce_forward_typed): writes
+ * grad_logits_dev [B,K,H,W] (the logits' type) = tcamcrf_loss_backward_logits_typed(weight = crf_weight), with the
+ * cross-entropy's gradient (scale = ce_weight) added on the labelled pixels.  Every element is rounded once from its
+ * float32 value: the bits of the float32 sequence (CRF gradient, then tcam_seed_ce_backward in place) cast to the
+ * logits' type. */
+int tcam_crf_seed_ce_backward_typed(const float *as_dev, const void *logits_dev, int logits_dtype, const int *sel_dev,
+                                    int kmax, int ksz, const float *count_dev, const float *grad_out_dev, int B, int K,
+                                    int H, int W, float n_norm, float crf_weight, float ce_weight,
+                                    void *grad_logits_dev, void *cuda_stream);
 
 /* ROI of every CAM of a batch by Otsu's threshold: roi = (cam*255 >= otsu(floor(cam*255))), 1/0 as int64, the
  * 'roi_all' branch of GetRoiSingleCam (dlib/cams/tcam_seeding.py:316-345,419-430; scikit-image threshold_otsu

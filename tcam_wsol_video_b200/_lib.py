@@ -29,6 +29,11 @@ FEAT_COLOR = 1
 
 STAGES = ("build", "neighbour", "splat", "blur", "slice", "loss", "backward", "prepare", "seed")
 
+# element types of logits (TCAMCRF_DTYPE_*)
+DTYPE_F32 = 0
+DTYPE_F16 = 1
+DTYPE_BF16 = 2
+
 DEV_TABLE_FULL = 1
 DEV_POOL_FULL = 2
 DEV_KEY_RANGE = 4
@@ -134,6 +139,20 @@ SIGNATURES = {
                                      c_void_p, c_void_p, c_float, c_void_p, c_void_p]),
     "tcam_seed_ce_backward": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p,
                                       c_float, c_void_p, c_void_p]),
+    "tcamcrf_loss_forward_logits_typed": (c_int, [_cfgp, c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int,
+                                                  c_int, c_int, c_float, c_void_p, c_size_t, c_void_p]),
+    "tcamcrf_loss_forward_host_frames_typed": (c_int, [_cfgp, c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p,
+                                                       c_void_p, c_int, c_int, c_int, c_int, c_float, c_void_p, c_size_t,
+                                                       c_void_p]),
+    "tcamcrf_loss_backward_logits_typed": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_int,
+                                                   c_int, c_float, c_float, c_void_p]),
+    "tcam_seed_ce_forward_typed": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p,
+                                           c_void_p, c_void_p, c_void_p, c_float, c_void_p, c_void_p]),
+    "tcam_seed_ce_backward_typed": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int,
+                                            c_void_p, c_void_p, c_float, c_void_p, c_void_p]),
+    "tcam_crf_seed_ce_backward_typed": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_void_p, c_void_p,
+                                                c_int, c_int, c_int, c_int, c_float, c_float, c_float, c_void_p,
+                                                c_void_p]),
     "tcam_seed_fused_supported": (c_int, [c_int, c_int]),
     "tcam_seed_fused": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_float, c_int, c_int,
                                 c_int, c_int, c_int, c_int, c_int, c_int, c_int, ctypes.c_longlong, c_void_p, c_void_p,

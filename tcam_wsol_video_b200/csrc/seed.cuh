@@ -17,9 +17,45 @@
 #pragma once
 #include <cstdint>
 #include <cooperative_groups.h>
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
 namespace tcamcrf {
+
+// Logits are read through ld_logit: float32 as they are, or 2-byte logits (fp16 or bf16, what autocast hands the
+// losses) widened on load.  Widening is exact, so everything after the load is the float32 code, bit for bit.  The
+// 2-byte element type is a run-time flag (uniform over a launch) rather than a template axis: one instantiation per
+// kernel variant serves both types.
+struct Logits16 {
+    const unsigned short *z;
+    int bf16;
+    __device__ __forceinline__ Logits16 operator+(size_t o) const { return {z + o, bf16}; }
+};
+__device__ __forceinline__ float ld_logit(const float *z) { return __ldg(z); }
+__device__ __forceinline__ float ld_logit(Logits16 z)
+{
+    const unsigned short u = __ldg(z.z);
+    return z.bf16 ? __bfloat162float(__ushort_as_bfloat16(u)) : __half2float(__ushort_as_half(u));
+}
+
+// A gradient in the logits' 2-byte type: the float32 value, rounded once to nearest even (what casting the float32
+// gradient to the logits' dtype does)
+struct Grad16 {
+    unsigned short *g;
+    int bf16;
+    __device__ __forceinline__ Grad16 operator+(size_t o) const { return {g + o, bf16}; }
+};
+__device__ __forceinline__ void st_grad(float *g, float v) { *g = v; }
+__device__ __forceinline__ void st_grad(Grad16 g, float v)
+{
+    *g.g = g.bf16 ? __bfloat16_as_ushort(__float2bfloat16_rn(v)) : __half_as_ushort(__float2half_rn(v));
+}
+__device__ __forceinline__ float ld_grad(Grad16 g)
+{
+    const unsigned short u = *g.g;
+    return g.bf16 ? __bfloat162float(__ushort_as_bfloat16(u)) : __half2float(__ushort_as_half(u));
+}
 
 constexpr int kSeedThreads = 1024;
 
@@ -957,7 +993,7 @@ __global__ void __launch_bounds__(kSeedFusedThreads) seed_fused_kernel(const See
 // sides cover it -- exactly seed_labels_kernel's rule (tcam_seeding.py:239-254).  Same value and gradient as torch's
 // call on the label map; the sums run in a fixed order (one block per sample, ticketed final fold): deterministic.
 struct SeedCeParams {
-    const float *logits;   // [B][K][HW]
+    const void *logits;    // [B][K][HW]: float32, or 2-byte logits for seed_ce_forward_lowp_kernel
     const int *sel;        // [B][2][kmax]
     float *partial;        // [B][2]: loss sum, labelled pixels of the sample
     int *ticket;           // [1], zero before the first call; left at zero
@@ -967,6 +1003,7 @@ struct SeedCeParams {
     float *total_out;      // optional [1]: add + weight * loss
     float weight;
     int B, K, H, W, kmax, ksz;
+    int bf16;              // 2-byte logits: bf16 (1) or fp16 (0)
 };
 
 // label of window pixel `off` of seed j on `side`, or -1 when the item does not count (outside the frame, an earlier
@@ -994,7 +1031,8 @@ __device__ __forceinline__ int seed_window_label(const int *sel_b, int kmax, int
     return side == 0 ? 1 : 0;                     // side 0 = foreground seeds -> class 1
 }
 
-__global__ void __launch_bounds__(256) seed_ce_forward_kernel(const SeedCeParams p)
+template <typename Z>
+__device__ __forceinline__ void seed_ce_forward_body(const SeedCeParams &p, Z logits)
 {
     __shared__ float s_l[8];
     __shared__ int s_c[8];
@@ -1002,7 +1040,7 @@ __global__ void __launch_bounds__(256) seed_ce_forward_kernel(const SeedCeParams
     const int b = blockIdx.x;
     const int HW = p.H * p.W;
     const int *sel_b = p.sel + (size_t)b * 2 * p.kmax;
-    const float *z = p.logits + (size_t)b * p.K * HW;
+    const Z z = logits + (size_t)b * p.K * HW;
     const int win = p.ksz * p.ksz, items = 2 * p.kmax * win;
     float lsum = 0.f;
     int cnt = 0;
@@ -1012,12 +1050,12 @@ __global__ void __launch_bounds__(256) seed_ce_forward_kernel(const SeedCeParams
         const int label = seed_window_label(sel_b, p.kmax, p.ksz, p.H, p.W, side, rest / win, rest % win, pix);
         if (label < 0) continue;
         float zmax = -INFINITY;
-        for (int k = 0; k < p.K; k++) zmax = fmaxf(zmax, __ldg(z + (size_t)k * HW + pix));
+        for (int k = 0; k < p.K; k++) zmax = fmaxf(zmax, ld_logit(z + (size_t)k * HW + pix));
         float sum = 0.f;
-        for (int k = 0; k < p.K; k++) sum += expf(__ldg(z + (size_t)k * HW + pix) - zmax);
+        for (int k = 0; k < p.K; k++) sum += expf(ld_logit(z + (size_t)k * HW + pix) - zmax);
         // -log_softmax(z)[label], rounded like torch's (z - max) - log(sum): forming log(sum) + zmax first would
         // round a confident pixel's loss (~e^-margin) at the magnitude of zmax
-        lsum += (zmax - __ldg(z + (size_t)label * HW + pix)) + logf(sum);
+        lsum += (zmax - ld_logit(z + (size_t)label * HW + pix)) + logf(sum);
         cnt++;
     }
 #pragma unroll
@@ -1053,6 +1091,17 @@ __global__ void __launch_bounds__(256) seed_ce_forward_kernel(const SeedCeParams
     p.count_out[0] = n;
     if (p.total_out) p.total_out[0] = __fadd_rn(p.add ? p.add[0] : 0.f, __fmul_rn(ce, p.weight));
     *p.ticket = 0;
+}
+
+__global__ void __launch_bounds__(256) seed_ce_forward_kernel(const SeedCeParams p)
+{
+    seed_ce_forward_body(p, static_cast<const float *>(p.logits));
+}
+
+// the same on fp16 / bf16 logits (the loss stays float32)
+__global__ void __launch_bounds__(256) seed_ce_forward_lowp_kernel(const SeedCeParams p)
+{
+    seed_ce_forward_body(p, Logits16{static_cast<const unsigned short *>(p.logits), p.bf16});
 }
 
 // grad[b][k][pix] += (g * scale) * (softmax_k - [k == label]) / count   on the labelled pixels (every labelled pixel

@@ -115,6 +115,8 @@ static Tuning &tuning()
 constexpr int kThreads = 256;
 constexpr int kFlagLogits = 1;        // segs holds logits, softmax on the fly
 constexpr int kFlagReverseBlur = 2;   // blur axes d..0: the transposed filter
+constexpr int kFlagLowp = 4;          // with kFlagLogits: the logits are 2-byte (fp16, or bf16 with kFlagBF16)
+constexpr int kFlagBF16 = 8;
 
 
 
@@ -946,7 +948,8 @@ __device__ __forceinline__ void store_vec(float *addr, const float (&v)[V])
 }
 
 struct PixelParams {
-    const float *segs;      // [n][K][P]: class probabilities, or logits when `logits` is set
+    const void *segs;       // [n][K][P]: float32 class probabilities, or logits when `logits` is set (2-byte
+                            // logits for the *_lowp kernels)
     int logits;             // 1: segs holds logits; softmax over K is taken on the fly (never stored)
     float *as_out;          // [n][K][P]
     int *offset;            // [n][r][P]; entry index on entry to splat, dense id afterwards
@@ -964,26 +967,43 @@ struct PixelParams {
     int dense;              // host-side hint: the lattices of this workspace have been dense lately (splat variant)
     long long pool;
     float alpha;
+    int bf16;               // *_lowp kernels: the logits are bf16 (1) or fp16 (0)
 };
+
+// The segmentations of a launch as the body of a pixel kernel reads them: float32, or 2-byte logits (*_lowp kernels)
+template <typename Z>
+__device__ __forceinline__ Z segs_of(const PixelParams &p);
+template <>
+__device__ __forceinline__ const float *segs_of<const float *>(const PixelParams &p)
+{
+    return static_cast<const float *>(p.segs);
+}
+template <>
+__device__ __forceinline__ Logits16 segs_of<Logits16>(const PixelParams &p)
+{
+    return Logits16{static_cast<const unsigned short *>(p.segs), p.bf16};
+}
 
 // softmax over the K planes of one pixel without storing it: max and sum first, then
 // prob_k = exp(z_k - max) / sum, the order of operations of torch's softmax forward
 struct SoftmaxStat {
     float zmax, sum;
 };
-__device__ __forceinline__ SoftmaxStat softmax_stat(const float *z, int K, int P)
+// (Z: const float * or Logits16, see ld_logit)
+template <typename Z>
+__device__ __forceinline__ SoftmaxStat softmax_stat(Z z, int K, int P)
 {
     SoftmaxStat s;
     s.zmax = -INFINITY;
-    for (int k = 0; k < K; k++) s.zmax = fmaxf(s.zmax, __ldg(z + (size_t)k * P));
+    for (int k = 0; k < K; k++) s.zmax = fmaxf(s.zmax, ld_logit(z + (size_t)k * P));
     s.sum = 0.f;
-    for (int k = 0; k < K; k++) s.sum += expf(__ldg(z + (size_t)k * P) - s.zmax);
+    for (int k = 0; k < K; k++) s.sum += expf(ld_logit(z + (size_t)k * P) - s.zmax);
     return s;
 }
-template <bool L>
-__device__ __forceinline__ float seg_value(const float *z, int k, int P, const SoftmaxStat &st)
+template <bool L, typename Z>
+__device__ __forceinline__ float seg_value(Z z, int k, int P, const SoftmaxStat &st)
 {
-    const float v = __ldg(z + (size_t)k * P);
+    const float v = ld_logit(z + (size_t)k * P);
     return L ? __fdiv_rn(expf(v - st.zmax), st.sum) : v;
 }
 
@@ -994,9 +1014,10 @@ __device__ __forceinline__ float seg_value(const float *z, int k, int P, const S
 // the same bits.
 struct Prob2 {
     float p0, p1;
-    __device__ __forceinline__ void load(const float *z, int P)
+    template <typename Z>
+    __device__ __forceinline__ void load(Z z, int P)
     {
-        const float z0 = __ldg(z), z1 = __ldg(z + P);
+        const float z0 = ld_logit(z), z1 = ld_logit(z + P);
         const float zmax = fmaxf(fmaxf(-INFINITY, z0), z1);
         const float e0 = expf(z0 - zmax), e1 = expf(z1 - zmax);
         const float sum = (0.f + e0) + e1;
@@ -1006,13 +1027,16 @@ struct Prob2 {
     __device__ __forceinline__ float get(int k) const { return k == 0 ? p0 : p1; }
 };
 
-template <int D, int V, bool L>
-__global__ void __launch_bounds__(kThreads) splat_kernel(const PixelParams p)
+// Pixel-kernel bodies shared by the float32 kernels and their *_lowp twins (Z: the logits' source, see segs_of).
+// `tid` is threadIdx.x read by the kernel itself, where __launch_bounds__ bounds it: read inside the inlined body the
+// bound is lost and the index arithmetic compiles to other (slower to issue) instructions.
+template <int D, int V, bool L, typename Z>
+__device__ __forceinline__ void splat_body(const PixelParams p, unsigned int tid)
 {
     const int n = blockIdx.y;
-    const int pix = blockIdx.x * kThreads + threadIdx.x;
+    const int pix = blockIdx.x * kThreads + tid;
     const bool valid = pix < p.P;
-    const int lane = threadIdx.x & 31;
+    const int lane = tid & 31;
     const size_t base = (size_t)(p.frame0 + n) * (D + 1) * p.P + (valid ? pix : 0);
     int id[D + 1];
     float w[D + 1];
@@ -1043,7 +1067,7 @@ __global__ void __launch_bounds__(kThreads) splat_kernel(const PixelParams p)
         }
         id[r] = v;
     }
-    const float *seg = p.segs + (size_t)n * p.K * p.P + (valid ? pix : 0);
+    const Z seg = segs_of<Z>(p) + (size_t)n * p.K * p.P + (valid ? pix : 0);
     SoftmaxStat sm = {0.f, 1.f};
     Prob2 p2 = {0.f, 0.f};
     const bool two = L && p.K == 2;
@@ -1094,6 +1118,19 @@ __global__ void __launch_bounds__(kThreads) splat_kernel(const PixelParams p)
     }
 }
 
+template <int D, int V, bool L>
+__global__ void __launch_bounds__(kThreads) splat_kernel(const PixelParams p)
+{
+    splat_body<D, V, L, const float *>(p, threadIdx.x);
+}
+
+// the same from fp16 / bf16 logits
+template <int D, int V>
+__global__ void __launch_bounds__(kThreads) splat_lowp_kernel(const PixelParams p)
+{
+    splat_body<D, V, true, Logits16>(p, threadIdx.x);
+}
+
 // ---------------------------------------------------------------------------------------------------------
 // Row-cooperative splat for value rows of 2..4 float4s (K = 5..16), used on DENSE lattices.
 //
@@ -1120,8 +1157,8 @@ struct RowMap {
     static constexpr int kPpb = (kThreads / 32) * kPpw;        // pixels per block
 };
 
-template <int D, int KV, bool L>
-__global__ void __launch_bounds__(kThreads) splat_rows_kernel(const PixelParams p)
+template <int D, int KV, bool L, typename Z>
+__device__ __forceinline__ void splat_rows_body(const PixelParams p, unsigned int tid)
 {
     constexpr int kPpw = RowMap<KV>::kPpw, kPpb = RowMap<KV>::kPpb;
     constexpr int Kp = 4 * KV;
@@ -1134,7 +1171,7 @@ __global__ void __launch_bounds__(kThreads) splat_rows_kernel(const PixelParams 
     const int npix = min(kPpb, p.P - pix0);
     const size_t base = (size_t)(p.frame0 + n) * (D + 1) * p.P + pix0;
     // ahead of the wait (see splat_kernel): coalesced loads, id look-ups
-    for (int t = threadIdx.x; t < (D + 1) * kPpb; t += kThreads) {
+    for (int t = tid; t < (D + 1) * kPpb; t += kThreads) {
         const int r = t / kPpb, q = t - r * kPpb;
         int raw = -1, v = -1;
         float w = 0.f;
@@ -1150,13 +1187,13 @@ __global__ void __launch_bounds__(kThreads) splat_rows_kernel(const PixelParams 
         s_id[r][q] = v;
         s_w[r][q] = w;
     }
-    const float *seg = p.segs + (size_t)n * p.K * p.P + pix0;
-    for (int t = threadIdx.x; t < Kp * kPpb; t += kThreads) {
+    const Z seg = segs_of<Z>(p) + (size_t)n * p.K * p.P + pix0;
+    for (int t = tid; t < Kp * kPpb; t += kThreads) {
         const int k = t / kPpb, q = t - k * kPpb;
-        s_seg[k][q] = (k < p.K && q < npix) ? __ldg(seg + (size_t)k * p.P + q) : 0.f;
+        s_seg[k][q] = (k < p.K && q < npix) ? ld_logit(seg + (size_t)k * p.P + q) : 0.f;
     }
     __syncthreads();
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int lane = tid & 31, warp = tid >> 5;
     const int j = lane / KV, c = lane - j * KV;                // pixel slot within the warp, float4 column
     const bool lane_on = j < kPpw;
     const int q = warp * kPpw + (lane_on ? j : 0);             // pixel slot within the block
@@ -1183,7 +1220,7 @@ __global__ void __launch_bounds__(kThreads) splat_rows_kernel(const PixelParams 
     pdl_wait();   // the value rows are cleared by the previous kernel
     pdl_launch_dependents();
     // entry indices become tagged vertex ids (coalesced write-back of the fresh ones)
-    for (int t = threadIdx.x; t < (D + 1) * kPpb; t += kThreads) {
+    for (int t = tid; t < (D + 1) * kPpb; t += kThreads) {
         const int r = t / kPpb, qq = t - r * kPpb;
         if (s_raw[r][qq] >= 0) {
             const int v = s_id[r][qq];
@@ -1223,6 +1260,19 @@ __global__ void __launch_bounds__(kThreads) splat_rows_kernel(const PixelParams 
         }
         if (issue) red_add(p.values + (size_t)id[r] * Kp + 4 * c, t);
     }
+}
+
+template <int D, int KV, bool L>
+__global__ void __launch_bounds__(kThreads) splat_rows_kernel(const PixelParams p)
+{
+    splat_rows_body<D, KV, L, const float *>(p, threadIdx.x);
+}
+
+// the same from fp16 / bf16 logits
+template <int D, int KV>
+__global__ void __launch_bounds__(kThreads) splat_rows_lowp_kernel(const PixelParams p)
+{
+    splat_rows_body<D, KV, true, Logits16>(p, threadIdx.x);
 }
 
 struct BlurParams {
@@ -1328,8 +1378,8 @@ __device__ __forceinline__ void fold_loss_partials(const PixelParams &p)
     }
 }
 
-template <int D, int V, bool L>
-__global__ void __launch_bounds__(kThreads) slice_kernel(const PixelParams p)
+template <int D, int V, bool L, typename Z>
+__device__ __forceinline__ void slice_body(const PixelParams p)
 {
     __shared__ float s_red[kThreads / 32];
     const int n = blockIdx.y;
@@ -1337,7 +1387,7 @@ __global__ void __launch_bounds__(kThreads) slice_kernel(const PixelParams p)
     float dot = 0.f;
     int id[D + 1];
     float w[D + 1];
-    const float *seg = p.segs + (size_t)n * p.K * p.P + pix;
+    const Z seg = segs_of<Z>(p) + (size_t)n * p.K * p.P + pix;
     SoftmaxStat sm = {0.f, 1.f};
     Prob2 p2 = {0.f, 0.f};
     const bool two = L && p.K == 2;
@@ -1405,6 +1455,19 @@ __global__ void __launch_bounds__(kThreads) slice_kernel(const PixelParams p)
     fold_loss_partials(p);
 }
 
+template <int D, int V, bool L>
+__global__ void __launch_bounds__(kThreads) slice_kernel(const PixelParams p)
+{
+    slice_body<D, V, L, const float *>(p);
+}
+
+// the same from fp16 / bf16 logits
+template <int D, int V>
+__global__ void __launch_bounds__(kThreads) slice_lowp_kernel(const PixelParams p)
+{
+    slice_body<D, V, true, Logits16>(p);
+}
+
 // grad = ((-2*g) * AS) / n  with the reference's rounding order (dense_crf_loss.py:73)
 __global__ void __launch_bounds__(kThreads) loss_backward_kernel(const float *__restrict__ as,
                                                                  const float *__restrict__ grad_out,
@@ -1432,43 +1495,123 @@ __global__ void __launch_bounds__(kThreads) loss_backward_kernel(const float *__
     for (size_t i = n4 * 4 + tid; i < count; i += stride) grad[i] = __fdiv_rn(__fmul_rn(t, as[i]), n_norm);
 }
 
-// Backward through the CRF loss AND the softmax that produced its input, in one pass:
+// Backward through the CRF loss AND the softmax that produced its input, for one pixel:
 //   g_k = ((-2*g) * AS_k) / n   (dense_crf_loss.py:73),   dz_k = p_k * (g_k - sum_j p_j g_j)
-// thread per pixel; logits / AS / grad planar [n][K][P]
+// out(k, dz_k, p_k) receives each class's gradient and probability; z / a point at class 0 of the pixel (stride P).
+template <typename Z, typename Out>
+__device__ __forceinline__ void softmax_crf_grad(Z z, const float *a, int K, int P, float t, float n_norm, Out &&out)
+{
+    if (K == 2) {   // fg / bg: everything loaded once, the four loads in flight together
+        const float a0 = __ldg(a), a1 = __ldg(a + P);
+        Prob2 p2;
+        p2.load(z, P);
+        const float g0 = __fdiv_rn(__fmul_rn(t, a0), n_norm), g1 = __fdiv_rn(__fmul_rn(t, a1), n_norm);
+        const float inner2 = fmaf(p2.p1, g1, fmaf(p2.p0, g0, 0.f));
+        out(0, p2.p0 * (g0 - inner2), p2.p0);
+        out(1, p2.p1 * (g1 - inner2), p2.p1);
+        return;
+    }
+    const SoftmaxStat sm = softmax_stat(z, K, P);
+    float inner = 0.f;
+    for (int k = 0; k < K; k++) {
+        const float pk = __fdiv_rn(expf(ld_logit(z + (size_t)k * P) - sm.zmax), sm.sum);
+        inner = fmaf(pk, __fdiv_rn(__fmul_rn(t, __ldg(a + (size_t)k * P)), n_norm), inner);
+    }
+    for (int k = 0; k < K; k++) {
+        const float pk = __fdiv_rn(expf(ld_logit(z + (size_t)k * P) - sm.zmax), sm.sum);
+        const float gk = __fdiv_rn(__fmul_rn(t, __ldg(a + (size_t)k * P)), n_norm);
+        out(k, pk * (gk - inner), pk);
+    }
+}
+
+// T *__restrict__ for a pointer type T *, T itself otherwise
+template <typename T>
+struct Restrict {
+    using type = T;
+};
+template <typename T>
+struct Restrict<T *> {
+    using type = T *__restrict__;
+};
+
+// thread per pixel; logits / AS / grad planar [n][K][P]; G: float * or Grad16 (the logits' 2-byte type)
+template <typename Z, typename G>
+__device__ __forceinline__ void loss_backward_logits_body(const float *__restrict__ as,
+                                                          typename Restrict<Z>::type logits,
+                                                          const float *__restrict__ grad_out,
+                                                          typename Restrict<G>::type grad, int K, int P,
+                                                          long long pixels, float n_norm, float weight,
+                                                          unsigned int tid)
+{
+    const float t = __fmul_rn(-2.0f, __fmul_rn(__ldg(grad_out), weight));
+    const long long stride = (long long)gridDim.x * kThreads;
+    for (long long i = (long long)blockIdx.x * kThreads + tid; i < pixels; i += stride) {
+        // (32-bit division when the pixel index fits: a 64-bit one is ~25 instructions more per pixel)
+        const long long n = pixels <= 0x7fffffffll ? (long long)((unsigned int)i / (unsigned int)P) : i / P;
+        const size_t base = (size_t)n * K * P + (i - n * P);
+        softmax_crf_grad(logits + base, as + base, K, P, t, n_norm,
+                         [&](int k, float v, float) { st_grad(grad + (base + (size_t)k * P), v); });
+    }
+}
+
 __global__ void __launch_bounds__(kThreads) loss_backward_logits_kernel(const float *__restrict__ as,
                                                                         const float *__restrict__ logits,
                                                                         const float *__restrict__ grad_out,
                                                                         float *__restrict__ grad, int K, int P,
                                                                         long long pixels, float n_norm, float weight)
 {
-    const float t = __fmul_rn(-2.0f, __fmul_rn(__ldg(grad_out), weight));
-    const long long stride = (long long)gridDim.x * kThreads;
-    for (long long i = (long long)blockIdx.x * kThreads + threadIdx.x; i < pixels; i += stride) {
-        // (32-bit division when the pixel index fits: a 64-bit one is ~25 instructions more per pixel)
-        const long long n = pixels <= 0x7fffffffll ? (long long)((unsigned int)i / (unsigned int)P) : i / P;
-        const size_t base = (size_t)n * K * P + (i - n * P);
-        const float *z = logits + base;
-        const float *a = as + base;
-        if (K == 2) {   // fg / bg: everything loaded once, the four loads in flight together
-            const float a0 = __ldg(a), a1 = __ldg(a + P);
-            Prob2 p2;
-            p2.load(z, P);
-            const float g0 = __fdiv_rn(__fmul_rn(t, a0), n_norm), g1 = __fdiv_rn(__fmul_rn(t, a1), n_norm);
-            const float inner2 = fmaf(p2.p1, g1, fmaf(p2.p0, g0, 0.f));
-            grad[base] = p2.p0 * (g0 - inner2);
-            grad[base + P] = p2.p1 * (g1 - inner2);
-            continue;
-        }
-        const SoftmaxStat sm = softmax_stat(z, K, P);
-        float inner = 0.f;
-        for (int k = 0; k < K; k++) {
-            const float pk = __fdiv_rn(expf(__ldg(z + (size_t)k * P) - sm.zmax), sm.sum);
-            inner = fmaf(pk, __fdiv_rn(__fmul_rn(t, __ldg(a + (size_t)k * P)), n_norm), inner);
-        }
-        for (int k = 0; k < K; k++) {
-            const float pk = __fdiv_rn(expf(__ldg(z + (size_t)k * P) - sm.zmax), sm.sum);
-            const float gk = __fdiv_rn(__fmul_rn(t, __ldg(a + (size_t)k * P)), n_norm);
-            grad[base + (size_t)k * P] = pk * (gk - inner);
+    loss_backward_logits_body<const float *, float *>(as, logits, grad_out, grad, K, P, pixels, n_norm, weight,
+                                                      threadIdx.x);
+}
+
+// the same on fp16 / bf16 logits; the gradient is written in their type, rounded once from the float32 value
+__global__ void __launch_bounds__(kThreads) loss_backward_logits_lowp_kernel(const float *__restrict__ as,
+                                                                             Logits16 logits,
+                                                                             const float *__restrict__ grad_out,
+                                                                             Grad16 grad, int K, int P,
+                                                                             long long pixels, float n_norm,
+                                                                             float weight)
+{
+    loss_backward_logits_body<Logits16, Grad16>(as, logits, grad_out, grad, K, P, pixels, n_norm, weight, threadIdx.x);
+}
+
+// seed_ce_backward_kernel (seed.cuh) on fp16 / bf16 logits, with the gradient in their type.  Each labelled pixel's
+// gradient is formed in float32 and rounded ONCE: base + coef * (p_k - [k == label]), where base is
+//   as == NULL: the gradient already in `grad`, widened (exact; zero for SeedCrossEntropyFunction)
+//   as != NULL: the float32 CRF gradient of the pixel, recomputed by softmax_crf_grad exactly as
+//               loss_backward_logits_lowp_kernel formed it before rounding (t = -2 * (g * crf_weight)):
+// the float32 sequence "CRF gradient, then the cross-entropy added in place" rounded once, where adding onto the
+// already rounded value would round twice.
+__global__ void __launch_bounds__(256) seed_ce_backward_lowp_kernel(Logits16 logits, const int *__restrict__ sel,
+                                                                    Grad16 grad, const float *__restrict__ count,
+                                                                    const float *__restrict__ grad_out, float scale,
+                                                                    int K, int H, int W, int kmax, int ksz,
+                                                                    const float *__restrict__ as, float n_norm,
+                                                                    float crf_weight)
+{
+    const int b = blockIdx.x;
+    const int HW = H * W;
+    const int *sel_b = sel + (size_t)b * 2 * kmax;
+    const Logits16 z = logits + (size_t)b * K * HW;
+    const Grad16 g = grad + (size_t)b * K * HW;
+    const float coef = __fdiv_rn(__fmul_rn(__ldg(grad_out), scale), __ldg(count));
+    const float t = __fmul_rn(-2.0f, __fmul_rn(__ldg(grad_out), crf_weight));
+    const int win = ksz * ksz, items = 2 * kmax * win;
+    for (int it = threadIdx.x; it < items; it += 256) {
+        const int side = it / (kmax * win), rest = it - side * kmax * win;
+        int pix;
+        const int label = seed_window_label(sel_b, kmax, ksz, H, W, side, rest / win, rest % win, pix);
+        if (label < 0) continue;
+        // (same expression as seed_ce_backward_kernel's `g += coef * (pk - onehot)`, contracted to one fma)
+        auto add_ce = [&](int k, float base, float pk) {
+            st_grad(g + ((size_t)k * HW + pix), fmaf(coef, pk - (k == label ? 1.f : 0.f), base));
+        };
+        if (as) {
+            softmax_crf_grad(z + (size_t)pix, as + (size_t)b * K * HW + pix, K, HW, t, n_norm, add_ce);
+        } else {
+            const SoftmaxStat sm = softmax_stat(z + (size_t)pix, K, HW);
+            for (int k = 0; k < K; k++)
+                add_ce(k, ld_grad(g + ((size_t)k * HW + pix)), seg_value<true>(z + (size_t)pix, k, HW, sm));
         }
     }
 }
@@ -1758,8 +1901,17 @@ static void launch_build(const BuildParams &bp, dim3 grid, bool dedup, cudaStrea
 }
 
 template <int D, int V>
-static void launch_pixel_v(bool splat, const PixelParams &pp, dim3 grid, cudaStream_t st)
+static void launch_pixel_v(bool splat, bool lowp, const PixelParams &pp, dim3 grid, cudaStream_t st)
 {
+    if constexpr (V > 1) {   // (2-byte logits always have K >= 2, hence V >= 2)
+        if (lowp) {
+            if (splat)
+                launch_chained(splat_lowp_kernel<D, V>, grid, st, pp);
+            else
+                launch_chained(slice_lowp_kernel<D, V>, grid, st, pp);
+            return;
+        }
+    }
     if (splat) {
         if (pp.logits)
             launch_chained(splat_kernel<D, V, true>, grid, st, pp);
@@ -1774,32 +1926,35 @@ static void launch_pixel_v(bool splat, const PixelParams &pp, dim3 grid, cudaStr
 }
 
 template <int D, int KV>
-static void launch_splat_rows(const PixelParams &pp, int frames, cudaStream_t st)
+static void launch_splat_rows(bool lowp, const PixelParams &pp, int frames, cudaStream_t st)
 {
     const dim3 grid((pp.P + RowMap<KV>::kPpb - 1) / RowMap<KV>::kPpb, frames);
-    if (pp.logits)
+    if (lowp)
+        launch_chained(splat_rows_lowp_kernel<D, KV>, grid, st, pp);
+    else if (pp.logits)
         launch_chained(splat_rows_kernel<D, KV, true>, grid, st, pp);
     else
         launch_chained(splat_rows_kernel<D, KV, false>, grid, st, pp);
 }
 
+// lowp: the logits are 2-byte (pp.bf16 says which type)
 template <int D>
-static void launch_pixel(bool splat, int V, const PixelParams &pp, dim3 grid, cudaStream_t st)
+static void launch_pixel(bool splat, bool lowp, int V, const PixelParams &pp, dim3 grid, cudaStream_t st)
 {
     if (splat && pp.dense && V == 4) {
         switch (pp.Kp / 4) {   // rows of 2..4 float4s (K = 5..16)
-        case 2: return launch_splat_rows<D, 2>(pp, grid.y, st);
-        case 3: return launch_splat_rows<D, 3>(pp, grid.y, st);
-        case 4: return launch_splat_rows<D, 4>(pp, grid.y, st);
+        case 2: return launch_splat_rows<D, 2>(lowp, pp, grid.y, st);
+        case 3: return launch_splat_rows<D, 3>(lowp, pp, grid.y, st);
+        case 4: return launch_splat_rows<D, 4>(lowp, pp, grid.y, st);
         default: break;
         }
     }
     if (V == 4)
-        launch_pixel_v<D, 4>(splat, pp, grid, st);
+        launch_pixel_v<D, 4>(splat, lowp, pp, grid, st);
     else if (V == 2)
-        launch_pixel_v<D, 2>(splat, pp, grid, st);
+        launch_pixel_v<D, 2>(splat, lowp, pp, grid, st);
     else
-        launch_pixel_v<D, 1>(splat, pp, grid, st);
+        launch_pixel_v<D, 1>(splat, lowp, pp, grid, st);
 }
 
 template <int V, int KV>
@@ -1955,7 +2110,7 @@ static void density_hint_refresh(Device &dev, const Plan &pl, char *ws, cudaStre
 // Stage 2: splat -> blur x(d+1) -> slice (+ loss) for the frames [frame0, frame0 + nc) of a chunk whose lattice
 // is built.  segs / as_out point at frame0.  `zero_values`: the value rows were not cleared by lattice_stages.
 template <int D>
-static int value_stages(Device &dev, const Plan &pl, const float *segs, float *as_out, int frame0, int nc, char *ws,
+static int value_stages(Device &dev, const Plan &pl, const void *segs, float *as_out, int frame0, int nc, char *ws,
                         bool zero_values, bool want_loss, float *loss_final, float n_norm, int flags, cudaStream_t st)
 {
     int *ctrl = (int *)(ws + pl.off_ctrl);
@@ -1981,6 +2136,8 @@ static int value_stages(Device &dev, const Plan &pl, const float *segs, float *a
     PixelParams pp;
     pp.segs = segs;
     pp.logits = flags & kFlagLogits;
+    pp.bf16 = (flags & kFlagBF16) ? 1 : 0;
+    const bool lowp = (flags & kFlagLowp) != 0;
     pp.as_out = as_out;
     pp.offset = (int *)(ws + pl.off_offset);
     pp.bary = (float *)(ws + pl.off_bary);
@@ -2003,7 +2160,7 @@ static int value_stages(Device &dev, const Plan &pl, const float *segs, float *a
     pp.alpha = 1.0f / (1 + powf(2, -D));
     {
         StageScope scope(kStSplat, 1, st);
-        launch_pixel<D>(true, V, pp, pgrid, st);
+        launch_pixel<D>(true, lowp, V, pp, pgrid, st);
     }
 
     float *src = val0, *dst = val1;
@@ -2030,7 +2187,7 @@ static int value_stages(Device &dev, const Plan &pl, const float *segs, float *a
     pp.values = src;
     {
         StageScope scope(kStSlice, 1, st);
-        launch_pixel<D>(false, V, pp, pgrid, st);
+        launch_pixel<D>(false, lowp, V, pp, pgrid, st);
     }
     CUDA_TRY(cudaGetLastError());
     return TCAMCRF_OK;
@@ -2054,7 +2211,7 @@ static int run_lattice(Device &dev, const tcamcrf_config *cfg, const Plan &pl, b
     TCAMCRF_DISPATCH_D(pl.D, lattice_stages<D>(dev, cfg, pl, u8, images, frame0, nc, ws, zero_values, st));
 }
 
-static int run_values(Device &dev, const Plan &pl, const float *segs, float *as_out, int frame0, int nc, char *ws,
+static int run_values(Device &dev, const Plan &pl, const void *segs, float *as_out, int frame0, int nc, char *ws,
                       bool zero_values, bool want_loss, float *loss_final, float n_norm, int flags, cudaStream_t st)
 {
     TCAMCRF_DISPATCH_D(pl.D, value_stages<D>(dev, pl, segs, as_out, frame0, nc, ws, zero_values, want_loss, loss_final,
@@ -2062,7 +2219,7 @@ static int run_values(Device &dev, const Plan &pl, const float *segs, float *as_
 }
 
 static int run_chunk(Device &dev, const tcamcrf_config *cfg, const Plan &pl, bool u8, const void *images,
-                     const float *segs, float *as_out, int nc, char *ws, bool want_loss, float *loss_final,
+                     const void *segs, float *as_out, int nc, char *ws, bool want_loss, float *loss_final,
                      float n_norm, int flags, cudaStream_t st)
 {
     int rc = run_lattice(dev, cfg, pl, u8, images, 0, nc, ws, true, st);
@@ -2080,7 +2237,7 @@ static int run_chunk(Device &dev, const tcamcrf_config *cfg, const Plan &pl, boo
 //
 // One chunk whose frames come from the host: `img_host` / `img_dev` point at frame 0 of the chunk.
 static int run_chunk_host_frames(Device &dev, const tcamcrf_config *cfg, const Plan &pl, bool u8, const char *img_host,
-                                 char *img_dev, const float *segs, float *as_out, int nc, bool first_chunk,
+                                 char *img_dev, const void *segs, float *as_out, int nc, bool first_chunk,
                                  bool last_chunk, char *ws, bool want_loss, float *loss_final, float n_norm, int flags,
                                  cudaStream_t st)
 {
@@ -2123,8 +2280,8 @@ static int run_chunk_host_frames(Device &dev, const tcamcrf_config *cfg, const P
 }
 
 // `images_host` != NULL: the frames are there (same element type) and `images` is the device buffer they are
-// staged in.
-static int run_filter(const tcamcrf_config *cfg, bool u8, const void *images, const float *segs, float *as_out,
+// staged in.  `segs` holds float32 values, or 2-byte logits with kFlagLowp.
+static int run_filter(const tcamcrf_config *cfg, bool u8, const void *images, const void *segs, float *as_out,
                       float *loss, int N, int K, int H, int W, float n_norm, void *workspace, size_t ws_bytes,
                       cudaStream_t st, int flags = 0, const void *images_host = nullptr)
 {
@@ -2135,8 +2292,9 @@ static int run_filter(const tcamcrf_config *cfg, bool u8, const void *images, co
     if (ws_bytes < pl.total)
         return fail(TCAMCRF_ERR_WORKSPACE, "workspace too small: %zu < %zu bytes", ws_bytes, pl.total);
     if (((uintptr_t)workspace & 255) != 0) return fail(TCAMCRF_ERR_WORKSPACE, "workspace must be 256-byte aligned");
-    if (((uintptr_t)segs & 3) || ((uintptr_t)as_out & 3) || (!u8 && ((uintptr_t)images & 3)))
-        return fail(TCAMCRF_ERR_INVALID, "float buffers must be 4-byte aligned");
+    const size_t seg_elem = (flags & kFlagLowp) ? 2 : 4;
+    if (((uintptr_t)segs & (seg_elem - 1)) || ((uintptr_t)as_out & 3) || (!u8 && ((uintptr_t)images & 3)))
+        return fail(TCAMCRF_ERR_INVALID, "buffers must be aligned to their element size");
     Device *dev = nullptr;
     rc = this_device(&dev);
     if (rc) return rc;
@@ -2151,11 +2309,11 @@ static int run_filter(const tcamcrf_config *cfg, bool u8, const void *images, co
         if (images_host)
             rc = run_chunk_host_frames(*dev, cfg, pl, u8,
                                        (const char *)images_host + (size_t)n0 * cfg->image_stride_planes * pl.P * img_elem,
-                                       const_cast<char *>(img), segs + (size_t)n0 * K * pl.P,
+                                       const_cast<char *>(img), (const char *)segs + (size_t)n0 * K * pl.P * seg_elem,
                                        as_out + (size_t)n0 * K * pl.P, nc, n0 == 0, last, ws, loss != nullptr,
                                        last ? loss : nullptr, n_norm, flags, st);
         else
-            rc = run_chunk(*dev, cfg, pl, u8, img, segs + (size_t)n0 * K * pl.P, as_out + (size_t)n0 * K * pl.P, nc, ws,
+            rc = run_chunk(*dev, cfg, pl, u8, img, (const char *)segs + (size_t)n0 * K * pl.P * seg_elem, as_out + (size_t)n0 * K * pl.P, nc, ws,
                            loss != nullptr, last ? loss : nullptr, n_norm, flags, st);
         if (rc) return rc;
     }
@@ -2752,19 +2910,52 @@ int tcamcrf_loss_forward(const tcamcrf_config *cfg, const float *images_dev, con
                       workspace_bytes, (cudaStream_t)cuda_stream);
 }
 
-int tcamcrf_loss_forward_host_frames(const tcamcrf_config *cfg, const void *images_host, void *images_stage_dev,
-                                     int images_u8, const float *segs_dev, float *as_dev, float *loss_dev, int logits,
-                                     int N, int K, int H, int W, float n_norm, void *workspace,
-                                     size_t workspace_bytes, void *cuda_stream)
+// run_filter flags for logits of TCAMCRF_DTYPE_* `dtype`, or -1 (with an error set) for an unknown code
+static int logits_flags(int dtype)
+{
+    switch (dtype) {
+    case TCAMCRF_DTYPE_F32: return kFlagLogits;
+    case TCAMCRF_DTYPE_F16: return kFlagLogits | kFlagLowp;
+    case TCAMCRF_DTYPE_BF16: return kFlagLogits | kFlagLowp | kFlagBF16;
+    }
+    fail(TCAMCRF_ERR_INVALID, "unknown logits dtype code %d", dtype);
+    return -1;
+}
+
+static int host_frames_forward(const tcamcrf_config *cfg, const void *images_host, void *images_stage_dev,
+                               int images_u8, const void *segs_dev, float *as_dev, float *loss_dev, int flags, int N,
+                               int K, int H, int W, float n_norm, void *workspace, size_t workspace_bytes,
+                               void *cuda_stream)
 {
     if (!images_host || !images_stage_dev) return fail(TCAMCRF_ERR_INVALID, "null image pointer");
     if (cfg && cfg->channels > cfg->image_stride_planes)
         return fail(TCAMCRF_ERR_INVALID, "overlapping image windows (stride < channels) need device frames or the "
                     "host-pointer API");
+    const bool logits = (flags & kFlagLogits) != 0;
     if (logits && K < 2) return fail(TCAMCRF_ERR_INVALID, "softmax needs at least two classes");
     if (logits && !loss_dev) return fail(TCAMCRF_ERR_INVALID, "null loss pointer");
     return run_filter(cfg, images_u8 != 0, images_stage_dev, segs_dev, as_dev, loss_dev, N, K, H, W, n_norm, workspace,
-                      workspace_bytes, (cudaStream_t)cuda_stream, logits ? kFlagLogits : 0, images_host);
+                      workspace_bytes, (cudaStream_t)cuda_stream, flags, images_host);
+}
+
+int tcamcrf_loss_forward_host_frames(const tcamcrf_config *cfg, const void *images_host, void *images_stage_dev,
+                                     int images_u8, const float *segs_dev, float *as_dev, float *loss_dev, int logits,
+                                     int N, int K, int H, int W, float n_norm, void *workspace,
+                                     size_t workspace_bytes, void *cuda_stream)
+{
+    return host_frames_forward(cfg, images_host, images_stage_dev, images_u8, segs_dev, as_dev, loss_dev,
+                               logits ? kFlagLogits : 0, N, K, H, W, n_norm, workspace, workspace_bytes, cuda_stream);
+}
+
+int tcamcrf_loss_forward_host_frames_typed(const tcamcrf_config *cfg, const void *images_host, void *images_stage_dev,
+                                           int images_u8, const void *logits_dev, int logits_dtype, float *as_dev,
+                                           float *loss_dev, int N, int K, int H, int W, float n_norm, void *workspace,
+                                           size_t workspace_bytes, void *cuda_stream)
+{
+    const int flags = logits_flags(logits_dtype);
+    if (flags < 0) return TCAMCRF_ERR_INVALID;
+    return host_frames_forward(cfg, images_host, images_stage_dev, images_u8, logits_dev, as_dev, loss_dev, flags, N,
+                               K, H, W, n_norm, workspace, workspace_bytes, cuda_stream);
 }
 
 int tcamcrf_loss_forward_u8(const tcamcrf_config *cfg, const uint8_t *images_dev, const float *segs_dev,
@@ -2780,10 +2971,21 @@ int tcamcrf_loss_forward_logits(const tcamcrf_config *cfg, const void *images_de
                                 const float *logits_dev, float *as_dev, float *loss_dev, int N, int K, int H, int W,
                                 float n_norm, void *workspace, size_t workspace_bytes, void *cuda_stream)
 {
+    return tcamcrf_loss_forward_logits_typed(cfg, images_dev, images_u8, logits_dev, TCAMCRF_DTYPE_F32, as_dev,
+                                             loss_dev, N, K, H, W, n_norm, workspace, workspace_bytes, cuda_stream);
+}
+
+int tcamcrf_loss_forward_logits_typed(const tcamcrf_config *cfg, const void *images_dev, int images_u8,
+                                      const void *logits_dev, int logits_dtype, float *as_dev, float *loss_dev, int N,
+                                      int K, int H, int W, float n_norm, void *workspace, size_t workspace_bytes,
+                                      void *cuda_stream)
+{
+    const int flags = logits_flags(logits_dtype);
+    if (flags < 0) return TCAMCRF_ERR_INVALID;
     if (!loss_dev) return fail(TCAMCRF_ERR_INVALID, "null loss pointer");
     if (K < 2) return fail(TCAMCRF_ERR_INVALID, "softmax needs at least two classes");
     return run_filter(cfg, images_u8 != 0, images_dev, logits_dev, as_dev, loss_dev, N, K, H, W, n_norm, workspace,
-                      workspace_bytes, (cudaStream_t)cuda_stream, kFlagLogits);
+                      workspace_bytes, (cudaStream_t)cuda_stream, flags);
 }
 
 int tcamcrf_loss_backward_logits(const float *as_dev, const float *logits_dev, const float *grad_out_dev,
@@ -2797,6 +2999,15 @@ int tcamcrf_loss_backward_logits_weighted(const float *as_dev, const float *logi
                                           float *grad_logits_dev, int N, int K, int H, int W, float n_norm,
                                           float weight, void *cuda_stream)
 {
+    return tcamcrf_loss_backward_logits_typed(as_dev, logits_dev, TCAMCRF_DTYPE_F32, grad_out_dev, grad_logits_dev, N,
+                                              K, H, W, n_norm, weight, cuda_stream);
+}
+
+int tcamcrf_loss_backward_logits_typed(const float *as_dev, const void *logits_dev, int logits_dtype,
+                                       const float *grad_out_dev, void *grad_logits_dev, int N, int K, int H, int W,
+                                       float n_norm, float weight, void *cuda_stream)
+{
+    if (logits_flags(logits_dtype) < 0) return TCAMCRF_ERR_INVALID;
     if (!as_dev || !logits_dev || !grad_out_dev || !grad_logits_dev)
         return fail(TCAMCRF_ERR_INVALID, "null pointer argument");
     if (N < 1 || K < 2 || H < 1 || W < 1) return fail(TCAMCRF_ERR_INVALID, "N,H,W must be positive and K >= 2");
@@ -2806,8 +3017,15 @@ int tcamcrf_loss_backward_logits_weighted(const float *as_dev, const float *logi
     long long blocks = (pixels + kThreads - 1) / kThreads;
     if (blocks > persistent_grid(*dev)) blocks = persistent_grid(*dev);
     StageScope scope(kStBackward, 1, (cudaStream_t)cuda_stream);
-    loss_backward_logits_kernel<<<(unsigned)blocks, kThreads, 0, (cudaStream_t)cuda_stream>>>(
-        as_dev, logits_dev, grad_out_dev, grad_logits_dev, K, H * W, pixels, n_norm, weight);
+    if (logits_dtype == TCAMCRF_DTYPE_F32) {
+        loss_backward_logits_kernel<<<(unsigned)blocks, kThreads, 0, (cudaStream_t)cuda_stream>>>(
+            as_dev, (const float *)logits_dev, grad_out_dev, (float *)grad_logits_dev, K, H * W, pixels, n_norm, weight);
+    } else {
+        const int bf16 = logits_dtype == TCAMCRF_DTYPE_BF16;
+        loss_backward_logits_lowp_kernel<<<(unsigned)blocks, kThreads, 0, (cudaStream_t)cuda_stream>>>(
+            as_dev, Logits16{(const unsigned short *)logits_dev, bf16}, grad_out_dev,
+            Grad16{(unsigned short *)grad_logits_dev, bf16}, K, H * W, pixels, n_norm, weight);
+    }
     CUDA_TRY(cudaGetLastError());
     return TCAMCRF_OK;
 }
@@ -3159,6 +3377,15 @@ int tcam_seed_ce_forward(const float *logits_dev, const int *sel_dev, int kmax, 
                          float *scratch_dev, float *loss_dev, float *count_dev, const float *add_dev, float weight,
                          float *total_dev, void *cuda_stream)
 {
+    return tcam_seed_ce_forward_typed(logits_dev, TCAMCRF_DTYPE_F32, sel_dev, kmax, B, K, H, W, ksz, scratch_dev,
+                                      loss_dev, count_dev, add_dev, weight, total_dev, cuda_stream);
+}
+
+int tcam_seed_ce_forward_typed(const void *logits_dev, int logits_dtype, const int *sel_dev, int kmax, int B, int K,
+                               int H, int W, int ksz, float *scratch_dev, float *loss_dev, float *count_dev,
+                               const float *add_dev, float weight, float *total_dev, void *cuda_stream)
+{
+    if (logits_flags(logits_dtype) < 0) return TCAMCRF_ERR_INVALID;
     if (!logits_dev || !sel_dev || !scratch_dev || !loss_dev || !count_dev)
         return fail(TCAMCRF_ERR_INVALID, "null pointer argument");
     if (B < 1 || K < 2 || H < 1 || W < 1 || kmax < 1 || ksz < 1)
@@ -3179,8 +3406,12 @@ int tcam_seed_ce_forward(const float *logits_dev, const int *sel_dev, int kmax, 
     sp.W = W;
     sp.kmax = kmax;
     sp.ksz = ksz;
+    sp.bf16 = logits_dtype == TCAMCRF_DTYPE_BF16;
     StageScope scope(kStSeed, 1, (cudaStream_t)cuda_stream);
-    seed_ce_forward_kernel<<<B, 256, 0, (cudaStream_t)cuda_stream>>>(sp);
+    if (logits_dtype == TCAMCRF_DTYPE_F32)
+        seed_ce_forward_kernel<<<B, 256, 0, (cudaStream_t)cuda_stream>>>(sp);
+    else
+        seed_ce_forward_lowp_kernel<<<B, 256, 0, (cudaStream_t)cuda_stream>>>(sp);
     CUDA_TRY(cudaGetLastError());
     return TCAMCRF_OK;
 }
@@ -3189,15 +3420,56 @@ int tcam_seed_ce_backward(const float *logits_dev, const int *sel_dev, int kmax,
                           const float *count_dev, const float *grad_out_dev, float scale, float *grad_logits_dev,
                           void *cuda_stream)
 {
+    return tcam_seed_ce_backward_typed(logits_dev, TCAMCRF_DTYPE_F32, sel_dev, kmax, B, K, H, W, ksz, count_dev,
+                                       grad_out_dev, scale, grad_logits_dev, cuda_stream);
+}
+
+// the cross-entropy's share of the backward pass; crf_as_dev != NULL: grad_logits_dev holds the CRF gradient of
+// loss_backward_logits_lowp_kernel, which the labelled pixels recompute in float32 (seed_ce_backward_lowp_kernel)
+static int seed_ce_backward_any(const void *logits_dev, int logits_dtype, const int *sel_dev, int kmax, int B, int K,
+                                int H, int W, int ksz, const float *count_dev, const float *grad_out_dev, float scale,
+                                void *grad_logits_dev, const float *crf_as_dev, float n_norm, float crf_weight,
+                                cudaStream_t st)
+{
     if (!logits_dev || !sel_dev || !count_dev || !grad_out_dev || !grad_logits_dev)
         return fail(TCAMCRF_ERR_INVALID, "null pointer argument");
     if (B < 1 || K < 2 || H < 1 || W < 1 || kmax < 1 || ksz < 1)
         return fail(TCAMCRF_ERR_INVALID, "B,H,W,kmax,ksz must be positive and K >= 2");
-    StageScope scope(kStSeed, 1, (cudaStream_t)cuda_stream);
-    seed_ce_backward_kernel<<<B, 256, 0, (cudaStream_t)cuda_stream>>>(logits_dev, sel_dev, grad_logits_dev, count_dev,
-                                                                     grad_out_dev, scale, K, H, W, kmax, ksz);
+    StageScope scope(kStSeed, 1, st);
+    if (logits_dtype == TCAMCRF_DTYPE_F32) {
+        seed_ce_backward_kernel<<<B, 256, 0, st>>>((const float *)logits_dev, sel_dev, (float *)grad_logits_dev,
+                                                   count_dev, grad_out_dev, scale, K, H, W, kmax, ksz);
+    } else {
+        const int bf16 = logits_dtype == TCAMCRF_DTYPE_BF16;
+        seed_ce_backward_lowp_kernel<<<B, 256, 0, st>>>(
+            Logits16{(const unsigned short *)logits_dev, bf16}, sel_dev, Grad16{(unsigned short *)grad_logits_dev, bf16},
+            count_dev, grad_out_dev, scale, K, H, W, kmax, ksz, crf_as_dev, n_norm, crf_weight);
+    }
     CUDA_TRY(cudaGetLastError());
     return TCAMCRF_OK;
+}
+
+int tcam_seed_ce_backward_typed(const void *logits_dev, int logits_dtype, const int *sel_dev, int kmax, int B, int K,
+                                int H, int W, int ksz, const float *count_dev, const float *grad_out_dev, float scale,
+                                void *grad_logits_dev, void *cuda_stream)
+{
+    if (logits_flags(logits_dtype) < 0) return TCAMCRF_ERR_INVALID;
+    return seed_ce_backward_any(logits_dev, logits_dtype, sel_dev, kmax, B, K, H, W, ksz, count_dev, grad_out_dev,
+                                scale, grad_logits_dev, nullptr, 0.f, 0.f, (cudaStream_t)cuda_stream);
+}
+
+int tcam_crf_seed_ce_backward_typed(const float *as_dev, const void *logits_dev, int logits_dtype, const int *sel_dev,
+                                    int kmax, int ksz, const float *count_dev, const float *grad_out_dev, int B, int K,
+                                    int H, int W, float n_norm, float crf_weight, float ce_weight,
+                                    void *grad_logits_dev, void *cuda_stream)
+{
+    int rc = tcamcrf_loss_backward_logits_typed(as_dev, logits_dev, logits_dtype, grad_out_dev, grad_logits_dev, B, K,
+                                                H, W, n_norm, crf_weight, cuda_stream);
+    if (rc) return rc;
+    // float32: the cross-entropy is added in place onto the float32 CRF gradient, exactly as before
+    return seed_ce_backward_any(logits_dev, logits_dtype, sel_dev, kmax, B, K, H, W, ksz, count_dev, grad_out_dev,
+                                ce_weight, grad_logits_dev, logits_dtype == TCAMCRF_DTYPE_F32 ? nullptr : as_dev,
+                                n_norm, crf_weight, (cudaStream_t)cuda_stream);
 }
 
 int tcam_seed_labels(const int *sel_dev, int kmax, int B, int H, int W, int ksz, long long ignore_idx,

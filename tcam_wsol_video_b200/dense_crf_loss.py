@@ -142,15 +142,20 @@ class DenseCRFLoss(nn.Module):
 
 class DenseCRFLossFromLogitsFunction(Function):
     """``DenseCRFLossFunction`` applied to ``softmax(logits, dim=1)`` with the softmax (forward and backward)
-    fused into the CRF kernels -- the probabilities are never written to memory (SURVEY.md §8f.1)."""
+    fused into the CRF kernels -- the probabilities are never written to memory (SURVEY.md §8f.1).
+
+    float16 and bfloat16 logits (what a model run under autocast produces) are read as they are and get their
+    gradient in their own dtype: no float32 copy, no cast of the gradient.  The computation is float32 throughout, so
+    the gradient has the bits of the float32 path on the widened logits cast back.  Other dtypes are cast to float32
+    (ops.library_logits); this holds for the three logits Functions below."""
 
     @staticmethod
-    @torch.amp.custom_fwd(device_type='cuda', cast_inputs=torch.float32)
+    @torch.amp.custom_fwd(device_type='cuda')
     def forward(ctx, images, logits, sigma_rgb, sigma_xy, weight=1.0):
         n = logits.shape[0]
         cfg = _lib.make_config(ops.FEAT_XY_RGB, 3, sigma_rgb, sigma_xy, loss_weight=weight)
         _lib.require_key_range(cfg, logits.shape[2], logits.shape[3])
-        logits = logits.detach().contiguous()
+        logits = ops.library_logits(logits.detach())
         as_t, loss, _ = ops.crf_forward_logits(images, logits, cfg, n_norm=float(n))
         ctx.AS = as_t
         ctx.logits = logits
@@ -196,9 +201,9 @@ class SeedCrossEntropyFunction(Function):
     loss and its gradient come from the labelled pixels alone (csrc/seed.cuh, seed_ce_*_kernel)."""
 
     @staticmethod
-    @torch.amp.custom_fwd(device_type='cuda', cast_inputs=torch.float32)
+    @torch.amp.custom_fwd(device_type='cuda')
     def forward(ctx, logits, sel, ksz):
-        logits = logits.detach().contiguous()
+        logits = ops.library_logits(logits.detach())
         loss, count, _ = ops.seed_ce_forward(logits, sel, ksz)
         ctx.logits, ctx.sel, ctx.ksz, ctx.count = logits, sel, int(ksz), count
         return loss
@@ -219,12 +224,12 @@ class CrfAndSeedCEFromLogitsFunction(Function):
     only the total carries a gradient."""
 
     @staticmethod
-    @torch.amp.custom_fwd(device_type='cuda', cast_inputs=torch.float32)
+    @torch.amp.custom_fwd(device_type='cuda')
     def forward(ctx, images, logits, sigma_rgb, sigma_xy, crf_weight, sel, ksz, ce_weight):
         n = logits.shape[0]
         cfg = _lib.make_config(ops.FEAT_XY_RGB, 3, sigma_rgb, sigma_xy, loss_weight=crf_weight)
         _lib.require_key_range(cfg, logits.shape[2], logits.shape[3])
-        logits = logits.detach().contiguous()
+        logits = ops.library_logits(logits.detach())
         as_t, crf_loss, _ = ops.crf_forward_logits(images, logits, cfg, n_norm=float(n))
         # the kernel that finishes the cross-entropy also forms total = crf + ce_weight * ce: no torch glue launches
         ce_loss, count, total = ops.seed_ce_forward(logits, sel, ksz, add=crf_loss, weight=float(ce_weight))
@@ -237,6 +242,6 @@ class CrfAndSeedCEFromLogitsFunction(Function):
     @staticmethod
     @torch.amp.custom_bwd(device_type='cuda')
     def backward(ctx, grad_total, _g_crf, _g_ce):
-        grad = ops.crf_backward_logits(ctx.AS, ctx.logits, grad_total, float(ctx.N), ctx.crf_weight)
-        ops.seed_ce_backward_(grad, ctx.logits, ctx.sel, ctx.ksz, ctx.count, grad_total, ctx.ce_weight)
+        grad = ops.crf_seed_ce_backward(ctx.AS, ctx.logits, ctx.sel, ctx.ksz, ctx.count, grad_total, float(ctx.N),
+                                        ctx.crf_weight, ctx.ce_weight)
         return None, grad, None, None, None, None, None, None

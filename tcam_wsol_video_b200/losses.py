@@ -96,6 +96,14 @@ class ElementaryLoss(nn.Module):
         self.c_epoch = epoch
 
 
+def _check_seeds(seeds: SparseSeeds, fcams: torch.Tensor) -> None:
+    """SparseSeeds label pixels by index: seeds made for other frames (another resolution or batch) would label the
+    wrong pixels, where the reference's cross-entropy raises on the mismatched target."""
+    if (seeds.h, seeds.w) != tuple(fcams.shape[2:]) or seeds.sel.shape[0] != fcams.shape[0]:
+        raise ValueError(f'seeds were made for {seeds.sel.shape[0]} frames of {seeds.h}x{seeds.w}, the maps are '
+                         f'{tuple(fcams.shape)}')
+
+
 class SelfLearningTcams(ElementaryLoss):
     """Cross-entropy of the decoder's maps against the sampled seeds (tcam.py:48-77)."""
 
@@ -112,6 +120,7 @@ class SelfLearningTcams(ElementaryLoss):
         if isinstance(seeds, SparseSeeds):
             if seeds.ignore_idx != self.seg_ignore_idx:
                 raise ValueError('seeds were made with another ignore index')
+            _check_seeds(seeds, fcams)
             return SeedCrossEntropyFunction.apply(fcams, seeds.sel, seeds.ksz) * self.lambda_
         return self.loss(input=fcams, target=seeds) * self.lambda_
 
@@ -161,6 +170,7 @@ class FusedTcamLosses(nn.Module):
                    and seeds.ignore_idx == self.sl.seg_ignore_idx)
         if not fusable:
             return self.sl(epoch=epoch, fcams=fcams, seeds=seeds) + self.crf(epoch=epoch, fcams=fcams, raw_img=raw_img)
+        _check_seeds(seeds, fcams)
         total, self.last_crf, ce = CrfAndSeedCEFromLogitsFunction.apply(
             raw_img, fcams, self.crf.sigma_rgb, self.crf.sigma_xy, w_crf, seeds.sel, seeds.ksz, w_sl)
         self.last_ce = ce           # the unweighted cross-entropy; last_crf is the weighted CRF term (for logging)

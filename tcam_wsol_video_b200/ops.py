@@ -270,16 +270,39 @@ class Lattice:
         return workspace_status(ws)
 
 
+# logits the kernels read as they are (TCAMCRF_DTYPE_*): float32, and the two autocast dtypes
+_LOGIT_DTYPES = {torch.float32: _lib.DTYPE_F32, torch.float16: _lib.DTYPE_F16, torch.bfloat16: _lib.DTYPE_BF16}
+
+
+def library_logits(logits: torch.Tensor) -> torch.Tensor:
+    """`logits` as the library reads them: float32, float16 and bfloat16 as they are (no copy when contiguous), any
+    other dtype cast to float32; contiguous."""
+    if logits.dtype not in _LOGIT_DTYPES:
+        logits = logits.float()
+    return logits.contiguous()
+
+
+def _logits_code(logits: torch.Tensor) -> int:
+    """TCAMCRF_DTYPE_* of logits about to be handed to the library: 4-D, contiguous, CUDA, of a dtype it reads."""
+    _require_cuda(logits, "logits")
+    if logits.ndim != 4:
+        raise TcamCrfError(f"logits must be [B,K,H,W], got {tuple(logits.shape)}")
+    if not logits.is_contiguous():
+        raise TcamCrfError("logits must be contiguous")
+    if logits.dtype not in _LOGIT_DTYPES:
+        raise TcamCrfError(f"logits must be float32, float16 or bfloat16, got {logits.dtype}")
+    return _LOGIT_DTYPES[logits.dtype]
+
+
 def crf_forward_logits(images: torch.Tensor, logits: torch.Tensor, cfg: _lib.Config, n_norm: Optional[float] = None,
                        check: Optional[bool] = None):
     """Like crf_forward(want_loss=True) with segs = softmax(logits, dim=1) formed inside the kernels.
-    Returns (AS, loss [1], workspace)."""
+    float16 and bfloat16 logits are read as they are (see library_logits).  Returns (AS float32, loss [1], workspace)."""
     lib = _lib.load()
     _require_cuda(logits, "logits")
     device = logits.device
-    if logits.dtype != torch.float32:
-        logits = logits.float()
-    logits = logits.contiguous()
+    logits = library_logits(logits)
+    dtype = _logits_code(logits)
     n, k, h, w = logits.shape
     if k < 2:
         raise TcamCrfError("the fused softmax needs at least two classes")
@@ -302,19 +325,19 @@ def crf_forward_logits(images: torch.Tensor, logits: torch.Tensor, cfg: _lib.Con
         ws = _workspace(device, nbytes)
         ws_ptr = (ws.data_ptr() + 255) // 256 * 256
         ws_bytes = ws.numel() - (ws_ptr - ws.data_ptr())
-        as_out = torch.empty_like(logits)
+        as_out = torch.empty(logits.shape, dtype=torch.float32, device=device)
         loss = torch.empty(1, dtype=torch.float32, device=device)
         if host_frames is not None:
-            rc = lib.tcamcrf_loss_forward_host_frames(
-                byref(cfg), host_frames.data_ptr(), images.data_ptr(), 1 if u8 else 0, logits.data_ptr(),
-                as_out.data_ptr(), loss.data_ptr(), 1, n, k, h, w, float(n if n_norm is None else n_norm), ws_ptr, ws_bytes,
+            rc = lib.tcamcrf_loss_forward_host_frames_typed(
+                byref(cfg), host_frames.data_ptr(), images.data_ptr(), 1 if u8 else 0, logits.data_ptr(), dtype,
+                as_out.data_ptr(), loss.data_ptr(), n, k, h, w, float(n if n_norm is None else n_norm), ws_ptr, ws_bytes,
                 _stream_ptr(device))
             _keep_until_done(host_frames, device)
         else:
-            rc = lib.tcamcrf_loss_forward_logits(byref(cfg), images.data_ptr(), 1 if u8 else 0, logits.data_ptr(),
-                                                 as_out.data_ptr(), loss.data_ptr(), n, k, h, w,
-                                                 float(n if n_norm is None else n_norm), ws_ptr, ws_bytes,
-                                                 _stream_ptr(device))
+            rc = lib.tcamcrf_loss_forward_logits_typed(byref(cfg), images.data_ptr(), 1 if u8 else 0, logits.data_ptr(),
+                                                       dtype, as_out.data_ptr(), loss.data_ptr(), n, k, h, w,
+                                                       float(n if n_norm is None else n_norm), ws_ptr, ws_bytes,
+                                                       _stream_ptr(device))
         _lib.check(rc, "tcamcrf_loss_forward_logits")
         if STRICT if check is None else check:
             _raise_on_status(ws if ws_ptr == ws.data_ptr() else ws[ws_ptr - ws.data_ptr():])
@@ -324,19 +347,29 @@ def crf_forward_logits(images: torch.Tensor, logits: torch.Tensor, cfg: _lib.Con
 def crf_backward_logits(as_t: torch.Tensor, logits: torch.Tensor, grad_output: torch.Tensor, n_norm: float,
                         weight: float = 1.0):
     """Gradient w.r.t. the logits (CRF gradient chained through the softmax) in one kernel; `weight`: the module's
-    weight when it was folded into the forward (cfg.loss_weight)."""
+    weight when it was folded into the forward (cfg.loss_weight).  The gradient has the dtype the library read the
+    logits in (library_logits): float16 / bfloat16 logits get theirs, rounded once from the float32 value."""
     lib = _lib.load()
     _require_cuda(as_t, "AS")
     n, k, h, w = as_t.shape
-    logits = logits.detach().float().contiguous()
+    logits = library_logits(logits.detach())
+    dtype = _logits_code(logits)
+    _check_as(as_t, logits)
     g = grad_output.detach().reshape(-1)[:1].to(device=as_t.device, dtype=torch.float32).contiguous()
-    grad = torch.empty_like(as_t)
+    grad = torch.empty_like(logits)
     with torch.cuda.device(as_t.device):
-        _lib.check(lib.tcamcrf_loss_backward_logits_weighted(as_t.data_ptr(), logits.data_ptr(), g.data_ptr(),
-                                                             grad.data_ptr(), n, k, h, w, float(n_norm), float(weight),
-                                                             _stream_ptr(as_t.device)),
-                   "tcamcrf_loss_backward_logits_weighted")
+        _lib.check(lib.tcamcrf_loss_backward_logits_typed(as_t.data_ptr(), logits.data_ptr(), dtype, g.data_ptr(),
+                                                          grad.data_ptr(), n, k, h, w, float(n_norm), float(weight),
+                                                          _stream_ptr(as_t.device)),
+                   "tcamcrf_loss_backward_logits_typed")
     return grad
+
+
+def _check_as(as_t: torch.Tensor, logits: torch.Tensor) -> None:
+    if as_t.dtype != torch.float32 or not as_t.is_contiguous() or as_t.shape != logits.shape or \
+            as_t.device != logits.device:
+        raise TcamCrfError(f"AS must be contiguous float32 {tuple(logits.shape)} on {logits.device}, got "
+                           f"{as_t.dtype} {tuple(as_t.shape)} on {as_t.device}")
 
 
 def crf_backward(as_t: torch.Tensor, grad_output: torch.Tensor, n_norm: float, weight: float = 1.0) -> torch.Tensor:
@@ -356,12 +389,26 @@ def crf_backward(as_t: torch.Tensor, grad_output: torch.Tensor, n_norm: float, w
 _seed_ce_scratch: Dict[Tuple[int, int, int], torch.Tensor] = {}
 
 
+def _check_seeds(logits: torch.Tensor, sel: torch.Tensor) -> None:
+    """sel: the int32 [B,2,kmax] seeds of the B samples of `logits`, contiguous, on their device."""
+    if sel.dtype != torch.int32 or sel.ndim != 3 or sel.shape[0] != logits.shape[0] or sel.shape[1] != 2 or \
+            sel.shape[2] < 1 or sel.device != logits.device or not sel.is_contiguous():
+        raise TcamCrfError(f"sel must be contiguous int32 [{logits.shape[0]},2,kmax] on {logits.device}, got "
+                           f"{sel.dtype} {tuple(sel.shape)} on {sel.device}")
+
+
 def seed_ce_forward(logits: torch.Tensor, sel: torch.Tensor, ksz: int, add: Optional[torch.Tensor] = None,
                     weight: float = 1.0):
     """Cross-entropy of `logits` [B,K,H,W] on the seeds `sel` [B,2,kmax] (see tcam_seed_ce_forward): returns
-    (loss [1], count [1] float32 = labelled pixels, total [1] = add + weight * loss or None without `add`)."""
+    (loss [1], count [1] float32 = labelled pixels, total [1] = add + weight * loss or None without `add`).
+    float16 and bfloat16 logits are read as they are, other dtypes cast to float32 (library_logits); the results are
+    float32."""
     lib = _lib.load()
     _require_cuda(logits, "logits")
+    if logits.dtype not in _LOGIT_DTYPES:
+        logits = logits.float()
+    dtype = _logits_code(logits)
+    _check_seeds(logits, sel)
     b, k, h, w = logits.shape
     device = logits.device
     key = (device.index if device.index is not None else torch.cuda.current_device(), _stream_ptr(device), b)
@@ -372,25 +419,64 @@ def seed_ce_forward(logits: torch.Tensor, sel: torch.Tensor, ksz: int, add: Opti
             _seed_ce_scratch[key] = scratch
     out = torch.empty(3, dtype=torch.float32, device=device)     # loss, count, total
     with torch.cuda.device(device):
-        _lib.check(lib.tcam_seed_ce_forward(logits.data_ptr(), sel.data_ptr(), int(sel.shape[2]), b, k, h, w, int(ksz),
-                                            scratch.data_ptr(), out.data_ptr(), out.data_ptr() + 4,
-                                            add.data_ptr() if add is not None else None, float(weight),
-                                            out.data_ptr() + 8 if add is not None else None, _stream_ptr(device)),
+        _lib.check(lib.tcam_seed_ce_forward_typed(logits.data_ptr(), dtype, sel.data_ptr(), int(sel.shape[2]), b, k, h,
+                                                  w, int(ksz), scratch.data_ptr(), out.data_ptr(), out.data_ptr() + 4,
+                                                  add.data_ptr() if add is not None else None, float(weight),
+                                                  out.data_ptr() + 8 if add is not None else None, _stream_ptr(device)),
                    "tcam_seed_ce_forward")
     return out[0:1], out[1:2], (out[2:3] if add is not None else None)
 
 
+def _check_grad(grad_logits: torch.Tensor, logits: torch.Tensor) -> None:
+    if grad_logits.dtype != logits.dtype or grad_logits.shape != logits.shape or \
+            grad_logits.device != logits.device or not grad_logits.is_contiguous():
+        raise TcamCrfError(f"the gradient buffer must be contiguous {logits.dtype} {tuple(logits.shape)} on "
+                           f"{logits.device}, got {grad_logits.dtype} {tuple(grad_logits.shape)} on {grad_logits.device}")
+
+
 def seed_ce_backward_(grad_logits: torch.Tensor, logits: torch.Tensor, sel: torch.Tensor, ksz: int, count: torch.Tensor,
                       grad_output: torch.Tensor, scale: float = 1.0) -> torch.Tensor:
-    """grad_logits += (grad_output * scale) * d CE / d logits, in place on the labelled pixels."""
+    """grad_logits += (grad_output * scale) * d CE / d logits, in place on the labelled pixels.  grad_logits has the
+    dtype the library reads the logits in (library_logits); a float16 / bfloat16 element is rounded once from the
+    float32 sum."""
     lib = _lib.load()
+    _require_cuda(logits, "logits")
+    if logits.dtype not in _LOGIT_DTYPES:
+        logits = logits.float()
+    dtype = _logits_code(logits)
+    _check_seeds(logits, sel)
+    _check_grad(grad_logits, logits)
     b, k, h, w = logits.shape
     g = grad_output.detach().reshape(-1)[:1].to(device=logits.device, dtype=torch.float32).contiguous()
     with torch.cuda.device(logits.device):
-        _lib.check(lib.tcam_seed_ce_backward(logits.data_ptr(), sel.data_ptr(), int(sel.shape[2]), b, k, h, w, int(ksz),
-                                             count.data_ptr(), g.data_ptr(), float(scale), grad_logits.data_ptr(),
-                                             _stream_ptr(logits.device)), "tcam_seed_ce_backward")
+        _lib.check(lib.tcam_seed_ce_backward_typed(logits.data_ptr(), dtype, sel.data_ptr(), int(sel.shape[2]), b, k, h,
+                                                   w, int(ksz), count.data_ptr(), g.data_ptr(), float(scale),
+                                                   grad_logits.data_ptr(), _stream_ptr(logits.device)),
+                   "tcam_seed_ce_backward")
     return grad_logits
+
+
+def crf_seed_ce_backward(as_t: torch.Tensor, logits: torch.Tensor, sel: torch.Tensor, ksz: int, count: torch.Tensor,
+                         grad_output: torch.Tensor, n_norm: float, crf_weight: float, ce_weight: float) -> torch.Tensor:
+    """Gradient w.r.t. the logits of crf_weight * CRF(softmax(logits)) + ce_weight * CE(logits, seeds)
+    (tcam_crf_seed_ce_backward_typed): crf_backward_logits with the cross-entropy's gradient added on the labelled
+    pixels, every element rounded once to the dtype the library read the logits in."""
+    lib = _lib.load()
+    _require_cuda(as_t, "AS")
+    logits = library_logits(logits.detach())
+    dtype = _logits_code(logits)
+    _check_as(as_t, logits)
+    _check_seeds(logits, sel)
+    b, k, h, w = logits.shape
+    g = grad_output.detach().reshape(-1)[:1].to(device=logits.device, dtype=torch.float32).contiguous()
+    grad = torch.empty_like(logits)
+    with torch.cuda.device(logits.device):
+        _lib.check(lib.tcam_crf_seed_ce_backward_typed(as_t.data_ptr(), logits.data_ptr(), dtype, sel.data_ptr(),
+                                                       int(sel.shape[2]), int(ksz), count.data_ptr(), g.data_ptr(), b,
+                                                       k, h, w, float(n_norm), float(crf_weight), float(ce_weight),
+                                                       grad.data_ptr(), _stream_ptr(logits.device)),
+                   "tcam_crf_seed_ce_backward_typed")
+    return grad
 
 
 def temporal_cam_max(cams: torch.Tensor, renorm_h: float = 0.0) -> torch.Tensor:
@@ -486,5 +572,5 @@ def roi_components(cams: torch.Tensor, largest_only: bool, p_min_area: float, th
     return roi, mask, bbox.float()
 
 
-__all__ = ["Lattice", "seed_ce_forward", "seed_ce_backward_", "otsu_roi", "roi_components", "crf_filter_transposed", "crf_forward", "crf_backward", "crf_forward_logits", "crf_backward_logits", "temporal_cam_max", "prepare_std_cams", "workspace_status", "release_workspaces",
+__all__ = ["Lattice", "library_logits", "seed_ce_forward", "seed_ce_backward_", "crf_seed_ce_backward", "otsu_roi", "roi_components", "crf_filter_transposed", "crf_forward", "crf_backward", "crf_forward_logits", "crf_backward_logits", "temporal_cam_max", "prepare_std_cams", "workspace_status", "release_workspaces",
            "FEAT_COLOR", "FEAT_XY_RGB"]
